@@ -6,6 +6,7 @@
     python bench.py --scaling strong ...                          # 5000 images TOTAL, interleaved over the ranks
     python bench.py --config producer [--producer-dtype fp32]     # configs[4]: DPT-L producer -> reasoning, 1024x1024
     python bench.py --config antialias [--images 16]              # the second resize mode (tile path), image by image
+    python bench.py ... --dump-outputs DIR                        # also write the last timed step's result as .npy
 
 configs[1] (default): a COCO-val-shaped synthetic batch — 5000 images of 480x640 fields, 4096 proposals per
 image — through discovery (existence check, center reasoning, iterative boundary refinement, NMS), scoring +
@@ -13,6 +14,16 @@ mask rasterisation and the post-process predicate.  One "step" = one pass over t
 JSON line (rank 0).  Default scaling is weak (every rank owns `--images` images, seeds = global image index);
 the only collective is ONE all_gather_into_tensor of the fixed-capacity detection-row buffer at the end of a
 step, inside the timed region, with no host synchronisation in front of it.
+
+``--dump-outputs DIR`` writes what the last timed step delivered to its caller as ``DIR/<name>.npy``.  The inputs
+are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
+  * reasoning and producer configs: ``detections`` float64 ``[K, 6]`` rows ``(image_id, x, y, w, h, score)`` (COCO
+    xywh boxes), image-sorted: the gathered detection rows.
+  * antialias config: ``discovery`` float64 ``[D, 5]`` rows ``(image, x1, y1, x2, y2)``; ``annotations`` float64
+    ``[A, 10]`` rows ``(image, x, y, w, h, score, existence_score, center_score, boundary_score, area_score)``;
+    ``masks`` float32 ``[M, H, W]``, a seeded sample of at most DUMP_MASKS of the annotation masks, and
+    ``mask_index`` float64 ``[M]``, the annotation rows they belong to.
+Above DUMP_BYTES in all, every array keeps a fixed, seeded sample of its rows.
 """
 from __future__ import annotations
 
@@ -31,6 +42,8 @@ sys.path.insert(0, ROOT)
 H, W, N_PROP = 480, 640, 4096
 WORKLOAD = "configs[1]: 5000 synthetic 480x640 field stacks x 4096 proposals/image, discovery + scoring"
 XU_CYCLES_PER_ROW = 98.0   # 12.2 MUFU warp-instructions per output row (ex2, rcp, sqrt per pixel) x 8 cycles on the 4-lane XU pipe of one SM sub-partition
+DUMP_BYTES = 64_000_000    # upper bound of what --dump-outputs writes
+DUMP_MASKS = 16            # masks --dump-outputs keeps in the antialias config (1.2 MB each in float32 at 480x640)
 
 
 def parse():
@@ -51,7 +64,34 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """{name: float32 / float64 array (numpy or torch, any device)} -> out_dir/<name>.npy.  If the arrays hold
+    more than DUMP_BYTES together, each one keeps a share of DUMP_BYTES in proportion to its size: a fixed,
+    seeded choice of its rows (first axis), in their order."""
+    import numpy as np
+    arrs = {k: v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v) for k, v in arrays.items()}
+    for k, a in arrs.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{k}: {a.dtype} (dumps are float32 or float64)")
+    total = sum(a.nbytes for a in arrs.values())
+    budget = DUMP_BYTES - 4096 * len(arrs)   # 4096: room for each .npy header
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        if total > budget and a.ndim and a.shape[0]:
+            cap = (budget * a.nbytes // total) // a[:1].nbytes
+            if a.shape[0] > cap:
+                a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], cap, replace=False))]
+        np.save(os.path.join(out_dir, f"{k}.npy"), np.ascontiguousarray(a))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -218,12 +258,16 @@ def run_antialias(args):
     props = [synth.make_proposals(i, args.proposals, H, W) for i in range(n_img)]
 
     def step():
-        n = 0
-        for f, p in zip(imgs, props):
+        """-> (annotations, [(image, discovered boxes)], [annotations with their masks])"""
+        n, dets, anns = 0, [], []
+        for k, (f, p) in enumerate(zip(imgs, props)):
             det = od.discover_image(f, p)
+            dets.append((k, det))
             if len(det):
-                n += len(sc.score_image(f, det.astype(np.float64).tolist()))
-        return n
+                a = sc.score_image(f, det.astype(np.float64).tolist(), image_id=k)
+                n += len(a)
+                anns += a
+        return n, dets, anns
 
     for _ in range(max(1, min(args.warmup, 1))):
         step()
@@ -231,9 +275,18 @@ def run_antialias(args):
     l0 = ops.LAUNCHES
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        n_ann = step()
+        n_ann, dets, anns = step()
     torch.cuda.synchronize()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs is not None:
+        keys = ("score", "existence_score", "center_score", "boundary_score", "area_score")
+        masks = np.stack([a["segmentation"]["mask"] for a in anns]) if anns else np.zeros((0, H, W), np.uint8)
+        pick = np.sort(np.random.default_rng(0).choice(len(anns), min(len(anns), DUMP_MASKS), replace=False))
+        dump_outputs(args.dump_outputs, {
+            "discovery": np.array([[k, *b] for k, det in dets for b in det], np.float64).reshape(-1, 5),
+            "annotations": np.array([[a["image_id"], *a["bbox"], *(a[c] for c in keys)] for a in anns],
+                                    np.float64).reshape(-1, 10),
+            "masks": masks[pick].astype(np.float32), "mask_index": pick.astype(np.float64)})
     print(json.dumps({"metric": "object_reasoning_images_per_sec", "value": n_img / dt, "unit": "images/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
                       "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -405,6 +458,8 @@ def main():
         raise RuntimeError("detection row buffer overflowed: raise max_rows")
     result_rows = merged[: int(total.item())]
     digest = rows_digest(result_rows)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, {"detections": result_rows})
 
     # ---- hardware equality: rank 0 recomputes, on its own, a slice of images that ANOTHER rank owned and
     # compares the rows the collective delivered for them, bit for bit (outside the timed region)
@@ -603,7 +658,7 @@ def main():
         freed[0].record(); freed[1].record()
         e2e_step()
         barrier()
-        reps = max(1, min(args.steps, 2))
+        reps = args.steps   # timed end-to-end steps, like the device-resident ones
         t0 = time.perf_counter()
         for _ in range(reps):
             last = e2e_step()
@@ -631,7 +686,7 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dt, dt_rows = float(t[0].item()), float(t[1].item())
         e2e = {"value": n_global / dt, "unit": "images/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h_full,
-               "host_pool_images": pool, "ms_per_step": dt * 1e3,
+               "host_pool_images": pool, "ms_per_step": dt * 1e3, "steps": reps,
                "result": "detection rows (image_id, x, y, w, h, score) fp64 + COCO RLE run lengths of every kept mask "
                          "(unmore_mask_rle_counts; the existing run lengths of each mask + its length, int32)",
                "masks_rle_per_step": n_rle_full, "rle_complete": bool(rle_ok),

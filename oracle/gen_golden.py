@@ -4,6 +4,7 @@ reference (/root/reference) on CPU through oracle/ref_harness.py.
 Run in the build container (the reference does not exist on the GPU box):
 
     python -m oracle.gen_golden            # writes tests/golden/
+    python -m oracle.gen_golden signatures # only tests/golden/reference_signatures.json
 
 Everything stored is an output of reference code (or a library op the reference calls
 at the cited line), never of this repo's oracle or CUDA path.
@@ -35,6 +36,34 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 def _quiet(fn, *a, **k):
     with redirect_stdout(io.StringIO()):
         return fn(*a, **k)
+
+
+def _ast_params(path, class_name=None):
+    """{function name: [positional parameter names]} of a module (or one class of it), read with ``ast``."""
+    import ast
+    with open(path) as f:
+        tree = ast.parse(f.read())
+    body = tree.body
+    if class_name is not None:
+        body = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == class_name).body
+    return {n.name: [x.arg for x in n.args.posonlyargs + n.args.args] for n in body if isinstance(n, ast.FunctionDef)}
+
+
+def reference_signatures(root):
+    """Parameter lists of the reference's Object_Discovery / Object_Scoring methods, batch_erode and
+    convert_pred_annotations_to_training_format (what tests/test_cpu_host.py pins the mirrors against)."""
+    misc = _ast_params(os.path.join(root, "utils", "misc.py"))
+    post = _ast_params(os.path.join(root, "post_process.py"))
+    return {"Object_Discovery": _ast_params(os.path.join(root, "object_reasoning.py"), "Object_Discovery"),
+            "Object_Scoring": _ast_params(os.path.join(root, "object_scoring.py"), "Object_Scoring"),
+            "functions": {"batch_erode": misc["batch_erode"],
+                          "convert_pred_annotations_to_training_format": post["convert_pred_annotations_to_training_format"]}}
+
+
+def gen_signatures():
+    with open(os.path.join(GOLD, "reference_signatures.json"), "w") as f:
+        json.dump(reference_signatures(rh.REFERENCE_ROOT), f, indent=1)
+    print("reference_signatures.json written")
 
 
 def gen_units(od):
@@ -365,7 +394,11 @@ def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 1)
     od = rh.make_discovery(480, 640)
-    which = sys.argv[1:] or ["units", "scene_a", "scene_b", "main", "scene_cc"]
+    which = sys.argv[1:] or ["signatures", "units", "scene_a", "scene_b", "main", "scene_cc"]
+    if "signatures" in which:
+        gen_signatures()
+        if which == ["signatures"]:
+            return
     if "units" in which:
         gen_units(od)
     if "units_aa" in which:

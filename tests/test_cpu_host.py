@@ -219,53 +219,49 @@ def test_header_is_plain_c_and_links(tmp_path):
     subprocess.run(["g++", "-std=c++17", "-Wall", "-Werror", "-I", inc, "-c", str(cpp), "-o", str(tmp_path / "t.o")], check=True)
 
 
-def _ast_signatures(path, class_name=None):
-    """{function name: [positional parameter names]} of a module (or one class of it) WITHOUT importing it."""
-    import ast
-    with open(path) as f:
-        tree = ast.parse(f.read())
-    body = tree.body
-    if class_name is not None:
-        body = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == class_name).body
-    out = {}
-    for n in body:
-        if isinstance(n, ast.FunctionDef):
-            a = n.args
-            names = [x.arg for x in a.posonlyargs + a.args]
-            n_def = len(a.defaults)
-            out[n.name] = (names, names[: len(names) - n_def] if n_def else names)
-    return out
+GOLDEN_SIGNATURES = os.path.join(ROOT, "tests", "golden", "reference_signatures.json")
+REFERENCE_ROOT = os.environ.get("UNMORE_REFERENCE_ROOT", "")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference sources only exist in the build container")
+def _reference_signatures():
+    """Parameter lists of the reference's public entry points: the stored ones (``python -m oracle.gen_golden
+    signatures`` with UNMORE_REFERENCE_ROOT set writes them), else read from a reference checkout."""
+    import json
+    if os.path.isfile(GOLDEN_SIGNATURES):
+        with open(GOLDEN_SIGNATURES) as f:
+            return json.load(f)
+    if os.path.isdir(REFERENCE_ROOT):
+        from oracle.gen_golden import reference_signatures
+        return reference_signatures(REFERENCE_ROOT)
+    pytest.skip("the reference's signatures are not stored in tests/golden/reference_signatures.json "
+                "and UNMORE_REFERENCE_ROOT names no checkout of the original vLAR-group/unMORE sources")
+
+
 def test_mirror_signatures_match_the_reference():
     """Every public method of the reference's Object_Discovery / Object_Scoring, batch_erode and
     convert_pred_annotations_to_training_format exists here under the same name, with the reference's
     parameters as a prefix in the same order, and can be called with exactly the reference's required
-    arguments (extra parameters here must be optional).  Read with ``ast``: nothing is imported."""
+    arguments (extra parameters here must be optional).  The reference is read with ``ast``: nothing is imported."""
     import inspect
     from unmore_b200 import object_reasoning, object_scoring, post_process
     from unmore_b200.utils import misc
-    pairs = [("/root/reference/object_reasoning.py", "Object_Discovery", object_reasoning.Object_Discovery),
-             ("/root/reference/object_scoring.py", "Object_Scoring", object_scoring.Object_Scoring)]
+    refsig = _reference_signatures()
     checked = 0
-    for path, cname, cls in pairs:
-        for name, (params, required) in _ast_signatures(path, cname).items():
+    for cname, cls in [("Object_Discovery", object_reasoning.Object_Discovery),
+                       ("Object_Scoring", object_scoring.Object_Scoring)]:
+        for name, params in refsig[cname].items():
             assert hasattr(cls, name), f"{cname}.{name} missing"
             sig = inspect.signature(getattr(cls, name))
             ours = list(sig.parameters)
-            ref = [p for p in params if p != "self"]
-            mine = [p for p in ours if p != "self"]
-            if name == "get_prediction_with_proposal_images":   # a @staticmethod that still lists self in the reference
-                ref = [p for p in ref if p != "self"]
+            ref = [p for p in params if p != "self"]   # also the @staticmethod get_prediction_with_proposal_images,
+            mine = [p for p in ours if p != "self"]     # which still lists self in the reference
             assert mine[: len(ref)] == ref, f"{cname}.{name}: {mine} vs reference {ref}"
             for p in mine[len(ref):]:
                 assert sig.parameters[p].default is not inspect.Parameter.empty, f"{cname}.{name}: extra required parameter {p}"
             checked += 1
-    for path, fn, ours in [("/root/reference/utils/misc.py", "batch_erode", misc.batch_erode),
-                           ("/root/reference/post_process.py", "convert_pred_annotations_to_training_format",
-                            post_process.convert_pred_annotations_to_training_format)]:
-        params, _ = _ast_signatures(path)[fn]
+    for fn, ours in [("batch_erode", misc.batch_erode),
+                     ("convert_pred_annotations_to_training_format", post_process.convert_pred_annotations_to_training_format)]:
+        params = refsig["functions"][fn]
         assert list(inspect.signature(ours).parameters)[: len(params)] == params, fn
         checked += 1
     assert checked >= 24
