@@ -19,7 +19,10 @@
  *   - proposal lists are ragged with a fixed capacity: boxes [n_img, cap, 4] xyxy, fp32 or
  *     fp64 (boxes_f64 != 0; the reference hands fp64 anchors to round 0, object_reasoning.py
  *     :190-194), image i owning the first counts[i] rows; counts == NULL means all cap rows;
- *   - `ws` is a scheduling workspace of unmore_workspace_bytes(n_img) bytes.
+ *   - `ws` is a scheduling workspace of unmore_workspace_bytes(n_img) bytes (4-byte aligned): the work
+ *     counter and the per-image row offsets, then, from the next 32-byte boundary, one window cache of
+ *     unmore_boundary_refine per image (a fixed number of 32-byte slots each, 1 MB per image).  Every
+ *     call re-initialises what it uses; nothing in it outlives a call.
  *   - resize semantics: bilinear, align_corners=False, NO antialias (torchvision 0.14.1, the
  *     version the reference pins), arithmetic bit-identical to ATen's CPU kernels.
  */
@@ -40,7 +43,7 @@ typedef void* unmore_stream_t; /* cudaStream_t */
 
 const char* unmore_last_error(void);
 int unmore_version(void);
-/* bytes of the scheduling workspace `ws` used by the list-driven kernels */
+/* bytes of the scheduling workspace `ws` used by the list-driven kernels (grows by ~1 MB per image) */
 size_t unmore_workspace_bytes(int n_img);
 
 /* existence_checking — object_reasoning.py:491-523 (Binary_Classifier replaced by the mean of
@@ -124,7 +127,9 @@ int unmore_cc_cap(void);
  * With n_round=1, apply_small_filter=0 it is exactly optimize_one_image_single_round.
  * boxes_out [n_img, cap, 4] fp32; labels_out [n_img, cap] fp32: 1 / 0 / -1 as the reference,
  * -2 = removed by filter_small_proposal (not in the reference's returned list);
- * rounds_out [n_img, cap] int32 (nullable): rounds actually evaluated. */
+ * rounds_out [n_img, cap] int32 (nullable): rounds actually evaluated.
+ * Proposals of one image share the boundary terms of a crop window through the window cache in `ws`
+ * (fields up to 32767 px per side); the results are bit-identical to evaluating every window. */
 int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, int ch_sdf,
                            const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
                            int apply_small_filter, int early_exit, float proposal_area_thres,

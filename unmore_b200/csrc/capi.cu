@@ -37,7 +37,16 @@ int num_sms() {  // of the current device; a plain attribute query, no cached st
   return 148;
 }
 
-// ws layout: [0] work counter, [1 .. n_img+1] exclusive prefix of counts
+// ws layout: [0] work counter, [1 .. n_img+1] exclusive prefix of counts (ints); then, at the first 32-byte
+// aligned address after them, the window caches of unmore_boundary_refine: n_img tables of kWindowSlots
+// WindowSlot entries, zeroed by that call (a table lives for one call; the other kernels leave it alone)
+size_t worklist_bytes(int n_img) { return sizeof(int) * (size_t)(n_img + 2 > 2 ? n_img + 2 : 2); }
+
+WindowSlot* window_tables(void* ws, int n_img) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(ws) + worklist_bytes(n_img);
+  return reinterpret_cast<WindowSlot*>((a + alignof(WindowSlot) - 1) & ~(uintptr_t)(alignof(WindowSlot) - 1));
+}
+
 int make_worklist(WorkList& w, const int* counts, int n_img, int cap, void* ws, cudaStream_t s) {
   int* wsi = reinterpret_cast<int*>(ws);
   w.counter = wsi;
@@ -85,7 +94,10 @@ extern "C" {
 
 const char* unmore_last_error(void) { return g_err; }
 int unmore_version(void) { return 100; }
-size_t unmore_workspace_bytes(int n_img) { return sizeof(int) * (size_t)(n_img + 2 > 2 ? n_img + 2 : 2); }
+size_t unmore_workspace_bytes(int n_img) {
+  // the alignment slack lets `ws` be any 4-byte aligned pointer
+  return worklist_bytes(n_img) + (n_img > 0 ? alignof(WindowSlot) - 1 + sizeof(WindowSlot) * kWindowSlots * (size_t)n_img : 0);
+}
 
 int unmore_existence_scores(const float* fields, int n_img, int C, int H, int W, int ch_exist, const void* boxes,
                             int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
@@ -190,6 +202,11 @@ int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, 
   p.max_shrink_thres = max_shrink_threshold; p.delta_ratio = delta_ratio;
   p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.labels_out = labels_out; p.rounds_out = rounds_out;
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  if (W <= kWindowMaxSide && H <= kWindowMaxSide) {
+    p.windows = window_tables(ws, n_img);
+    const int e = (int)cudaMemsetAsync(p.windows, 0, sizeof(WindowSlot) * kWindowSlots * (size_t)n_img, s);
+    if (e) return cuda_fail(e, "memset window tables");
+  }
   return cuda_fail(launch_refine(p, num_sms(), s), "refine_kernel");
 }
 

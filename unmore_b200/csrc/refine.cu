@@ -91,6 +91,8 @@ struct BorderCols {
   float bot[kCrop];
   double acc[4][32];   // sum A, sum A*g, sum B, sum B*g per lane
   int2 tapy[kCrop];    // vertical taps of the current window: (i0, bits of l1) per output row
+  int pub;             // lane 0: window-cache slot to publish this round's terms into, or -1 (in shared memory: a
+                       // register live across boundary_terms costs spills around its row loop)
 };
 
 struct Deltas {
@@ -246,6 +248,66 @@ __device__ __forceinline__ Deltas boundary_terms(RowSrc& src, BorderCols& cols, 
   return d;
 }
 
+// ---- window cache (WindowSlot, unmore_internal.h) ----------------------------------------------------------
+// Deltas are a function of the field plane and the snapped window only, and boundary_terms gives the same bits
+// whichever warp runs it, so a round may take them from the warp that computed its window first.  Only lane 0
+// touches the table, once per round.  A slot goes 0 -> key (claimed: the claimer is computing) -> key | ready
+// (published with a release store after the terms).  A warp that finds its window claimed waits a bounded
+// number of polls (sleeping, so the other warps of the SM get its issue slots), then computes the terms itself
+// without publishing; so does a warp whose probe path is full.  No warp waits on another without a limit.
+#ifndef UNMORE_WINDOW_PROBES
+#define UNMORE_WINDOW_PROBES 16
+#endif
+#ifndef UNMORE_WINDOW_WAIT_POLLS
+#define UNMORE_WINDOW_WAIT_POLLS 160   // 64 ns doubling to 1 us per poll: at most ~160 us of sleep
+#endif
+constexpr unsigned long long kWindowReady = 1ull << 63;
+
+__device__ __forceinline__ unsigned long long window_key(const Window& w) {
+  return (unsigned long long)w.x1 | (unsigned long long)w.y1 << 15 | (unsigned long long)w.x2 << 30 |
+         (unsigned long long)w.y2 << 45;
+}
+__device__ __forceinline__ unsigned long long ld_acquire_key(const WindowSlot* s) {
+  unsigned long long v;
+  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(&s->key) : "memory");
+  return v;
+}
+
+// Lane 0.  true: `d` holds the published terms of the window.  false: the caller computes them, and publishes
+// them into slot `pub` when pub >= 0 (this warp claimed it).
+__device__ __forceinline__ bool window_lookup(WindowSlot* table, const Window& win, Deltas& d, int& pub) {
+  const unsigned long long key = window_key(win);
+  const unsigned h = (unsigned)((key * 0x9E3779B97F4A7C15ull) >> 32);
+  pub = -1;
+  for (int probe = 0; probe < UNMORE_WINDOW_PROBES; ++probe) {
+    const int i = (int)((h + probe) & (kWindowSlots - 1));
+    WindowSlot* s = table + i;
+    unsigned long long k = ld_acquire_key(s);
+    if (k == 0) {
+      if (atomicCAS(&s->key, 0ull, key) == 0ull) { pub = i; return false; }
+      k = ld_acquire_key(s);   // lost the race: the slot now holds some window, claimed or published
+    }
+    if ((k & ~kWindowReady) != key) continue;
+    for (int poll = 0, ns = 64; !(k & kWindowReady); ++poll) {
+      if (poll == UNMORE_WINDOW_WAIT_POLLS) return false;
+      __nanosleep(ns);
+      ns = min(2 * ns, 1024);
+      k = ld_acquire_key(s);
+    }
+    asm volatile("ld.relaxed.gpu.global.f32 %0, [%1];" : "=f"(d.max_sdf) : "l"(&s->max_sdf) : "memory");
+    asm volatile("ld.relaxed.gpu.global.v4.f32 {%0, %1, %2, %3}, [%4];"
+                 : "=f"(d.dx1), "=f"(d.dy1), "=f"(d.dx2), "=f"(d.dy2) : "l"(&s->d) : "memory");
+    return true;
+  }
+  return false;
+}
+
+__device__ __forceinline__ void window_publish(WindowSlot* s, const Window& win, const Deltas& d) {
+  s->max_sdf = d.max_sdf;
+  s->d = make_float4(d.dx1, d.dy1, d.dx2, d.dy2);
+  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(&s->key), "l"(window_key(win) | kWindowReady) : "memory");
+}
+
 template <typename T>
 struct BoxT { T x1, y1, x2, y2; };
 
@@ -344,12 +406,28 @@ __global__ void __launch_bounds__(kRefineWarps * 32, UNMORE_REFINE_MINBLOCKS) re
       float4 nb = make_float4(0.f, 0.f, 0.f, 0.f);
       int lab = -1;   // a zero-size crop (the reference would raise) is defined as "no object"
       bool fixed = false;
-      if (!win.empty()) {
+      // boundary_terms stays at the nesting depth it had without the cache: one more level of divergent control
+      // flow around it costs registers and instructions in its row loop
+      Deltas d;
+      int hit = 0;
+      if (p.windows && lane == 0 && !win.empty()) hit = window_lookup(p.windows + (size_t)img * kWindowSlots, win, d, cols.pub);
+      hit = __shfl_sync(kFullMask, hit, 0);
+      if (!win.empty() && !hit) {
         CropRows<ROW_ELEMS> src;
         src.taps.template init<kStrided>(lane, win.w());
         src.plane.init(plane, p.W, win);
         src.init_rows(lane, cols.tapy, win.h());
-        const Deltas d = boundary_terms(src, cols, lane);
+        d = boundary_terms(src, cols, lane);
+        if (p.windows && lane == 0 && cols.pub >= 0) window_publish(p.windows + (size_t)img * kWindowSlots + cols.pub, win, d);
+      }
+      if (hit) {
+        d.max_sdf = __shfl_sync(kFullMask, d.max_sdf, 0);
+        d.dx1 = __shfl_sync(kFullMask, d.dx1, 0);
+        d.dy1 = __shfl_sync(kFullMask, d.dy1, 0);
+        d.dx2 = __shfl_sync(kFullMask, d.dx2, 0);
+        d.dy2 = __shfl_sync(kFullMask, d.dy2, 0);
+      }
+      if (!win.empty()) {
         if (d.max_sdf > p.max_sdf_thres) {
           if (dbl) {
             BoxT<double> bd;

@@ -13,6 +13,22 @@ struct FieldDesc {
 };
 
 // ---- refine.cu -----------------------------------------------------------------------
+// Per-image window cache of the fused refine kernel: the boundary terms of a crop window depend only on the
+// field plane and the snapped integer window, and proposals of one image converge onto the same windows.
+// One open-addressed table of kWindowSlots 32-byte slots per image, in the workspace (make_worklist).
+#ifndef UNMORE_WINDOW_SLOTS
+#define UNMORE_WINDOW_SLOTS 32768   // power of two; ~15k distinct windows per benchmark image at most
+#endif
+constexpr int kWindowSlots = UNMORE_WINDOW_SLOTS;
+static_assert((kWindowSlots & (kWindowSlots - 1)) == 0, "UNMORE_WINDOW_SLOTS must be a power of two");
+constexpr int kWindowMaxSide = 32767;   // window corners are packed in 15 bits each; larger fields share nothing
+struct alignas(32) WindowSlot {
+  unsigned long long key;   // 0 = empty; packed window, bit 63 set once the terms below are published
+  float max_sdf, pad;
+  float4 d;                 // dx1, dy1, dx2, dy2
+};
+static_assert(sizeof(WindowSlot) == 32, "one sector per slot");
+
 struct RefineParams {
   const float* fields;
   int C, H, W, ch_sdf;
@@ -26,6 +42,7 @@ struct RefineParams {
   float4* boxes_out;   // [n_img, cap]
   float* labels_out;   // 1 / 0 / -1 as the reference; -2 = removed by filter_small_proposal
   int* rounds_out;     // rounds actually evaluated (nullable)
+  WindowSlot* windows; // [n_img][kWindowSlots], zeroed before launch; nullptr: every round computes its terms
 };
 struct TileParams {
   const float* tiles;  // [M, 128, 128]
