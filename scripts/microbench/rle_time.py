@@ -1,5 +1,5 @@
-"""Time of unmore_mask_rle_counts on one chunk worth of kept masks (1750 x 480x640); build with -DUNMORE_RLE_SERIAL for the
-bit-serial round-1 kernel: 1.60 ms vs 0.34 ms on one B200."""
+"""Time of unmore_mask_rle_counts on one chunk worth of kept masks (1750 x 480x640): 0.34 ms on one B200, where the
+bit-serial round-1 kernel took 1.60 ms."""
 import os, sys, torch, numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from unmore_b200 import ops

@@ -23,7 +23,7 @@ for line in res.splitlines():
     if name and "REG:" in line: usage[name] = line.strip(); name = None
 want = [("refine_kernelILi640", "refine_kernel_640", True), ("center_kernelILb0ELi307200ELb1", "center_kernel_spec", False), ("center_kernelILb0ELi307200ELb0", "center_kernel_spec_second_pass", False),
         ("rle_counts_kernelILb1", "rle_counts_kernel", False),
-        ("16existence_kernelE", "existence_kernel", False), ("existence_kernel_tma", "existence_kernel_tma", False), ("sat_kernel_tmaILi5", "sat_kernel_tma_5", False),
+        ("16existence_kernelE", "existence_kernel", False), ("sat_kernel_tmaILi5", "sat_kernel_tma_5", False),
         ("pack_kernel_vec", "pack_kernel_vec", False), ("score_kernel", "score_kernel", False)]
 KEY = ["UBLKCP", "UTMALDG", "SYNCS", "FFMA2", "FMUL2", "FADD2", "LDGSTS", "MUFU", "LDG", "LDS", "STS", "SHFL", "VOTE", "POPC", "IMAD", "BAR", "WARPSYNC"]
 for pat, tag, want_loop in want:

@@ -75,6 +75,18 @@ void anti_center_filter(double* filt) {
     }
 }
 
+// Both filter tables of the center kernel: fp64 for the exact pass, (channel 0, channel 1) fp32 pairs for the screening pass
+void center_filters(CenterParams& p) {
+  anti_center_filter(p.filt);
+  for (int i = 0; i < 5; ++i)
+    for (int j = 0; j < 5; ++j) {   // exact casts: the table is fp32-valued
+      const float f0 = (float)p.filt[i * 5 + j], f1 = (float)p.filt[j * 5 + i];
+      unsigned lo, hi;
+      memcpy(&lo, &f0, 4); memcpy(&hi, &f1, 4);
+      p.filt_pair[i * 5 + j] = ((unsigned long long)hi << 32) | lo;
+    }
+}
+
 int check_fields(const float* f, int n_img, int C, int H, int W) {
   if (!f || n_img <= 0 || C <= 0 || H <= 0 || W <= 0) return fail(UNMORE_E_INVALID, "bad field tensor");
   // the kernels are launched on the CURRENT device: a field stack that lives on another GPU would be read
@@ -172,14 +184,7 @@ int unmore_center_reasoning(const float* fields, int n_img, int C, int H, int W,
   if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
     return fail(UNMORE_E_INVALID, "unmore_center_reasoning: the three analyze_cc outputs go together");
   p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
-  anti_center_filter(p.filt);
-  for (int i = 0; i < 5; ++i)
-    for (int j = 0; j < 5; ++j) {   // exact casts: the table is fp32-valued
-      const float f0 = (float)p.filt[i * 5 + j], f1 = (float)p.filt[j * 5 + i];
-      unsigned lo, hi;
-      memcpy(&lo, &f0, 4); memcpy(&hi, &f1, 4);
-      p.filt_pair[i * 5 + j] = ((unsigned long long)hi << 32) | lo;
-    }
+  center_filters(p);
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
   return cuda_fail(launch_center(p, num_sms(), s), "center_kernel");
 }
@@ -238,14 +243,7 @@ int unmore_center_reasoning_from_tiles(const float* tiles, int n_img, int H, int
   if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
     return fail(UNMORE_E_INVALID, "unmore_center_reasoning_from_tiles: the three analyze_cc outputs go together");
   p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
-  anti_center_filter(p.filt);
-  for (int i = 0; i < 5; ++i)
-    for (int j = 0; j < 5; ++j) {
-      const float f0 = (float)p.filt[i * 5 + j], f1 = (float)p.filt[j * 5 + i];
-      unsigned lo, hi;
-      memcpy(&lo, &f0, 4); memcpy(&hi, &f1, 4);
-      p.filt_pair[i * 5 + j] = ((unsigned long long)hi << 32) | lo;
-    }
+  center_filters(p);
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
   return cuda_fail(launch_center(p, num_sms(), s), "center_kernel (tiles)");
 }
@@ -281,7 +279,7 @@ int unmore_score_and_rasterise_from_tiles(const float* tiles, const float* exist
   return cuda_fail(launch_score(p, (cudaStream_t)stream), "score_kernel (tiles)");
 }
 
-int unmore_cc_cap(void) { return UNMORE_CC_CAP; }
+int unmore_cc_cap(void) { return kCcCap; }
 
 int unmore_compact_boxes(const void* in, int in_f64, const int* counts_in, int cap_in, int group, int mode,
                          const void* pred, float thr, void* out, int out_f64, int cap_out, int* counts_out,
@@ -307,7 +305,7 @@ int unmore_box_nms(const float* boxes, const float* scores, const int* counts, i
   NmsParams p{};
   p.boxes = reinterpret_cast<const float4*>(boxes); p.scores = scores; p.counts = counts; p.cap = cap; p.n_img = n_img;
   p.iou_thr = iou_threshold; p.keep = keep_out; p.keep_counts = keep_counts_out;
-  p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.order_ws = order_ws; p.alive_ws = nullptr;
+  p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.order_ws = order_ws;
   return cuda_fail(launch_box_nms(p, (cudaStream_t)stream), "box_nms_kernel");
 }
 

@@ -15,19 +15,12 @@
 
 namespace unmore {
 
-#ifndef UNMORE_CENTER_LATTICE
-#define UNMORE_CENTER_LATTICE 1   // 0: resample all 128 rows of every proposal (the round-1 schedule); 2: timing-only, pre-pass without skipping
-#endif
-#ifndef UNMORE_CENTER_THREADS
-#define UNMORE_CENTER_THREADS 256
-#endif
-constexpr int kCenterThreads = UNMORE_CENTER_THREADS;
+constexpr int kCenterThreads = 256;
 constexpr int kCenterWarps = kCenterThreads / 32;
 constexpr int kWinLo = 10, kWinHi = 118, kWin = kWinHi - kWinLo;  // staged window of the center field
 constexpr int kWinStride = 110;   // pixels per staged row: 880 B, so 8 lanes on consecutive rows hit 8 distinct 16-B bank groups
 constexpr int kErode = 12;                                         // 3 rounds x radius 4
 constexpr int kCandCap = 1024;                                     // queue of pixels for the exact fp64 pass
-constexpr int kCcCap = UNMORE_CC_CAP;                               // component boxes kept per proposal
 
 struct CenterSmem {
   float2 c[kWin * kWinStride];     // staged center field, (row, col) channels interleaved: one aligned pair per pixel
@@ -395,10 +388,8 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
           }
           const unsigned long long clo = ~klo & (~0ull << kErode), chi = ~khi & (~0ull >> kErode);   // rows 12..63, 64..115
           if (!(clo | chi)) { no_survivors = true; break; }
-#if UNMORE_CENTER_LATTICE != 2   // 2: timing-only, pre-pass without skipping
           rmin = clo ? __ffsll((long long)clo) - 1 : 63 + __ffsll((long long)chi);
           rmax = chi ? 127 - __clzll((long long)chi) : 63 - __clzll((long long)clo);
-#endif
           const int rlo = rmin - kErode, n = rmax + kErode + 1 - rlo, per = (n + kCenterWarps - 1) / kCenterWarps;
           i_begin = rlo + warp * per; i_end = min(rlo + n, i_begin + per); i_step = 1;
         }
@@ -409,7 +400,6 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
       if (lane == 0) sm.red_f[warp] = cabs;
       __syncthreads();
       locate_next();
-#ifndef UNMORE_CENTER_SKIP_S23   // timing-only builds: profiles/r02_center_phase_times.md
       // ---- 2. erosion: 25-runs along rows, then AND of 25 rows
       if (tid == kCrop) sm.cand_n = 0;   // an idle thread of this phase; ordered by the barriers around it
       if (tid < kCrop) {
@@ -429,7 +419,6 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
         store_row(sm.ero[tid], e);
       }
       __syncthreads();
-#ifndef UNMORE_CENTER_SKIP_S3
       // ---- 3. anti-center map on surviving pixels, then masked max / first arg-max.
       // The map is needed in fp64 only where it can decide the result (the maximum).  So: (a) an
       // fp32 register-tiled 5x5x2 correlation over 1x8 pixel strips that contain surviving pixels
@@ -595,8 +584,6 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
         }
         best = ov; best_idx = oi;
       }
-#endif
-#endif
       }   // !no_survivors
     }
     if (tid == 0) {
@@ -794,7 +781,7 @@ int launch_center(const CenterParams& p, int num_sms, cudaStream_t stream) {
   const bool spec = p.H * p.W == kSpecPlaneElems && p.ch_crow == p.ch_sdf + 1 && p.ch_ccol == p.ch_sdf + 2;
   if (p.cc_counts) return spec ? launch_center_t<true, kSpecPlaneElems>(p, num_sms, stream) : launch_center_t<true, 0>(p, num_sms, stream);
   // row skipping (the lattice pre-pass) pays on the loose proposals of the first pass — the one that asks for split boxes
-  if (UNMORE_CENTER_LATTICE && p.splits)
+  if (p.splits)
     return spec ? launch_center_t<false, kSpecPlaneElems, true>(p, num_sms, stream) : launch_center_t<false, 0, true>(p, num_sms, stream);
   return spec ? launch_center_t<false, kSpecPlaneElems>(p, num_sms, stream) : launch_center_t<false, 0>(p, num_sms, stream);
 }

@@ -68,139 +68,6 @@ __global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const Exist
   }
 }
 
-// ---- TMA-fed variant (north-star (b): "field tiles staged in shared memory via TMA") -------------------------------
-// Same arithmetic as existence_kernel, but the source rows of the crop window arrive through the bulk-copy engine: lane 0
-// keeps up to `depth` whole window rows in flight with cp.async.bulk into a per-warp shared-memory ring (one mbarrier per
-// slot, like sat_kernel_tma), and the eight taps of a row become shared-memory loads.  The rows a window needs are known
-// up front — every row 0 .. last when in_h <= 256, the pairs (i0, i0 + 1) of each output row otherwise — and the row cache
-// asks for them in exactly that order, so the consumer just takes the next slot.  A slot holds the window row from its
-// 16-byte-aligned start; windows whose rows are too wide for `UNMORE_EXIST_TMA_MIN_DEPTH` slots take the gather path.
-// Built with -DUNMORE_EXIST_TMA; measured against the gather kernel in profiles/r02_tma_row_ring.md.
-#ifndef UNMORE_EXIST_RING_BYTES
-#define UNMORE_EXIST_RING_BYTES 4096
-#endif
-#ifndef UNMORE_EXIST_TMA_MIN_DEPTH
-#define UNMORE_EXIST_TMA_MIN_DEPTH 3
-#endif
-constexpr int kExistRing = UNMORE_EXIST_RING_BYTES;
-constexpr int kExistMaxDepth = 8;
-struct ExistWarpSmem {
-  int2 tapy[kCrop];
-  alignas(16) unsigned char ring[kExistRing];
-  alignas(8) uint64_t bar[kExistMaxDepth];
-};
-
-__global__ void __launch_bounds__(kExistWarps * 32) existence_kernel_tma(const ExistParams p) {
-  __shared__ __align__(16) ExistWarpSmem sm_all[kExistWarps];
-  const int lane = threadIdx.x & 31;
-  ExistWarpSmem& sm = sm_all[threadIdx.x >> 5];
-  int2* const tapy = sm.tapy;
-  const unsigned tapy_addr = smem_addr(tapy);
-  const unsigned ring_addr = smem_addr(sm.ring);
-  if (lane == 0) {
-    for (int k = 0; k < kExistMaxDepth; ++k) mbar_init(&sm.bar[k], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncwarp();
-  unsigned phase_bits = 0;   // expected parity of every slot's mbarrier
-  const int total = worklist_total(p.work);
-  int img = 0;
-  for (;;) {
-    const int id = worklist_next_warp(p.work);
-    if (id >= total) break;
-    int k;
-    worklist_locate(p.work, id, img, k);
-    const size_t row = (size_t)img * p.work.cap + k;
-    double x1, y1, x2, y2;
-    load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
-    const Window win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
-    float score = 0.f;
-    if (!win.empty()) {
-      ColTaps taps;
-      taps.init<kStrided>(lane, win.w());
-      const float* plane_base = p.fields + ((size_t)img * p.C + p.ch_exist) * p.H * p.W;
-      PlaneRows plane;
-      plane.init(plane_base, p.W, win);
-      const float scale_y = __fdiv_rn((float)win.h(), (float)kCrop);
-      const int in_h = win.h();
-      __syncwarp();
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const AxisTap t = axis_tap(scale_y, lane + 32 * q, in_h);
-        tapy[lane + 32 * q] = make_int2(t.i0, __float_as_int(t.l1));
-      }
-      __syncwarp();
-      // ---- ring geometry of this window
-      const int xa = win.x1 & ~3;                                     // 16-byte aligned start of a window row
-      const unsigned slot_bytes = ((unsigned)(win.x2 - xa) * 4u + 15u) & ~15u;
-      const int depth = min(kExistMaxDepth, (int)(kExistRing / slot_bytes));
-      const bool use_ring = warp_uniform(depth >= UNMORE_EXIST_TMA_MIN_DEPTH);
-      const bool pairs = in_h > 2 * kCrop;
-      const int n_need = pairs ? 2 * kCrop : min(tapy[kCrop - 1].x + 1, in_h - 1) + 1;
-      const float* src0 = plane_base + (size_t)win.y1 * p.W + xa;
-      const unsigned tap_off = (unsigned)(win.x1 - xa) * 4u;
-      auto needed_row = [&](int q) { return pairs ? tapy[q >> 1].x + (q & 1) : q; };   // q-th source row the window needs
-      int cons = 0, slot = 0;
-      if (use_ring && lane == 0) {
-        const int n0 = min(depth, n_need);
-        for (int q = 0; q < n0; ++q) {
-          mbar_expect_tx(&sm.bar[q], slot_bytes);
-          bulk_g2s(sm.ring + (size_t)q * slot_bytes, src0 + (size_t)needed_row(q) * p.W, slot_bytes, &sm.bar[q]);
-        }
-      }
-      // horizontally interpolated source row: the next slot of the ring (rows are asked for in ring order), or a gather
-      auto hrow = [&](int y, f32x2 out[2]) {
-        if (!use_ring) { plane.hrow(taps, y, out); return; }
-        mbar_wait(&sm.bar[slot], (phase_bits >> slot) & 1u);
-        const unsigned base = ring_addr + (unsigned)slot * slot_bytes + tap_off;
-        float v0[4], v1[4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v0[c]) : "r"(base + taps.x0[c]) : "memory");
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v1[c]) : "r"(base + taps.x1[c]) : "memory");
-        }
-#pragma unroll
-        for (int h = 0; h < 2; ++h)
-          out[h] = lerp_h2(pk2(v0[2 * h], v0[2 * h + 1]), pk2(v1[2 * h], v1[2 * h + 1]), taps.w0[h], taps.w1[h]);
-        __syncwarp();                      // every lane has taken its taps: the slot may be refilled
-        phase_bits ^= 1u << slot;
-        if (lane == 0 && cons + depth < n_need) {
-          mbar_expect_tx(&sm.bar[slot], slot_bytes);
-          bulk_g2s(sm.ring + (size_t)slot * slot_bytes, src0 + (size_t)needed_row(cons + depth) * p.W, slot_bytes, &sm.bar[slot]);
-        }
-        ++cons;
-        slot = slot + 1 == depth ? 0 : slot + 1;
-      };
-      double acc = 0.0;
-      f32x2 part = pk2(0.f, 0.f);
-      f32x2 ra[2], rb[2];
-      int cy0 = -1, cy1 = -1;
-      for (int i = 0; i < kCrop; ++i) {
-        int i0, l1b;
-        asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(i0), "=r"(l1b) : "r"(tapy_addr + 8u * (unsigned)i) : "memory");
-        const int i1 = min(i0 + 1, in_h - 1);
-        const float l1 = __int_as_float(l1b), l0 = __fsub_rn(1.f, l1);
-        if (i0 != cy0 || i1 != cy1) {          // warp-uniform; same row-cache walk as PlaneRows::row2
-          if (i0 == cy1) { ra[0] = rb[0]; ra[1] = rb[1]; } else hrow(i0, ra);
-          if (i1 == i0) { rb[0] = ra[0]; rb[1] = ra[1]; } else hrow(i1, rb);
-          cy0 = i0; cy1 = i1;
-        }
-        const f32x2 v0 = lerp_v2(ra[0], rb[0], l0, l1), v1 = lerp_v2(ra[1], rb[1], l0, l1);
-        part = add2(part, add2(v0, v1));
-        if ((i & 7) == 7) {
-          float lo, hi;
-          upk2(part, lo, hi);
-          acc += (double)(lo + hi);
-          part = pk2(0.f, 0.f);
-        }
-      }
-      acc = warp_sum(acc);
-      score = (float)(acc * (1.0 / (kCrop * kCrop)));
-    }
-    if (lane == 0) p.scores[row] = score;
-  }
-}
-
 // ---- a2 / a4 as a stand-alone op: the resized crops themselves --------------------------------
 // crop + Resize((128,128), BILINEAR) of object_reasoning.py:402-410 / get_prediction_with_proposals
 // (:301-337, object_scoring.py:112-157) for every (proposal, selected channel): out[row][k] is the
@@ -292,13 +159,6 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 }
 
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream) {
-#ifdef UNMORE_EXIST_TMA
-  // bulk copies need 16-byte aligned rows: W % 4 == 0 and an aligned field stack; everything else takes the gather kernel
-  if ((p.W & 3) == 0 && (reinterpret_cast<uintptr_t>(p.fields) & 15) == 0 && (((size_t)p.H * p.W) & 3) == 0) {
-    existence_kernel_tma<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
-    return (int)cudaGetLastError();
-  }
-#endif
   existence_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }

@@ -30,13 +30,8 @@ __device__ __forceinline__ uint32_t nz4(uint32_t w) {
 // current one, so the HBM pipe never drains between batches and there is no per-CTA launch / drain overhead (the
 // one-shot form reached 0.57 / 0.74 / 0.80 of the measured copy bandwidth at 1k / 4k / 16k masks; this form with 4
 // resident CTAs per SM: 0.79 / 0.88 / 0.94, where a plain device copy of the same bytes reaches 0.84 / 0.96 / 0.99).
-#ifndef UNMORE_PACK_UNROLL
-#define UNMORE_PACK_UNROLL 4
-#endif
-#ifndef UNMORE_PACK_CTAS_PER_SM
-#define UNMORE_PACK_CTAS_PER_SM 4   // measured: 2 / 3 / 4 / 5 / 8 CTAs per SM -> 0.82 / 0.92 / 0.94 / 0.91 / 0.87 of the copy bandwidth at 16k masks
-#endif
-constexpr int kPackUnroll = UNMORE_PACK_UNROLL;
+constexpr int kPackUnroll = 4;
+constexpr int kPackCtasPerSm = 4;   // measured: 2 / 3 / 4 / 5 / 8 CTAs per SM -> 0.82 / 0.92 / 0.94 / 0.91 / 0.87 of the copy bandwidth at 16k masks
 __global__ void __launch_bounds__(256) pack_kernel_vec(const uint4* __restrict__ in, uint32_t* __restrict__ out,
                                                        size_t n_vec) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;   // even: lane pairs stay together in every batch
@@ -85,7 +80,7 @@ int launch_mask_pack(const unsigned char* in, uint32_t* out, size_t n_masks, int
     const size_t n_vec = n_masks * H * (size_t)W / 16;
     const size_t per_block = 256 * (size_t)kPackUnroll;   // n_vec is even (W % 32 == 0), so lane pairs never straddle strides
     const size_t want = (n_vec + per_block - 1) / per_block;
-    const size_t resident = (size_t)num_sms * UNMORE_PACK_CTAS_PER_SM;
+    const size_t resident = (size_t)num_sms * kPackCtasPerSm;
     pack_kernel_vec<<<(unsigned)(want < resident ? want : resident), 256, 0, stream>>>(reinterpret_cast<const uint4*>(in), out, n_vec);
   } else {
     const size_t total = n_masks * H * (size_t)Wp;
@@ -423,7 +418,6 @@ int launch_rle_counts(const uint32_t* masks, int K, int H, int W, int max_runs, 
   if (K <= 0) return 0;
   const int Wp = (W + 31) >> 5, Hw = (H + 31) >> 5;
   const size_t smem_t = (size_t)W * Hw * sizeof(uint32_t), smem = smem_t + (size_t)H * (Wp | 1) * sizeof(uint32_t);
-#ifndef UNMORE_RLE_SERIAL
   // function attributes are per device: set on every launch (microseconds), no cached state
   if (smem <= (size_t)kRleMaxDynSmem) {
     cudaError_t e = cudaFuncSetAttribute(rle_counts_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -437,7 +431,6 @@ int launch_rle_counts(const uint32_t* masks, int K, int H, int W, int max_runs, 
     rle_counts_kernel<false><<<K, kRleThreads, smem_t, stream>>>(masks, K, H, W, Wp, max_runs, counts, n_runs);
     return (int)cudaGetLastError();
   }
-#endif
   rle_counts_kernel_serial<<<K, kRleThreads, 0, stream>>>(masks, K, H, W, Wp, max_runs, counts, n_runs);
   return (int)cudaGetLastError();
 }

@@ -255,12 +255,8 @@ __device__ __forceinline__ Deltas boundary_terms(RowSrc& src, BorderCols& cols, 
 // (published with a release store after the terms).  A warp that finds its window claimed waits a bounded
 // number of polls (sleeping, so the other warps of the SM get its issue slots), then computes the terms itself
 // without publishing; so does a warp whose probe path is full.  No warp waits on another without a limit.
-#ifndef UNMORE_WINDOW_PROBES
-#define UNMORE_WINDOW_PROBES 16
-#endif
-#ifndef UNMORE_WINDOW_WAIT_POLLS
-#define UNMORE_WINDOW_WAIT_POLLS 160   // 64 ns doubling to 1 us per poll: at most ~160 us of sleep
-#endif
+constexpr int kWindowProbes = 16;
+constexpr int kWindowWaitPolls = 160;   // 64 ns doubling to 1 us per poll: at most ~160 us of sleep
 constexpr unsigned long long kWindowReady = 1ull << 63;
 
 __device__ __forceinline__ unsigned long long window_key(const Window& w) {
@@ -279,7 +275,7 @@ __device__ __forceinline__ bool window_lookup(WindowSlot* table, const Window& w
   const unsigned long long key = window_key(win);
   const unsigned h = (unsigned)((key * 0x9E3779B97F4A7C15ull) >> 32);
   pub = -1;
-  for (int probe = 0; probe < UNMORE_WINDOW_PROBES; ++probe) {
+  for (int probe = 0; probe < kWindowProbes; ++probe) {
     const int i = (int)((h + probe) & (kWindowSlots - 1));
     WindowSlot* s = table + i;
     unsigned long long k = ld_acquire_key(s);
@@ -289,7 +285,7 @@ __device__ __forceinline__ bool window_lookup(WindowSlot* table, const Window& w
     }
     if ((k & ~kWindowReady) != key) continue;
     for (int poll = 0, ns = 64; !(k & kWindowReady); ++poll) {
-      if (poll == UNMORE_WINDOW_WAIT_POLLS) return false;
+      if (poll == kWindowWaitPolls) return false;
       __nanosleep(ns);
       ns = min(2 * ns, 1024);
       k = ld_acquire_key(s);
@@ -355,17 +351,11 @@ __device__ __forceinline__ int apply_update(const RefineParams& p, const Window&
   return label;
 }
 
-#ifndef UNMORE_REFINE_WARPS
-#define UNMORE_REFINE_WARPS 6
-#endif
-constexpr int kRefineWarps = UNMORE_REFINE_WARPS;
-
-#ifndef UNMORE_REFINE_MINBLOCKS
-#define UNMORE_REFINE_MINBLOCKS 3
-#endif
+constexpr int kRefineWarps = 6;
+constexpr int kRefineMinBlocks = 3;   // resident CTAs per SM, in __launch_bounds__ and in the grid of launch_refine
 constexpr int kSpecRowElems = 640;   // row pitch of the COCO-val-shaped fields the batch path runs on
 template <int ROW_ELEMS>
-__global__ void __launch_bounds__(kRefineWarps * 32, UNMORE_REFINE_MINBLOCKS) refine_kernel(const RefineParams p) {
+__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
   __shared__ BorderCols cols_all[kRefineWarps];
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
@@ -511,7 +501,7 @@ int launch_round_update(const RefineParams& p, const float4* deltas, const float
 }
 
 int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream) {
-  const int ctas = num_sms * UNMORE_REFINE_MINBLOCKS;  // resident CTAs per SM; warps pull proposals dynamically
+  const int ctas = num_sms * kRefineMinBlocks;  // warps pull proposals dynamically
   if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   else refine_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();

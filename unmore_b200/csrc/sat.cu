@@ -92,10 +92,7 @@ __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel(const float* __rest
 // registers, so a warp has 6 rows (15 KB at W=640) outstanding instead of one
 // (ring depth 3 / 4 / 6 / 8 measured: 4720 / 4699 / 5433 / 4387 GB/s at 3000 planes; 5-7 tie at 5950 GB/s at 8000).
 // Needs W % 4 == 0 (16-byte rows); launch_sat falls back to the register-fed kernel otherwise.
-#ifndef UNMORE_SAT_STAGES
-#define UNMORE_SAT_STAGES 6
-#endif
-constexpr int kSatStages = UNMORE_SAT_STAGES;
+constexpr int kSatStages = 6;
 
 template <int STEPS>
 __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel_tma(const float* __restrict__ in, double* __restrict__ out,
@@ -187,13 +184,11 @@ int launch_sat(const float* in, double* out, int n_planes, int H, int W, int C, 
   for (int i = 0; i < n_ch && i < 4; ++i) sel.ch[i] = channels[i];
   const int grid = (n_planes + kSatWarps - 1) / kSatWarps;
   const int steps = (W + 127) / 128;
-#ifndef UNMORE_SAT_NO_TMA
   // bulk-copy path: 16-byte aligned rows (W % 4 == 0; planes of a 16-byte aligned tensor then are too)
   if ((W & 3) == 0 && ((size_t)H * W & 3) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && steps <= 8) {
     if (steps <= 5) return launch_sat_tma<5>(in, out, n_planes, H, W, sel, grid, stream);
     return launch_sat_tma<8>(in, out, n_planes, H, W, sel, grid, stream);
   }
-#endif
   if (steps <= 5) sat_kernel<5><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel);
   else if (steps <= 8) sat_kernel<8><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel);
   else if (steps <= 16) sat_kernel<16><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel);

@@ -7,20 +7,12 @@
 
 namespace unmore {
 
-struct FieldDesc {
-  const float* data;  // [n_img, C, H, W] fp32 contiguous
-  int n_img, C, H, W;
-};
-
 // ---- refine.cu -----------------------------------------------------------------------
 // Per-image window cache of the fused refine kernel: the boundary terms of a crop window depend only on the
 // field plane and the snapped integer window, and proposals of one image converge onto the same windows.
 // One open-addressed table of kWindowSlots 32-byte slots per image, in the workspace (make_worklist).
-#ifndef UNMORE_WINDOW_SLOTS
-#define UNMORE_WINDOW_SLOTS 32768   // power of two; ~15k distinct windows per benchmark image at most
-#endif
-constexpr int kWindowSlots = UNMORE_WINDOW_SLOTS;
-static_assert((kWindowSlots & (kWindowSlots - 1)) == 0, "UNMORE_WINDOW_SLOTS must be a power of two");
+constexpr int kWindowSlots = 32768;   // ~15k distinct windows per benchmark image at most
+static_assert((kWindowSlots & (kWindowSlots - 1)) == 0, "kWindowSlots must be a power of two");
 constexpr int kWindowMaxSide = 32767;   // window corners are packed in 15 bits each; larger fields share nothing
 struct alignas(32) WindowSlot {
   unsigned long long key;   // 0 = empty; packed window, bit 63 set once the terms below are published
@@ -74,9 +66,7 @@ int launch_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, c
 int launch_mask_resize_aa(const unsigned char* masks, int B, int oh, int ow, unsigned char* out, float* scratch, cudaStream_t stream);
 
 // ---- center.cu -----------------------------------------------------------------------
-#ifndef UNMORE_CC_CAP
-#define UNMORE_CC_CAP 16   // connected-component boxes kept per proposal (--analyze_cc); overflow is counted
-#endif
+constexpr int kCcCap = 16;   // connected-component boxes kept per proposal (--analyze_cc); overflow is counted
 struct CenterParams {
   const float* tiles;   // nullable: pre-resampled [n_img * cap, 3, 128, 128] (sdf, center_row, center_col) instead of `fields`
   const float* fields;
@@ -96,8 +86,8 @@ struct CenterParams {
   unsigned long long filt_pair[25];
   // --analyze_cc (object_reasoning.py:561-572); all three null when off
   unsigned char* cc_counts;  // [n_img, cap] component boxes emitted (0 unless the proposal passes with >= 2 components)
-  double* cc_boxes;          // [n_img, cap, UNMORE_CC_CAP, 4] enlarged component boxes
-  int* cc_overflow;          // incremented once per proposal with more than UNMORE_CC_CAP components
+  double* cc_boxes;          // [n_img, cap, kCcCap, 4] enlarged component boxes
+  int* cc_overflow;          // incremented once per proposal with more than kCcCap components
 };
 int launch_center(const CenterParams& p, int num_sms, cudaStream_t stream);
 int launch_components(const unsigned char* masks, int B, int* counts, int* boxes, cudaStream_t stream);
@@ -142,7 +132,6 @@ struct NmsParams {
   int* keep_counts;      // [n_img]
   float4* boxes_out;     // nullable [n_img, cap] kept boxes, same order
   int* order_ws;         // [n_img, cap] workspace
-  unsigned char* alive_ws;  // [n_img, cap] workspace
 };
 int launch_box_nms(const NmsParams& p, cudaStream_t stream);
 
