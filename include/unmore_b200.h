@@ -66,8 +66,8 @@ int unmore_crop_resize(const float* fields, int n_img, int C, int H, int W,
  * what torchvision >= 0.17 makes of the reference's transforms.Resize calls (object_reasoning.py:319,407,505;
  * object_scoring.py:131,206,222) when the pinned 0.14.1 is not what is installed.  Bit-exact against torch 2.11
  * CPU (weights with ATen's float/double mix, horizontal pass first, its accumulation order).  The fused
- * kernels above implement antialias=False only; these produce the tiles for unmore_update_bbox_from_tiles and
- * for inspection.  `scratch`: n_img*cap*n_channels*H*128 floats (crop) / B*128*out_w floats (mask). */
+ * existence and refine kernels have antialiased forms (unmore_existence_scores_aa, unmore_boundary_refine_aa);
+ * these produce the tiles for the center and scoring stages, for unmore_update_bbox_from_tiles and for inspection.  `scratch`: n_img*cap*n_channels*H*128 floats (crop) / B*128*out_w floats (mask). */
 int unmore_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, const int* channels_host,
                           int n_channels, const void* boxes, int boxes_f64, const int* counts, int cap,
                           float* out, void* scratch, size_t scratch_bytes, unmore_stream_t stream);
@@ -136,6 +136,21 @@ int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, 
                            float max_sdf_thres, float max_shrink_threshold, float delta_ratio,
                            float* boxes_out, float* labels_out, int* rounds_out, void* ws,
                            unmore_stream_t stream);
+
+/* unmore_existence_scores and unmore_boundary_refine in the SECOND resize mode (antialias=True, see
+ * unmore_crop_resize_aa): same arguments, validation, workspace and outputs, with every crop resampled by ATen's
+ * antialiased kernel inside the fused kernels instead of materialised as a tile.  Bit-identical to the tile path:
+ * the existence score equals unmore_tile_means of the unmore_crop_resize_aa tile, and every refine round equals
+ * unmore_boundary_round_from_tiles on it (window cache, early exit and rounds_out as in the primary mode). */
+int unmore_existence_scores_aa(const float* fields, int n_img, int C, int H, int W, int ch_exist,
+                               const void* boxes, int boxes_f64, const int* counts, int cap,
+                               float* scores_out, void* ws, unmore_stream_t stream);
+int unmore_boundary_refine_aa(const float* fields, int n_img, int C, int H, int W, int ch_sdf,
+                              const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
+                              int apply_small_filter, int early_exit, float proposal_area_thres,
+                              float max_sdf_thres, float max_shrink_threshold, float delta_ratio,
+                              float* boxes_out, float* labels_out, int* rounds_out, void* ws,
+                              unmore_stream_t stream);
 
 /* update_bbox_with_boundary_fields — object_reasoning.py:140-174 on pre-resampled tiles
  * [M, 128, 128] fp32.  deltas_out [M, 4] = (delta_x1, delta_y1, delta_x2, delta_y2);

@@ -19,6 +19,7 @@ _d = C.c_double
 # name -> argtypes; every function returns int except where noted
 SIGNATURES = {
     "unmore_existence_scores": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _p, _p, _p],
+    "unmore_existence_scores_aa": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _p, _p, _p],
     "unmore_crop_resize": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _p, _p],
     "unmore_crop_resize_aa": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _p, _p, C.c_size_t, _p],
     "unmore_mask_resize_aa": [_p, _i, _i, _i, _i, _i, _p, _p, C.c_size_t, _p],
@@ -28,6 +29,7 @@ SIGNATURES = {
     "unmore_score_and_rasterise_from_tiles": [_p, _p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _p, _p, _p, _p],
     "unmore_center_reasoning": [_p, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
     "unmore_boundary_refine": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
+    "unmore_boundary_refine_aa": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
     "unmore_update_bbox_from_tiles": [_p, _i, _p, _p, _p],
     "unmore_compact_boxes": [_p, _i, _p, _i, _i, _i, _p, _f, _p, _i, _i, _p, _i, _p, _p, _p, _i, _p],
     "unmore_box_nms": [_p, _p, _p, _i, _i, _f, _p, _p, _p, _p, _p],

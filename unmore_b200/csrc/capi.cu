@@ -100,12 +100,54 @@ int check_fields(const float* f, int n_img, int C, int H, int W) {
   return 0;
 }
 
+// unmore_existence_scores / unmore_existence_scores_aa: the same call in either resize mode
+int existence_scores(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_exist,
+                     const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
+                     cudaStream_t s) {
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (!boxes || !scores_out || !ws || cap < 0 || ch_exist < 0 || ch_exist >= C)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (cap == 0) return 0;
+  ExistParams p{};
+  p.fields = fields; p.C = C; p.H = H; p.W = W; p.ch_exist = ch_exist;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.scores = scores_out;
+  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  if (aa) return cuda_fail(launch_existence_aa(p, num_sms(), s), "existence_aa_kernel");
+  return cuda_fail(launch_existence(p, num_sms(), s), "existence_kernel");
+}
+
+// unmore_boundary_refine / unmore_boundary_refine_aa
+int boundary_refine(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_sdf,
+                    const void* boxes, int boxes_f64, const int* counts, int cap, int n_round, int apply_small_filter,
+                    int early_exit, float proposal_area_thres, float max_sdf_thres, float max_shrink_threshold,
+                    float delta_ratio, float* boxes_out, float* labels_out, int* rounds_out, void* ws, cudaStream_t s) {
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (!boxes || !boxes_out || !labels_out || !ws || cap < 0 || n_round < 1 || ch_sdf < 0 || ch_sdf >= C)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (cap == 0) return 0;
+  RefineParams p{};
+  p.fields = fields; p.C = C; p.H = H; p.W = W; p.ch_sdf = ch_sdf;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64;
+  p.n_round = n_round; p.apply_small_filter = apply_small_filter; p.early_exit = early_exit;
+  p.area_thres = proposal_area_thres; p.max_sdf_thres = max_sdf_thres;
+  p.max_shrink_thres = max_shrink_threshold; p.delta_ratio = delta_ratio;
+  p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.labels_out = labels_out; p.rounds_out = rounds_out;
+  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  if (W <= kWindowMaxSide && H <= kWindowMaxSide) {
+    p.windows = window_tables(ws, n_img);
+    const int e = (int)cudaMemsetAsync(p.windows, 0, sizeof(WindowSlot) * kWindowSlots * (size_t)n_img, s);
+    if (e) return cuda_fail(e, "memset window tables");
+  }
+  if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s), "refine_aa_kernel");
+  return cuda_fail(launch_refine(p, num_sms(), s), "refine_kernel");
+}
+
 }  // namespace
 
 extern "C" {
 
 const char* unmore_last_error(void) { return g_err; }
-int unmore_version(void) { return 100; }
+int unmore_version(void) { return 101; }
 size_t unmore_workspace_bytes(int n_img) {
   // the alignment slack lets `ws` be any 4-byte aligned pointer
   return worklist_bytes(n_img) + (n_img > 0 ? alignof(WindowSlot) - 1 + sizeof(WindowSlot) * kWindowSlots * (size_t)n_img : 0);
@@ -114,16 +156,15 @@ size_t unmore_workspace_bytes(int n_img) {
 int unmore_existence_scores(const float* fields, int n_img, int C, int H, int W, int ch_exist, const void* boxes,
                             int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
                             unmore_stream_t stream) {
-  if (int e = check_fields(fields, n_img, C, H, W)) return e;
-  if (!boxes || !scores_out || !ws || cap < 0 || ch_exist < 0 || ch_exist >= C)
-    return fail(UNMORE_E_INVALID, "unmore_existence_scores: bad argument");
-  if (cap == 0) return 0;
-  cudaStream_t s = (cudaStream_t)stream;
-  ExistParams p{};
-  p.fields = fields; p.C = C; p.H = H; p.W = W; p.ch_exist = ch_exist;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.scores = scores_out;
-  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
-  return cuda_fail(launch_existence(p, num_sms(), s), "existence_kernel");
+  return existence_scores("unmore_existence_scores", false, fields, n_img, C, H, W, ch_exist, boxes, boxes_f64, counts, cap,
+                          scores_out, ws, (cudaStream_t)stream);
+}
+
+int unmore_existence_scores_aa(const float* fields, int n_img, int C, int H, int W, int ch_exist, const void* boxes,
+                               int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
+                               unmore_stream_t stream) {
+  return existence_scores("unmore_existence_scores_aa", true, fields, n_img, C, H, W, ch_exist, boxes, boxes_f64, counts, cap,
+                          scores_out, ws, (cudaStream_t)stream);
 }
 
 int unmore_crop_resize(const float* fields, int n_img, int C, int H, int W, const int* channels_host, int n_channels,
@@ -194,25 +235,19 @@ int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, 
                            int early_exit, float proposal_area_thres, float max_sdf_thres, float max_shrink_threshold,
                            float delta_ratio, float* boxes_out, float* labels_out, int* rounds_out, void* ws,
                            unmore_stream_t stream) {
-  if (int e = check_fields(fields, n_img, C, H, W)) return e;
-  if (!boxes || !boxes_out || !labels_out || !ws || cap < 0 || n_round < 1 || ch_sdf < 0 || ch_sdf >= C)
-    return fail(UNMORE_E_INVALID, "unmore_boundary_refine: bad argument");
-  if (cap == 0) return 0;
-  cudaStream_t s = (cudaStream_t)stream;
-  RefineParams p{};
-  p.fields = fields; p.C = C; p.H = H; p.W = W; p.ch_sdf = ch_sdf;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64;
-  p.n_round = n_round; p.apply_small_filter = apply_small_filter; p.early_exit = early_exit;
-  p.area_thres = proposal_area_thres; p.max_sdf_thres = max_sdf_thres;
-  p.max_shrink_thres = max_shrink_threshold; p.delta_ratio = delta_ratio;
-  p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.labels_out = labels_out; p.rounds_out = rounds_out;
-  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
-  if (W <= kWindowMaxSide && H <= kWindowMaxSide) {
-    p.windows = window_tables(ws, n_img);
-    const int e = (int)cudaMemsetAsync(p.windows, 0, sizeof(WindowSlot) * kWindowSlots * (size_t)n_img, s);
-    if (e) return cuda_fail(e, "memset window tables");
-  }
-  return cuda_fail(launch_refine(p, num_sms(), s), "refine_kernel");
+  return boundary_refine("unmore_boundary_refine", false, fields, n_img, C, H, W, ch_sdf, boxes, boxes_f64, counts, cap, n_round,
+                         apply_small_filter, early_exit, proposal_area_thres, max_sdf_thres, max_shrink_threshold,
+                         delta_ratio, boxes_out, labels_out, rounds_out, ws, (cudaStream_t)stream);
+}
+
+int unmore_boundary_refine_aa(const float* fields, int n_img, int C, int H, int W, int ch_sdf, const void* boxes,
+                              int boxes_f64, const int* counts, int cap, int n_round, int apply_small_filter,
+                              int early_exit, float proposal_area_thres, float max_sdf_thres, float max_shrink_threshold,
+                              float delta_ratio, float* boxes_out, float* labels_out, int* rounds_out, void* ws,
+                              unmore_stream_t stream) {
+  return boundary_refine("unmore_boundary_refine_aa", true, fields, n_img, C, H, W, ch_sdf, boxes, boxes_f64, counts, cap,
+                         n_round, apply_small_filter, early_exit, proposal_area_thres, max_sdf_thres, max_shrink_threshold,
+                         delta_ratio, boxes_out, labels_out, rounds_out, ws, (cudaStream_t)stream);
 }
 
 int unmore_update_bbox_from_tiles(const float* tiles, int M, float* deltas_out, float* max_out,

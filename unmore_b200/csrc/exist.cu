@@ -4,6 +4,7 @@
 //
 // One warp per proposal, lane owns 4 output columns; the horizontally interpolated source
 // rows are cached across output rows (resample.cuh), so small crops cost ~in_h row fetches.
+#include "aa_rows.cuh"
 #include "resample.cuh"
 #include "unmore_internal.h"
 
@@ -53,6 +54,50 @@ __global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const Exist
         vt.i0 = i0; vt.i1 = min(i0 + 1, in_h - 1);
         vt.l1 = __int_as_float(l1b); vt.l0 = __fsub_rn(1.f, vt.l1);
         plane.row2(taps, vt, v);
+        part = add2(part, add2(v[0], v[1]));
+        if ((i & 7) == 7) {
+          float lo, hi;
+          upk2(part, lo, hi);
+          acc += (double)(lo + hi);
+          part = pk2(0.f, 0.f);
+        }
+      }
+      acc = warp_sum(acc);
+      score = (float)(acc * (1.0 / (kCrop * kCrop)));
+    }
+    if (lane == 0) p.scores[row] = score;
+  }
+}
+
+// The second resize mode (antialias=True): the mean of the antialiased crop (aa_rows.cuh), summed in exactly the order
+// above, so the score equals tile_means_kernel on the tile of unmore_crop_resize_aa bit for bit.
+constexpr int kAaExistWarps = 2;   // 15 KB of shared memory per warp
+constexpr int kAaExistMinBlocks = 7;
+__global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_kernel(const ExistParams p) {
+  __shared__ AaRowsSmem rows_all[kAaExistWarps];
+  const int lane = threadIdx.x & 31;
+  AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
+  const int total = worklist_total(p.work);
+  int img = 0;
+  for (;;) {
+    const int id = worklist_next_warp(p.work);
+    if (id >= total) break;
+    int k;
+    worklist_locate(p.work, id, img, k);
+    const size_t row = (size_t)img * p.work.cap + k;
+    double x1, y1, x2, y2;
+    load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
+    const Window win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    float score = 0.f;
+    if (!win.empty()) {
+      AaCropRows src;
+      src.init(lane, rows, p.fields + ((size_t)img * p.C + p.ch_exist) * p.H * p.W, p.W, win);
+      double acc = 0.0;
+      f32x2 part = pk2(0.f, 0.f);
+      for (int i = 0; i < kCrop; ++i) {
+        f32x2 v[2];
+        src.issue(lane, i);
+        src.finish(v);
         part = add2(part, add2(v[0], v[1]));
         if ((i & 7) == 7) {
           float lo, hi;
@@ -160,6 +205,11 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream) {
   existence_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
+int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream) {
+  existence_aa_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

@@ -8,6 +8,7 @@
 // gradient averages, takes the four border maxima and applies the box update.  Proposals
 // are independent in the reference (no cross-proposal term anywhere in the loop), so the
 // per-round filter_small_proposal / boolean-mask compactions become per-proposal exits.
+#include "aa_rows.cuh"
 #include "resample.cuh"
 #include "unmore_internal.h"
 
@@ -354,11 +355,10 @@ __device__ __forceinline__ int apply_update(const RefineParams& p, const Window&
 constexpr int kRefineWarps = 6;
 constexpr int kRefineMinBlocks = 3;   // resident CTAs per SM, in __launch_bounds__ and in the grid of launch_refine
 constexpr int kSpecRowElems = 640;   // row pitch of the COCO-val-shaped fields the batch path runs on
-template <int ROW_ELEMS>
-__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
-  __shared__ BorderCols cols_all[kRefineWarps];
-  const int lane = threadIdx.x & 31;
-  BorderCols& cols = cols_all[threadIdx.x >> 5];
+// The persistent round loop: warps pull proposals from the worklist until it is empty.  `terms(plane, win)` computes
+// the boundary terms of a window from its resampled rows; the resize mode only changes where those rows come from.
+template <class Terms>
+__device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCols& cols, int lane, Terms terms) {
   const int total = worklist_total(p.work);
   int img = 0;   // image of the previous work item: the locate hint
   for (;;) {
@@ -403,11 +403,7 @@ __global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_ke
       if (p.windows && lane == 0 && !win.empty()) hit = window_lookup(p.windows + (size_t)img * kWindowSlots, win, d, cols.pub);
       hit = __shfl_sync(kFullMask, hit, 0);
       if (!win.empty() && !hit) {
-        CropRows<ROW_ELEMS> src;
-        src.taps.template init<kStrided>(lane, win.w());
-        src.plane.init(plane, p.W, win);
-        src.init_rows(lane, cols.tapy, win.h());
-        d = boundary_terms(src, cols, lane);
+        d = terms(plane, win);
         if (p.windows && lane == 0 && cols.pub >= 0) window_publish(p.windows + (size_t)img * kWindowSlots + cols.pub, win, d);
       }
       if (hit) {
@@ -452,6 +448,37 @@ __global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_ke
       if (p.rounds_out) p.rounds_out[row] = rounds;
     }
   }
+}
+
+template <int ROW_ELEMS>
+__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
+  __shared__ BorderCols cols_all[kRefineWarps];
+  const int lane = threadIdx.x & 31;
+  BorderCols& cols = cols_all[threadIdx.x >> 5];
+  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
+    CropRows<ROW_ELEMS> src;
+    src.taps.template init<kStrided>(lane, win.w());
+    src.plane.init(plane, p.W, win);
+    src.init_rows(lane, cols.tapy, win.h());
+    return boundary_terms(src, cols, lane);
+  });
+}
+
+// The second resize mode: the same round loop on antialiased rows (aa_rows.cuh).  A warp needs 15 KB more shared
+// memory for the weight table and the row ring, so fewer warps fit an SM.
+constexpr int kAaRefineWarps = 2;
+constexpr int kAaRefineMinBlocks = 5;
+__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_kernel(const RefineParams p) {
+  __shared__ BorderCols cols_all[kAaRefineWarps];
+  __shared__ AaRowsSmem rows_all[kAaRefineWarps];
+  const int lane = threadIdx.x & 31;
+  BorderCols& cols = cols_all[threadIdx.x >> 5];
+  AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
+  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
+    AaCropRows src;
+    src.init(lane, rows, plane, p.W, win);
+    return boundary_terms(src, cols, lane);
+  });
 }
 
 __global__ void __launch_bounds__(kRefineWarps * 32) tiles_kernel(const TileParams p) {
@@ -504,6 +531,11 @@ int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream) {
   const int ctas = num_sms * kRefineMinBlocks;  // warps pull proposals dynamically
   if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   else refine_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream) {
+  refine_aa_kernel<<<num_sms * kAaRefineMinBlocks, kAaRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

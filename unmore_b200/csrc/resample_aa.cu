@@ -1,7 +1,7 @@
 // The second resize mode: antialias=True, i.e. ATen's _upsample_bilinear2d_aa — what torchvision >= 0.17 gives
 // transforms.Resize by default at object_reasoning.py:319,407,505 and object_scoring.py:131,206,222 (the reference
 // pins torchvision 0.14.1, where tensors are never antialiased; antialias=False is this repo's primary mode and the
-// one the fused kernels implement).  Provided for the stand-alone ops a2 (crop + resize to 128x128) and N2 (mask
+// mode of most fused kernels).  Provided for the stand-alone ops a2 (crop + resize to 128x128) and N2 (mask
 // resize back to the box + round half to even), bit-exact against torch 2.11 CPU:
 //
 //   * weights (HelperInterpBase::_compute_indices_min_size_weights_aa, opmath = float, double literals):
@@ -14,8 +14,8 @@
 //     oracle/oracle.py::_aa_pass): t = s0*w0; then groups of four taps with separate multiply and add; the
 //     remaining (n-1) mod 4 taps with a fused multiply-add.
 //
-// Two kernels with the intermediate in a caller-provided scratch buffer: this is the tile path (tiles for the
-// *_from_tiles stages), not the fused hot path.
+// Two kernels with the intermediate in a caller-provided scratch buffer: tiles for the *_from_tiles stages.  The fused
+// existence and refine kernels compute the same values row by row (aa_rows.cuh).
 #include "resample_aa.cuh"
 #include "unmore_internal.h"
 
@@ -32,30 +32,6 @@ struct AaCropParams {
   float* out;      // [n_img, cap, n_ch, 128, 128]
   float* scratch;  // [n_img * cap * n_ch, H, 128]
 };
-
-// Weights of one output index, normalised exactly as aa_dot does (sequential fp32 sum, then r / total).
-__device__ __forceinline__ void aa_weights(const AaAxis& a, int i, int& xmin, int& n, float* w, int stride, int max_taps) {
-  float center;
-  a.span(i, center, xmin, n);
-  if (n <= 0 || n > max_taps) return;
-  float total = 0.f;
-  for (int k = 0; k < n; ++k) total = __fadd_rn(total, a.raw_weight(xmin + k, center));
-  for (int k = 0; k < n; ++k) {
-    const float r = a.raw_weight(xmin + k, center);
-    w[k * stride] = total != 0.f ? __fdiv_rn(r, total) : r;
-  }
-}
-// aa_dot's accumulation order over a weight table: first tap a product, groups of four with separate multiply and
-// add, the remaining (n-1) mod 4 fused
-template <class Src, class Wt>
-__device__ __forceinline__ float aa_accumulate(int n, Src src, Wt w) {
-  float t = __fmul_rn(src(0), w(0));
-  const int main_taps = ((n - 1) / 4) * 4;
-  int k = 1;
-  for (; k <= main_taps; ++k) t = __fadd_rn(t, __fmul_rn(src(k), w(k)));
-  for (; k < n; ++k) t = __fmaf_rn(src(k), w(k), t);
-  return t;
-}
 
 // Two passes with the intermediate in the caller's scratch buffer, grid = (tile, 8 row slices): the weight tables of
 // a block (the fp64 / division part: ~90% of the instructions of a dot) are built once in shared memory — thread j

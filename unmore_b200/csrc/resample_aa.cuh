@@ -1,5 +1,6 @@
 // Weights and accumulation order of ATen's antialiased bilinear kernel (_upsample_bilinear2d_aa), shared by the
-// stand-alone antialias ops (resample_aa.cu) and the antialiased mask rasteriser of the scoring kernel (score.cu).
+// stand-alone antialias ops (resample_aa.cu), the antialiased mask rasteriser of the scoring kernel (score.cu) and the
+// antialiased row source of the fused existence and refine kernels (aa_rows.cuh).
 // See resample_aa.cu for the arithmetic contract; pinned by oracle/oracle.py::aa_index_weights / _aa_pass.
 #pragma once
 #include "common.cuh"
@@ -47,6 +48,30 @@ __device__ __forceinline__ float aa_dot(const AaAxis& a, int i, Src src) {
   int j = 1;
   for (; j <= main_taps; ++j) t = __fadd_rn(t, __fmul_rn(src(xmin + j), w(j)));
   for (; j < n; ++j) t = __fmaf_rn(src(xmin + j), w(j), t);
+  return t;
+}
+
+// Weights of one output index, normalised exactly as aa_dot does (sequential fp32 sum, then r / total).
+__device__ __forceinline__ void aa_weights(const AaAxis& a, int i, int& xmin, int& n, float* w, int stride, int max_taps) {
+  float center;
+  a.span(i, center, xmin, n);
+  if (n <= 0 || n > max_taps) return;
+  float total = 0.f;
+  for (int k = 0; k < n; ++k) total = __fadd_rn(total, a.raw_weight(xmin + k, center));
+  for (int k = 0; k < n; ++k) {
+    const float r = a.raw_weight(xmin + k, center);
+    w[k * stride] = total != 0.f ? __fdiv_rn(r, total) : r;
+  }
+}
+// aa_dot's accumulation order over a weight table: first tap a product, groups of four with separate multiply and
+// add, the remaining (n-1) mod 4 fused
+template <class Src, class Wt>
+__device__ __forceinline__ float aa_accumulate(int n, Src src, Wt w) {
+  float t = __fmul_rn(src(0), w(0));
+  const int main_taps = ((n - 1) / 4) * 4;
+  int k = 1;
+  for (; k <= main_taps; ++k) t = __fadd_rn(t, __fmul_rn(src(k), w(k)));
+  for (; k < n; ++k) t = __fmaf_rn(src(k), w(k), t);
   return t;
 }
 

@@ -43,6 +43,7 @@ struct TileParams {
   float* max_sdf;      // [M] or nullptr
 };
 int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream);
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
 int launch_tiles(const TileParams& p, cudaStream_t stream);
 int launch_round_update(const RefineParams& p, const float4* deltas, const float* max_sdf, int M, cudaStream_t stream);
 
@@ -56,6 +57,7 @@ struct ExistParams {
   float* scores;  // [n_img, cap]
 };
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream);
+int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
 int launch_tile_means(const float* tiles, long long tile_stride, int M, float* out, cudaStream_t stream);
 int launch_crop_resize(const float* fields, int n_img, int C, int H, int W, const int* channels, int n_ch,
                        const void* boxes, int boxes_f64, const int* counts, int cap, float* out, cudaStream_t stream);

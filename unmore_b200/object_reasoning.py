@@ -85,9 +85,8 @@ class Object_Discovery:
         self.width = None
         self.test_dataset = test_dataset
         self.result_folder = result_folder
-        # resize mode of the STAND-ALONE tile ops (get_prediction_with_proposals): False = torchvision 0.14.1
-        # semantics (what the reference pins and the fused kernels implement), True = ATen's antialiased kernel
-        # (torchvision >= 0.17's default).  args.antialias, when present, sets it.
+        # resize mode: False = torchvision 0.14.1 semantics (what the reference pins), True = ATen's antialiased kernel
+        # (torchvision >= 0.17's default).  Both run batched on the device.  args.antialias, when present, sets it.
         self.antialias = bool(getattr(self.args, "antialias", False))
         # the reference's ORIGINAL mode: nets on every crop (producer.PerCropNets).  ``image`` is then the RGB image and
         # every stage runs on the tiles the provider makes (the tile path), in the provider's resize mode.
@@ -141,15 +140,12 @@ class Object_Discovery:
 
     @property
     def _tile_path(self) -> bool:
-        return self.antialias or self.tile_provider is not None
+        """Per-crop nets (a tile provider) run every stage on the provider's tiles, image by image."""
+        return self.tile_provider is not None
 
     def _field_tiles(self, f: torch.Tensor, boxes: torch.Tensor) -> torch.Tensor:
-        """[1,K,3,128,128] (sdf, center_row, center_col) tiles of ``boxes`` [1,K,4]: per-crop nets when a tile provider
-        is set, else antialiased crops of the per-image field stack."""
-        if self.tile_provider is not None:
-            return self.tile_provider.fields(f[0], boxes[0])[None]
-        ch = self.channels
-        return ops.crop_resize(f, boxes, [ch.sdf, ch.center_row, ch.center_col], antialias=True)
+        """[1,K,3,128,128] (sdf, center_row, center_col) tiles of ``boxes`` [1,K,4] from the tile provider."""
+        return self.tile_provider.fields(f[0], boxes[0])[None]
 
     # ---- a3 ---------------------------------------------------------------------------
     def existence_checking(self, image, proposals) -> Dict[str, torch.Tensor]:
@@ -159,10 +155,7 @@ class Object_Discovery:
             return {"existence_scores": torch.zeros((0,), dtype=torch.float32)}
         if self.tile_provider is not None:   # the reference's original mode: one classifier output per crop
             return {"existence_scores": self.tile_provider.existence(self._fields(image)[0], boxes[0]).cpu()}
-        if self.antialias:   # tile path: antialiased crops of the existence channel, then their means
-            tiles = ops.crop_resize(self._fields(image), boxes, [self.channels.exist], antialias=True)
-            return {"existence_scores": ops.tile_means(tiles[0, :, 0]).cpu()}
-        scores = ops.existence_scores(self._fields(image), boxes, ch=self.channels)
+        scores = ops.existence_scores(self._fields(image), boxes, ch=self.channels, antialias=self.antialias)
         return {"existence_scores": scores[0].cpu()}
 
     # ---- a4 ---------------------------------------------------------------------------
@@ -193,7 +186,7 @@ class Object_Discovery:
                                                                     thr=self.args.center_score_max_thres, analyze_cc=cc_on)
         else:
             _, argmax, splits, cc = ops.center_reasoning(self._fields(image), boxes, thr=self.args.center_score_max_thres,
-                                                         ch=self.channels, analyze_cc=cc_on)
+                                                         ch=self.channels, analyze_cc=cc_on, antialias=self.antialias)
         fail = argmax[0] >= 0
         new = splits[0][fail].reshape(-1, 4)
         if cc_on:
@@ -322,7 +315,7 @@ class Object_Discovery:
         out, lab, _ = ops.boundary_refine(self._fields(image), boxes, n_round=1, apply_small_filter=False,
                                           early_exit=False, proposal_area_thres=a.proposal_area_thres,
                                           max_sdf_thres=a.max_sdf_thres, max_shrink_threshold=a.max_shrink_threshold,
-                                          delta_ratio=a.delta_ratio, ch=self.channels)
+                                          delta_ratio=a.delta_ratio, ch=self.channels, antialias=self.antialias)
         return {"updated_bboxes": out[0], "labels": lab[0]}
 
     # ---- a13 --------------------------------------------------------------------------
@@ -339,22 +332,23 @@ class Object_Discovery:
         out, lab, _ = ops.boundary_refine(self._fields(image), boxes, n_round=a.n_round, apply_small_filter=True,
                                           early_exit=True, proposal_area_thres=a.proposal_area_thres,
                                           max_sdf_thres=a.max_sdf_thres, max_shrink_threshold=a.max_shrink_threshold,
-                                          delta_ratio=a.delta_ratio, ch=self.channels)
+                                          delta_ratio=a.delta_ratio, ch=self.channels, antialias=self.antialias)
         in_list = lab[0] > -2
         if int(in_list.sum()) == 0:
             return {"proposals": [], "labels": []}
         return {"proposals": out[0][in_list], "labels": lab[0][in_list]}
 
     def _sdf_tiles(self, f: torch.Tensor, boxes: torch.Tensor) -> torch.Tensor:
-        """[K,128,128] boundary-distance tiles of ``boxes`` [K,4] on the tile path."""
+        """[K,128,128] boundary-distance tiles of ``boxes`` [K,4]: the tile provider's, else antialiased crops (the
+        tile-by-tile form of the second resize mode, kept as the reference of the fused antialiased refine)."""
         if self.tile_provider is not None:
             return self.tile_provider.fields(f[0], boxes)[:, 0].contiguous()
         return ops.crop_resize(f, boxes[None].contiguous(), [self.channels.sdf], antialias=True)[0, :, 0]
 
     def _boundary_reasoning_tiles(self, f: torch.Tensor, cur: torch.Tensor):
-        """boundary_reasoning (object_reasoning.py:582-612) in the second resize mode: the round loop runs on the
-        host like the reference's, every round is crop (antialiased) -> tiles -> tile reductions -> box update on the
-        device.  Rows that reached label 1 with an unchanged box are exact fixed points and are not recomputed."""
+        """boundary_reasoning (object_reasoning.py:582-612) on tiles: the round loop runs on the host like the
+        reference's, every round is crop (the tile provider's, else antialiased) -> tiles -> tile reductions -> box
+        update on the device.  Rows that reached label 1 with an unchanged box are exact fixed points and are not recomputed."""
         a = self.args
         H, W = f.shape[-2], f.shape[-1]
         labels = torch.zeros((cur.shape[0],), dtype=torch.float32, device=self.device)
@@ -398,7 +392,7 @@ class Object_Discovery:
         return det[0, : int(cnt[0])].cpu().numpy()
 
     def _discover_image_tiles(self, image: torch.Tensor, proposals: torch.Tensor) -> np.ndarray:
-        """The loop body of main_object_discovery (:623-662) in the second resize mode, stage by stage through the
+        """The loop body of main_object_discovery (:623-662) with per-crop nets, stage by stage through the
         reference-named methods (each one on the tile path); empty intermediate lists end the image like the
         reference's ``continue``s (and an empty split list is 'no splits' instead of the reference's crash)."""
         a = self.args
@@ -440,7 +434,7 @@ class Object_Discovery:
         B, N = proposals.shape[0], proposals.shape[1]
         dev = fields.device
         f64 = torch.float64
-        if self._tile_path:   # second resize mode / per-crop nets: image by image on the tile path (not the fused kernels)
+        if self._tile_path:   # per-crop nets: image by image on the tile path (not the fused kernels)
             dets = [self._discover_image_tiles(fields[b], proposals[b] if counts is None else proposals[b, : int(counts[b])])
                     for b in range(B)]
             cap = max([len(d) for d in dets] + [1])
@@ -452,12 +446,13 @@ class Object_Discovery:
             return kb, kc
         ws = ops.workspace(B, dev)
         # Step 1: existence checking (:627-630)
-        ex = ops.existence_scores(fields, proposals, counts, ch=ch, ws=ws)
+        aa = self.antialias
+        ex = ops.existence_scores(fields, proposals, counts, ch=ch, ws=ws, antialias=aa)
         p1, c1, _ = ops.compact_boxes(proposals, counts, ops.MODE_SCORE_GE, ex, thr=a.class_score_thres, out_dtype=f64)
         # Step 2: center reasoning (:634-637)
         cc_on = bool(getattr(a, "analyze_cc", False))
         _, am1, sp1, cc = ops.center_reasoning(fields, p1, c1, thr=a.center_score_max_thres, ch=ch, ws=ws,
-                                               analyze_cc=cc_on)
+                                               analyze_cc=cc_on, antialias=aa)
         # 4 split boxes per failing proposal; with --analyze_cc the component boxes of passing proposals follow
         # (a speckled mask can carry dozens: the reference has no limit, here the list holds 4N + 4N + 256 rows)
         split_cap = 8 * N + 256 if cc_on else 4 * N
@@ -492,16 +487,17 @@ class Object_Discovery:
                     split[b, n_split:n_split + len(extra)] = torch.as_tensor(extra, device=dev)
                     sc[b] = n_split + len(extra)
         # re-check the split proposals (:639-646)
-        ex2 = ops.existence_scores(fields, split, sc, ch=ch, ws=ws)
+        ex2 = ops.existence_scores(fields, split, sc, ch=ch, ws=ws, antialias=aa)
         p2, c2, _ = ops.compact_boxes(split, sc, ops.MODE_SCORE_GE, ex2, thr=a.class_score_thres, out_dtype=f64)
-        _, am2, _, _ = ops.center_reasoning(fields, p2, c2, thr=a.center_score_max_thres, ch=ch, ws=ws, want_splits=False)
+        _, am2, _, _ = ops.center_reasoning(fields, p2, c2, thr=a.center_score_max_thres, ch=ch, ws=ws, want_splits=False,
+                                            antialias=aa)
         ops.compact_boxes(p2, c2, ops.MODE_ARGMAX_LT0, am2, out=refine_in, counts_out=rc, append=True)
         # Step 3: boundary reasoning (:650-658)
         rb, lab, rounds = ops.boundary_refine(fields, refine_in, rc, n_round=a.n_round, apply_small_filter=True,
                                               early_exit=True, proposal_area_thres=a.proposal_area_thres,
                                               max_sdf_thres=a.max_sdf_thres,
                                               max_shrink_threshold=a.max_shrink_threshold, delta_ratio=a.delta_ratio,
-                                              ch=ch, ws=ws, want_rounds=stats is not None)
+                                              ch=ch, ws=ws, want_rounds=stats is not None, antialias=aa)
         # label-1 survivors; the NMS kernel holds its alive set for at most 32768 boxes per image
         lost1 = torch.zeros((1,), dtype=torch.int32, device=dev) if cap_out > 32768 else None
         fin, fc, _ = ops.compact_boxes(rb, rc, ops.MODE_LABEL_EQ, lab, thr=1.0, out_dtype=torch.float32,
