@@ -287,6 +287,42 @@ int unmore_mask_nms(const uint32_t* masks, int K, int H, int W, const float* sco
                     const int* tight, float iou_threshold, int* order_ws, void* matrix_ws,
                     int* keep_out, int* keep_count_out, unmore_stream_t stream);
 
+/* ---- Images of different sizes in one call ----------------------------------------------------------------------
+ * A padded stack: fields [n_img, C, H, W] where (H, W) is the PITCH (the largest image), and image_hw [n_img, 2] int32
+ * in DEVICE memory of the current device (8-byte aligned) holding (h_i, w_i), 1 <= h_i <= H, 1 <= w_i <= W.  Image i is
+ * fields[i, :, :h_i, :w_i]; the padding may hold anything and no result depends on it.  Every address comes from the
+ * pitch, every use of the image size (window snap, edge tests, clips) from (h_i, w_i); the kernels clamp the extents to
+ * [1, pitch], so a bad table gives wrong numbers, never an out-of-range access.  Each call takes the arguments of its
+ * uniform counterpart with image_hw after W, and gives every image exactly what the uniform call gives it alone.
+ * Masks of unmore_score_and_rasterise_hw stay on the pitched canvas [n_img, cap, H, ceil(W/32)]: image i's are the
+ * [:h_i, :ceil(w_i/32)] corner, every bit outside the image is 0.  unmore_sat_build_fields_hw reads the padding as
+ * zeros, so entries [:h_i+1, :w_i+1] of image i's tables are those of the image alone; unmore_box_sums_hw takes such
+ * tables.  A null, misaligned, host or other-device image_hw is rejected (UNMORE_E_INVALID) before anything runs. */
+int unmore_existence_scores_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_exist,
+                               const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out,
+                               void* ws, unmore_stream_t stream);
+int unmore_center_reasoning_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                               int ch_center_row, int ch_center_col, const void* boxes, int boxes_f64,
+                               const int* counts, int cap, double center_score_max_thres, double* max_values_out,
+                               int* argmax_out, double* splits_out, unsigned char* cc_counts_out,
+                               double* cc_boxes_out, int* cc_overflow, void* ws, unmore_stream_t stream);
+int unmore_boundary_refine_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                              const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
+                              int apply_small_filter, int early_exit, float proposal_area_thres,
+                              float max_sdf_thres, float max_shrink_threshold, float delta_ratio,
+                              float* boxes_out, float* labels_out, int* rounds_out, void* ws,
+                              unmore_stream_t stream);
+int unmore_score_and_rasterise_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                                  int ch_sdf, int ch_center_row, int ch_center_col, int ch_exist,
+                                  const void* boxes, int boxes_f64, const int* counts, int cap,
+                                  float* scores_out, float* tight_out, int* areas_out, uint32_t* masks_out,
+                                  unmore_stream_t stream);
+int unmore_box_sums_hw(const double* sat, int n_img, int planes_per_img, int plane, int H, int W,
+                       const int* image_hw, const void* boxes, int boxes_f64, const int* counts, int cap,
+                       double* sums_out, double* means_out, unmore_stream_t stream);
+int unmore_sat_build_fields_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                               const int* channels_host, int n_channels, double* out, unmore_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -48,6 +48,13 @@ SIGNATURES = {
     "unmore_mask_stats": [_p, _i, _i, _i, _p, _p, _p],
     "unmore_mask_rle_counts": [_p, _i, _i, _i, _i, _p, _p, _p],
     "unmore_mask_nms": [_p, _i, _i, _i, _p, _p, _p, _f, _p, _p, _p, _p, _p],
+    # padded stacks of images of different sizes: H, W are the pitch, the pointer after W is image_hw [n_img, 2]
+    "unmore_existence_scores_hw": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _p, _p, _p],
+    "unmore_center_reasoning_hw": [_p, _i, _i, _i, _i, _p, _i, _i, _i, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
+    "unmore_boundary_refine_hw": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
+    "unmore_score_and_rasterise_hw": [_p, _i, _i, _i, _i, _p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _p, _p, _p, _p],
+    "unmore_box_sums_hw": [_p, _i, _i, _i, _i, _i, _p, _p, _i, _p, _i, _p, _p, _p],
+    "unmore_sat_build_fields_hw": [_p, _i, _i, _i, _i, _p, _p, _i, _p, _p],
 }
 
 _lib = None

@@ -100,27 +100,46 @@ int check_fields(const float* f, int n_img, int C, int H, int W) {
   return 0;
 }
 
-// unmore_existence_scores / unmore_existence_scores_aa: the same call in either resize mode
+// The (h, w) table of a padded field stack (the *_hw entry points): the kernels read it, so it must be device memory
+// of the current device, and 8-byte aligned (one int2 per image).  Host memory dereferenced in a kernel faults.
+int check_extents(const char* name, const int* image_hw) {
+  if (!image_hw) return fail(UNMORE_E_INVALID, "%s: image_hw is null", name);
+  if (reinterpret_cast<uintptr_t>(image_hw) & 7) return fail(UNMORE_E_INVALID, "%s: image_hw must be 8-byte aligned", name);
+  cudaPointerAttributes attr;
+  int dev = -1;
+  if (cudaPointerGetAttributes(&attr, image_hw) == cudaSuccess) {
+    if (attr.type == cudaMemoryTypeHost || attr.type == cudaMemoryTypeUnregistered)
+      return fail(UNMORE_E_INVALID, "%s: image_hw is host memory (it must be a device tensor)", name);
+    if (attr.type == cudaMemoryTypeDevice && cudaGetDevice(&dev) == cudaSuccess && attr.device != dev)
+      return fail(UNMORE_E_INVALID, "%s: image_hw lives on device %d but the current device is %d", name, attr.device, dev);
+  }
+  (void)cudaGetLastError();
+  return 0;
+}
+
+// unmore_existence_scores / unmore_existence_scores_aa / unmore_existence_scores_hw: the same call in either resize
+// mode, and on a padded stack (image_hw non-null)
 int existence_scores(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_exist,
                      const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
-                     cudaStream_t s) {
+                     cudaStream_t s, const int* image_hw = nullptr) {
   if (int e = check_fields(fields, n_img, C, H, W)) return e;
   if (!boxes || !scores_out || !ws || cap < 0 || ch_exist < 0 || ch_exist >= C)
     return fail(UNMORE_E_INVALID, "%s: bad argument", name);
   if (cap == 0) return 0;
   ExistParams p{};
   p.fields = fields; p.C = C; p.H = H; p.W = W; p.ch_exist = ch_exist;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.scores = scores_out;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.scores = scores_out; p.image_hw = image_hw;
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
   if (aa) return cuda_fail(launch_existence_aa(p, num_sms(), s), "existence_aa_kernel");
   return cuda_fail(launch_existence(p, num_sms(), s), "existence_kernel");
 }
 
-// unmore_boundary_refine / unmore_boundary_refine_aa
+// unmore_boundary_refine / unmore_boundary_refine_aa / unmore_boundary_refine_hw
 int boundary_refine(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_sdf,
                     const void* boxes, int boxes_f64, const int* counts, int cap, int n_round, int apply_small_filter,
                     int early_exit, float proposal_area_thres, float max_sdf_thres, float max_shrink_threshold,
-                    float delta_ratio, float* boxes_out, float* labels_out, int* rounds_out, void* ws, cudaStream_t s) {
+                    float delta_ratio, float* boxes_out, float* labels_out, int* rounds_out, void* ws, cudaStream_t s,
+                    const int* image_hw = nullptr) {
   if (int e = check_fields(fields, n_img, C, H, W)) return e;
   if (!boxes || !boxes_out || !labels_out || !ws || cap < 0 || n_round < 1 || ch_sdf < 0 || ch_sdf >= C)
     return fail(UNMORE_E_INVALID, "%s: bad argument", name);
@@ -139,7 +158,63 @@ int boundary_refine(const char* name, bool aa, const float* fields, int n_img, i
     if (e) return cuda_fail(e, "memset window tables");
   }
   if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s), "refine_aa_kernel");
-  return cuda_fail(launch_refine(p, num_sms(), s), "refine_kernel");
+  return cuda_fail(launch_refine(p, num_sms(), s, image_hw), "refine_kernel");
+}
+
+// unmore_center_reasoning / unmore_center_reasoning_hw
+int center_reasoning(const char* name, const float* fields, int n_img, int C, int H, int W, int ch_sdf, int ch_center_row,
+                     int ch_center_col, const void* boxes, int boxes_f64, const int* counts, int cap,
+                     double center_score_max_thres, double* max_values_out, int* argmax_out, double* splits_out,
+                     unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow, void* ws, cudaStream_t s,
+                     const int* image_hw = nullptr) {
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (!boxes || !max_values_out || !argmax_out || !ws || cap < 0 || ch_sdf < 0 || ch_sdf >= C || ch_center_row < 0 ||
+      ch_center_row >= C || ch_center_col < 0 || ch_center_col >= C)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (cap == 0) return 0;
+  CenterParams p{};
+  p.fields = fields; p.C = C; p.H = H; p.W = W;
+  p.ch_sdf = ch_sdf; p.ch_crow = ch_center_row; p.ch_ccol = ch_center_col;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.thr = center_score_max_thres;
+  p.max_values = max_values_out; p.argmax = argmax_out; p.splits = splits_out;
+  if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
+    return fail(UNMORE_E_INVALID, "%s: the three analyze_cc outputs go together", name);
+  p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
+  p.image_hw = image_hw;
+  center_filters(p);
+  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  return cuda_fail(launch_center(p, num_sms(), s), "center_kernel");
+}
+
+// unmore_score_and_rasterise / unmore_score_and_rasterise_hw
+int score_and_rasterise(const char* name, const float* fields, int n_img, int C, int H, int W, int ch_sdf, int ch_center_row,
+                        int ch_center_col, int ch_exist, const void* boxes, int boxes_f64, const int* counts, int cap,
+                        float* scores_out, float* tight_out, int* areas_out, uint32_t* masks_out, cudaStream_t s,
+                        const int* image_hw = nullptr) {
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (!boxes || !scores_out || !tight_out || !areas_out || cap < 0 || ch_sdf < 0 || ch_sdf >= C || ch_center_row < 0 ||
+      ch_center_row >= C || ch_center_col < 0 || ch_center_col >= C || ch_exist < 0 || ch_exist >= C)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (n_img > 65535) return fail(UNMORE_E_CAPACITY, "%s: n_img > 65535 per call", name);
+  ScoreParams p{};
+  p.fields = fields; p.n_img = n_img; p.C = C; p.H = H; p.W = W;
+  p.ch_sdf = ch_sdf; p.ch_crow = ch_center_row; p.ch_ccol = ch_center_col; p.ch_exist = ch_exist;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
+  p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
+  p.areas = areas_out; p.masks = masks_out;
+  return cuda_fail(launch_score(p, s, image_hw), "score_kernel");
+}
+
+// unmore_box_sums / unmore_box_sums_hw
+int box_sums(const char* name, const double* sat, int n_img, int planes_per_img, int plane, int H, int W, const void* boxes,
+             int boxes_f64, const int* counts, int cap, double* sums_out, double* means_out, cudaStream_t s,
+             const int* image_hw = nullptr) {
+  if (!sat || !boxes || !sums_out || n_img < 0 || cap < 0 || plane < 0 || plane >= planes_per_img ||
+      (image_hw && (H <= 0 || W <= 0)))
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  return cuda_fail(launch_box_sums(sat, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap, n_img, sums_out,
+                                   means_out, image_hw, s),
+                   "box_sums_kernel");
 }
 
 }  // namespace
@@ -147,7 +222,7 @@ int boundary_refine(const char* name, bool aa, const float* fields, int n_img, i
 extern "C" {
 
 const char* unmore_last_error(void) { return g_err; }
-int unmore_version(void) { return 101; }
+int unmore_version(void) { return 102; }
 size_t unmore_workspace_bytes(int n_img) {
   // the alignment slack lets `ws` be any 4-byte aligned pointer
   return worklist_bytes(n_img) + (n_img > 0 ? alignof(WindowSlot) - 1 + sizeof(WindowSlot) * kWindowSlots * (size_t)n_img : 0);
@@ -211,23 +286,9 @@ int unmore_center_reasoning(const float* fields, int n_img, int C, int H, int W,
                             double center_score_max_thres, double* max_values_out, int* argmax_out,
                             double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow,
                             void* ws, unmore_stream_t stream) {
-  if (int e = check_fields(fields, n_img, C, H, W)) return e;
-  if (!boxes || !max_values_out || !argmax_out || !ws || cap < 0 || ch_sdf < 0 || ch_sdf >= C || ch_center_row < 0 ||
-      ch_center_row >= C || ch_center_col < 0 || ch_center_col >= C)
-    return fail(UNMORE_E_INVALID, "unmore_center_reasoning: bad argument");
-  if (cap == 0) return 0;
-  cudaStream_t s = (cudaStream_t)stream;
-  CenterParams p{};
-  p.fields = fields; p.C = C; p.H = H; p.W = W;
-  p.ch_sdf = ch_sdf; p.ch_crow = ch_center_row; p.ch_ccol = ch_center_col;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.thr = center_score_max_thres;
-  p.max_values = max_values_out; p.argmax = argmax_out; p.splits = splits_out;
-  if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
-    return fail(UNMORE_E_INVALID, "unmore_center_reasoning: the three analyze_cc outputs go together");
-  p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
-  center_filters(p);
-  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
-  return cuda_fail(launch_center(p, num_sms(), s), "center_kernel");
+  return center_reasoning("unmore_center_reasoning", fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes,
+                          boxes_f64, counts, cap, center_score_max_thres, max_values_out, argmax_out, splits_out,
+                          cc_counts_out, cc_boxes_out, cc_overflow, ws, (cudaStream_t)stream);
 }
 
 int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, int ch_sdf, const void* boxes,
@@ -384,18 +445,9 @@ int unmore_score_and_rasterise(const float* fields, int n_img, int C, int H, int
                                int ch_center_col, int ch_exist, const void* boxes, int boxes_f64, const int* counts,
                                int cap, float* scores_out, float* tight_out, int* areas_out, uint32_t* masks_out,
                                unmore_stream_t stream) {
-  if (int e = check_fields(fields, n_img, C, H, W)) return e;
-  if (!boxes || !scores_out || !tight_out || !areas_out || cap < 0 || ch_sdf < 0 || ch_sdf >= C || ch_center_row < 0 ||
-      ch_center_row >= C || ch_center_col < 0 || ch_center_col >= C || ch_exist < 0 || ch_exist >= C)
-    return fail(UNMORE_E_INVALID, "unmore_score_and_rasterise: bad argument");
-  if (n_img > 65535) return fail(UNMORE_E_CAPACITY, "unmore_score_and_rasterise: n_img > 65535 per call");
-  ScoreParams p{};
-  p.fields = fields; p.n_img = n_img; p.C = C; p.H = H; p.W = W;
-  p.ch_sdf = ch_sdf; p.ch_crow = ch_center_row; p.ch_ccol = ch_center_col; p.ch_exist = ch_exist;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
-  p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
-  p.areas = areas_out; p.masks = masks_out;
-  return cuda_fail(launch_score(p, (cudaStream_t)stream), "score_kernel");
+  return score_and_rasterise("unmore_score_and_rasterise", fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col,
+                             ch_exist, boxes, boxes_f64, counts, cap, scores_out, tight_out, areas_out, masks_out,
+                             (cudaStream_t)stream);
 }
 
 int unmore_mask_resize(const unsigned char* masks, int B, int H, int W, int out_h, int out_w, unsigned char* out,
@@ -451,11 +503,8 @@ int unmore_sat_build_fields(const float* fields, int n_img, int C, int H, int W,
 int unmore_box_sums(const double* sat, int n_img, int planes_per_img, int plane, int H, int W, const void* boxes,
                     int boxes_f64, const int* counts, int cap, double* sums_out, double* means_out,
                     unmore_stream_t stream) {
-  if (!sat || !boxes || !sums_out || n_img < 0 || cap < 0 || plane < 0 || plane >= planes_per_img)
-    return fail(UNMORE_E_INVALID, "unmore_box_sums: bad argument");
-  return cuda_fail(launch_box_sums(sat, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap, n_img, sums_out,
-                                   means_out, (cudaStream_t)stream),
-                   "box_sums_kernel");
+  return box_sums("unmore_box_sums", sat, n_img, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap, sums_out,
+                  means_out, (cudaStream_t)stream);
 }
 
 int unmore_mask_pack(const unsigned char* in, size_t K, int H, int W, uint32_t* out, unmore_stream_t stream) {
@@ -489,6 +538,73 @@ int unmore_mask_nms(const uint32_t* masks, int K, int H, int W, const float* sco
                                      iou_threshold, order_ws, reinterpret_cast<unsigned long long*>(matrix_ws), keep_out,
                                      keep_count_out, (cudaStream_t)stream),
                    "mask matrix nms");
+}
+
+// ---- padded stacks of images of different sizes: H, W are the pitch, image_hw [n_img, 2] int32 (device) the extents --
+int unmore_existence_scores_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_exist,
+                               const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
+                               unmore_stream_t stream) {
+  const char* name = "unmore_existence_scores_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return existence_scores(name, false, fields, n_img, C, H, W, ch_exist, boxes, boxes_f64, counts, cap, scores_out, ws,
+                          (cudaStream_t)stream, image_hw);
+}
+
+int unmore_center_reasoning_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                               int ch_center_row, int ch_center_col, const void* boxes, int boxes_f64, const int* counts,
+                               int cap, double center_score_max_thres, double* max_values_out, int* argmax_out,
+                               double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow,
+                               void* ws, unmore_stream_t stream) {
+  const char* name = "unmore_center_reasoning_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return center_reasoning(name, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes, boxes_f64, counts, cap,
+                          center_score_max_thres, max_values_out, argmax_out, splits_out, cc_counts_out, cc_boxes_out,
+                          cc_overflow, ws, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_boundary_refine_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                              const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
+                              int apply_small_filter, int early_exit, float proposal_area_thres, float max_sdf_thres,
+                              float max_shrink_threshold, float delta_ratio, float* boxes_out, float* labels_out,
+                              int* rounds_out, void* ws, unmore_stream_t stream) {
+  const char* name = "unmore_boundary_refine_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return boundary_refine(name, false, fields, n_img, C, H, W, ch_sdf, boxes, boxes_f64, counts, cap, n_round,
+                         apply_small_filter, early_exit, proposal_area_thres, max_sdf_thres, max_shrink_threshold,
+                         delta_ratio, boxes_out, labels_out, rounds_out, ws, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_score_and_rasterise_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                                  int ch_center_row, int ch_center_col, int ch_exist, const void* boxes, int boxes_f64,
+                                  const int* counts, int cap, float* scores_out, float* tight_out, int* areas_out,
+                                  uint32_t* masks_out, unmore_stream_t stream) {
+  const char* name = "unmore_score_and_rasterise_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return score_and_rasterise(name, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, ch_exist, boxes, boxes_f64,
+                             counts, cap, scores_out, tight_out, areas_out, masks_out, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_box_sums_hw(const double* sat, int n_img, int planes_per_img, int plane, int H, int W, const int* image_hw,
+                       const void* boxes, int boxes_f64, const int* counts, int cap, double* sums_out, double* means_out,
+                       unmore_stream_t stream) {
+  const char* name = "unmore_box_sums_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return box_sums(name, sat, n_img, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap, sums_out, means_out,
+                  (cudaStream_t)stream, image_hw);
+}
+
+int unmore_sat_build_fields_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                               const int* channels_host, int n_channels, double* out, unmore_stream_t stream) {
+  const char* name = "unmore_sat_build_fields_hw";
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (int e = check_extents(name, image_hw)) return e;
+  if (!out || !channels_host || n_channels < 1 || n_channels > 4)
+    return fail(UNMORE_E_INVALID, "%s: bad argument (1..4 channels)", name);
+  for (int i = 0; i < n_channels; ++i)
+    if (channels_host[i] < 0 || channels_host[i] >= C) return fail(UNMORE_E_INVALID, "%s: channel out of range", name);
+  if (W > 2048) return fail(UNMORE_E_CAPACITY, "%s: W %d > 2048", name, W);
+  return cuda_fail(launch_sat_hw(fields, out, n_img, H, W, C, channels_host, n_channels, image_hw, (cudaStream_t)stream),
+                   "sat_hw_kernel");
 }
 
 }  // extern "C"

@@ -225,8 +225,10 @@ struct CenterTileRows {
 
 // PLANE_ELEMS: 0 = any field size / channel order; H*W = the three channels are consecutive planes of a field
 // of exactly that size (the COCO-val shape the batch path runs on), see MultiPlaneRows.
+// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window snap and the
+// --analyze_cc clip use the image's extent; plane addressing and PLANE_ELEMS go by the pitch.
 constexpr int kSpecPlaneElems = 480 * 640;
-template <bool ANALYZE_CC, int PLANE_ELEMS, bool ROW_SKIP>
+template <bool ANALYZE_CC, int PLANE_ELEMS, bool ROW_SKIP, bool SIZED = false>
 __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   CenterSmem& sm = *reinterpret_cast<CenterSmem*>(smem_raw);
@@ -286,7 +288,13 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
         next_located = true;
       }
     };
-    const Window win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    Window win;
+    if constexpr (SIZED) {
+      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
+    } else {
+      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    }
     double best = 0.0;
     int best_idx = -1;
     if (!win.empty()) {
@@ -627,8 +635,14 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
             double* o = p.cc_boxes + (row * kCcCap + tid) * 4;
             o[0] = (double)(int)fmax(cx - nw / 2, 0.0);
             o[1] = (double)(int)fmax(cy - nh / 2, 0.0);
-            o[2] = (double)(int)fmin(cx + nw / 2, (double)p.W);
-            o[3] = (double)(int)fmin(cy + nh / 2, (double)p.H);
+            if constexpr (SIZED) {
+              const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+              o[2] = (double)(int)fmin(cx + nw / 2, (double)e.y);
+              o[3] = (double)(int)fmin(cy + nh / 2, (double)e.x);
+            } else {
+              o[2] = (double)(int)fmin(cx + nw / 2, (double)p.W);
+              o[3] = (double)(int)fmin(cy + nh / 2, (double)p.H);
+            }
           }
           if (tid == 0 && n_comp > kCcCap) atomicAdd(p.cc_overflow, 1);
         }
@@ -770,6 +784,14 @@ int launch_components(const unsigned char* masks, int B, int* counts, int* boxes
 template <bool CC, int PE, bool RS = false>
 static int launch_center_t(const CenterParams& p, int num_sms, cudaStream_t stream) {
   // function attributes are per device: set on every launch (microseconds), no cached state
+  if constexpr (PE >= 0) {
+    if (p.image_hw) {   // a padded stack: the sized variant
+      cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CenterSmem));
+      if (e != cudaSuccess) return (int)e;
+      center_kernel<CC, PE, RS, true><<<num_sms * 2, kCenterThreads, sizeof(CenterSmem), stream>>>(p);
+      return (int)cudaGetLastError();
+    }
+  }
   cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CenterSmem));
   if (e != cudaSuccess) return (int)e;
   center_kernel<CC, PE, RS><<<num_sms * 2, kCenterThreads, sizeof(CenterSmem), stream>>>(p);

@@ -232,6 +232,16 @@ struct Window {
   __device__ __forceinline__ bool empty() const { return x2 <= x1 || y2 <= y1; }
 };
 
+// Extent (h, w) of image `img` of a padded field stack, from its [n_img, 2] int32 table (one 8-byte read-only load;
+// the table is 8-byte aligned, checked by the C ABI).  Clamped to [1, pitch]: a bad entry gives wrong numbers, never
+// an address outside the pitched planes.  The load is volatile so that a kernel which reads the extent again after a
+// long stretch of work (refine) really re-reads it (an L1 hit) instead of holding it in two registers meanwhile.
+__device__ __forceinline__ int2 image_extent(const int* image_hw, int img, int H, int W) {
+  int2 e;
+  asm volatile("ld.global.nc.v2.s32 {%0, %1}, [%2];" : "=r"(e.x), "=r"(e.y) : "l"(image_hw + 2 * (size_t)img));
+  return make_int2(min(max(e.x, 1), H), min(max(e.y, 1), W));
+}
+
 template <typename T>
 __device__ __forceinline__ Window snap_window(T x1, T y1, T x2, T y2, int W, int H) {
   Window w;

@@ -12,7 +12,10 @@ namespace unmore {
 
 constexpr int kExistWarps = 8;
 
-__global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const ExistParams p) {
+// SIZED: the fields are a padded stack and p.image_hw holds each image's (h, w) inside the (H, W) pitch; addresses
+// come from the pitch, the window snap from the image's own extent.
+template <bool SIZED>
+__device__ __forceinline__ void existence_items(const ExistParams& p) {
   __shared__ int2 tapy_all[kExistWarps][kCrop];   // vertical taps of the warp's current window: (i0, bits of l1)
   const int lane = threadIdx.x & 31;
   int2* const tapy = tapy_all[threadIdx.x >> 5];
@@ -27,7 +30,13 @@ __global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const Exist
     const size_t row = (size_t)img * p.work.cap + k;
     double x1, y1, x2, y2;
     load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
-    const Window win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    Window win;
+    if constexpr (SIZED) {
+      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
+    } else {
+      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    }
     float score = 0.f;  // zero-size crop: the reference raises; defined as "nothing there"
     if (!win.empty()) {
       ColTaps taps;
@@ -68,6 +77,9 @@ __global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const Exist
     if (lane == 0) p.scores[row] = score;
   }
 }
+
+__global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const ExistParams p) { existence_items<false>(p); }
+__global__ void __launch_bounds__(kExistWarps * 32) existence_hw_kernel(const ExistParams p) { existence_items<true>(p); }
 
 // The second resize mode (antialias=True): the mean of the antialiased crop (aa_rows.cuh), summed in exactly the order
 // above, so the score equals tile_means_kernel on the tile of unmore_crop_resize_aa bit for bit.
@@ -204,7 +216,8 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 }
 
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream) {
-  existence_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
+  if (p.image_hw) existence_hw_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
+  else existence_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

@@ -311,11 +311,13 @@ struct BoxT { T x1, y1, x2, y2; };
 // The box update of one round for one proposal, arithmetic in T (double on round 0 when the caller hands in
 // fp64 proposals — promotion at object_reasoning.py:190-194 — float afterwards).
 // Returns the label of this round and the updated box (fp32, :479).
+// (W, H): the image's size (its own extent in a padded stack).
 template <typename T>
-__device__ __forceinline__ int apply_update(const RefineParams& p, const Window& win, const Deltas& d, BoxT<T> b, float4& out) {
+__device__ __forceinline__ int apply_update(const RefineParams& p, int W, int H, const Window& win, const Deltas& d, BoxT<T> b,
+                                            float4& out) {
   // signed deltas: >0 expands, <0 shrinks; expansion is ignored on sides glued to the image edge (:444-447)
   float sg[4] = {-d.dx1, -d.dy1, d.dx2, d.dy2};
-  const bool edge[4] = {win.x1 == 0, win.y1 == 0, win.x2 == p.W, win.y2 == p.H};
+  const bool edge[4] = {win.x1 == 0, win.y1 == 0, win.x2 == W, win.y2 == H};
 #pragma unroll
   for (int k = 0; k < 4; ++k)
     if (sg[k] > 0.f && edge[k]) sg[k] = 0.f;
@@ -346,8 +348,8 @@ __device__ __forceinline__ int apply_update(const RefineParams& p, const Window&
   }
   if (nx1 < (T)0) nx1 = (T)0;
   if (ny1 < (T)0) ny1 = (T)0;
-  if (nx2 > (T)p.W) nx2 = (T)p.W;
-  if (ny2 > (T)p.H) ny2 = (T)p.H;
+  if (nx2 > (T)W) nx2 = (T)W;
+  if (ny2 > (T)H) ny2 = (T)H;
   out = make_float4((float)nx1, (float)ny1, (float)nx2, (float)ny2);
   return label;
 }
@@ -357,8 +359,11 @@ constexpr int kRefineMinBlocks = 3;   // resident CTAs per SM, in __launch_bound
 constexpr int kSpecRowElems = 640;   // row pitch of the COCO-val-shaped fields the batch path runs on
 // The persistent round loop: warps pull proposals from the worklist until it is empty.  `terms(plane, win)` computes
 // the boundary terms of a window from its resampled rows; the resize mode only changes where those rows come from.
-template <class Terms>
-__device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCols& cols, int lane, Terms terms) {
+// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The extent is read where the
+// window is snapped and again where the box is updated, so it is not live across the terms (registers are tight).
+template <bool SIZED, class Terms>
+__device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCols& cols, int lane, Terms terms,
+                                                 const int* image_hw = nullptr) {
   const int total = worklist_total(p.work);
   int img = 0;   // image of the previous work item: the locate hint
   for (;;) {
@@ -383,14 +388,19 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
       const bool dbl = (r == 0) && p.boxes_f64;
       Window win;
       bool keep;
+      int ih = p.H, iw = p.W;
+      if constexpr (SIZED) {
+        const int2 e = image_extent(image_hw, img, p.H, p.W);
+        ih = e.x; iw = e.y;
+      }
       if (dbl) {
         BoxT<double> bd;
         load_box<double>(p.boxes, true, row, bd.x1, bd.y1, bd.x2, bd.y2);
         keep = __dmul_rn(__dsub_rn(bd.x2, bd.x1), __dsub_rn(bd.y2, bd.y1)) > (double)p.area_thres;
-        win = snap_window<double>(bd.x1, bd.y1, bd.x2, bd.y2, p.W, p.H);
+        win = snap_window<double>(bd.x1, bd.y1, bd.x2, bd.y2, iw, ih);
       } else {
         keep = __fmul_rn(__fsub_rn(bf.x2, bf.x1), __fsub_rn(bf.y2, bf.y1)) > p.area_thres;
-        win = snap_window<float>(bf.x1, bf.y1, bf.x2, bf.y2, p.W, p.H);
+        win = snap_window<float>(bf.x1, bf.y1, bf.x2, bf.y2, iw, ih);
       }
       if (p.apply_small_filter && !keep) { label = -2.f; break; }  // filter_small_proposal (:293-299), strict '>'
       float4 nb = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -415,15 +425,21 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
       }
       if (!win.empty()) {
         if (d.max_sdf > p.max_sdf_thres) {
+          if constexpr (SIZED) {
+            const int2 e = image_extent(image_hw, img, p.H, p.W);
+            ih = e.x; iw = e.y;
+          } else {
+            ih = p.H; iw = p.W;
+          }
           if (dbl) {
             BoxT<double> bd;
             load_box<double>(p.boxes, true, row, bd.x1, bd.y1, bd.x2, bd.y2);
-            lab = apply_update<double>(p, win, d, bd, nb);
+            lab = apply_update<double>(p, iw, ih, win, d, bd, nb);
             // fp64 round 0: the fp32 cast must be exact and the fp32 area test of round 1 must agree
             fixed = (double)nb.x == bd.x1 && (double)nb.y == bd.y1 && (double)nb.z == bd.x2 && (double)nb.w == bd.y2 &&
                     (!p.apply_small_filter || __fmul_rn(__fsub_rn(nb.z, nb.x), __fsub_rn(nb.w, nb.y)) > p.area_thres);
           } else {
-            lab = apply_update<float>(p, win, d, bf, nb);
+            lab = apply_update<float>(p, iw, ih, win, d, bf, nb);
             fixed = true;
           }
         }
@@ -450,18 +466,29 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
   }
 }
 
-template <int ROW_ELEMS>
-__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
+template <int ROW_ELEMS, bool SIZED>
+__device__ __forceinline__ void refine_crops(const RefineParams& p, const int* image_hw) {
   __shared__ BorderCols cols_all[kRefineWarps];
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
-  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
+  refine_proposals<SIZED>(p, cols, lane, [&](const float* plane, const Window& win) {
     CropRows<ROW_ELEMS> src;
     src.taps.template init<kStrided>(lane, win.w());
     src.plane.init(plane, p.W, win);
     src.init_rows(lane, cols.tapy, win.h());
     return boundary_terms(src, cols, lane);
-  });
+  }, image_hw);
+}
+
+template <int ROW_ELEMS>
+__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
+  refine_crops<ROW_ELEMS, false>(p, nullptr);
+}
+// the same on a padded stack: image_hw [n_img, 2] holds each image's (h, w) inside the (H, W) pitch
+template <int ROW_ELEMS>
+__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_hw_kernel(const RefineParams p,
+                                                                                        const int* __restrict__ image_hw) {
+  refine_crops<ROW_ELEMS, true>(p, image_hw);
 }
 
 // The second resize mode: the same round loop on antialiased rows (aa_rows.cuh).  A warp needs 15 KB more shared
@@ -474,7 +501,7 @@ __global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refin
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
   AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
-  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
+  refine_proposals<false>(p, cols, lane, [&](const float* plane, const Window& win) {
     AaCropRows src;
     src.init(lane, rows, plane, p.W, win);
     return boundary_terms(src, cols, lane);
@@ -512,9 +539,9 @@ __global__ void __launch_bounds__(128) round_update_kernel(const RefineParams p,
     Deltas d;
     d.max_sdf = max_sdf[m]; d.dx1 = dl.x; d.dy1 = dl.y; d.dx2 = dl.z; d.dy2 = dl.w;
     if (p.boxes_f64) {
-      lab = apply_update<double>(p, win, d, BoxT<double>{x1, y1, x2, y2}, nb);
+      lab = apply_update<double>(p, p.W, p.H, win, d, BoxT<double>{x1, y1, x2, y2}, nb);
     } else {
-      lab = apply_update<float>(p, win, d, BoxT<float>{(float)x1, (float)y1, (float)x2, (float)y2}, nb);
+      lab = apply_update<float>(p, p.W, p.H, win, d, BoxT<float>{(float)x1, (float)y1, (float)x2, (float)y2}, nb);
     }
   }
   p.boxes_out[m] = nb;
@@ -527,9 +554,12 @@ int launch_round_update(const RefineParams& p, const float4* deltas, const float
   return (int)cudaGetLastError();
 }
 
-int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream) {
+int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw) {
   const int ctas = num_sms * kRefineMinBlocks;  // warps pull proposals dynamically
-  if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
+  if (image_hw) {   // the row-pitch specialisation goes by the pitch
+    if (p.W == kSpecRowElems) refine_hw_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p, image_hw);
+    else refine_hw_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p, image_hw);
+  } else if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   else refine_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }

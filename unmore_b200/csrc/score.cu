@@ -65,8 +65,13 @@ __device__ __forceinline__ bool resized_mask_bit_aa(const uint32_t m[kCrop][4], 
 // of the reference's original mode); the masks are rasterised back to the box with the antialiased kernel when
 // p.aa_raster is set and with the plain one otherwise; p.exist_scores, when given, replaces the mean of the fourth
 // tile (the reference's classifier puts out one scalar per crop, object_scoring.py:140-150).
-template <bool TILES_AA>
-__global__ void __launch_bounds__(kScoreThreads) score_kernel(const ScoreParams p) {
+// SIZED (fused path only): a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window
+// snaps to the image's extent; the mask canvas stays H x ceil(W/32) words (bits outside the image stay 0).
+template <bool SIZED> struct ScoreArgs { using type = ScoreParams; };
+template <> struct ScoreArgs<true> { using type = ScoreHwParams; };
+
+template <bool TILES_AA, bool SIZED = false>
+__global__ void __launch_bounds__(kScoreThreads) score_kernel(const typename ScoreArgs<SIZED>::type p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ScoreSmem& sm = *reinterpret_cast<ScoreSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -76,7 +81,13 @@ __global__ void __launch_bounds__(kScoreThreads) score_kernel(const ScoreParams 
   const size_t row = (size_t)img * p.cap + k;
   double bx1, by1, bx2, by2;
   load_box<double>(p.boxes, p.boxes_f64 != 0, row, bx1, by1, bx2, by2);
-  const Window win = snap_window<double>(bx1, by1, bx2, by2, p.W, p.H);
+  Window win;
+  if constexpr (SIZED) {
+    const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+    win = snap_window<double>(bx1, by1, bx2, by2, e.y, e.x);
+  } else {
+    win = snap_window<double>(bx1, by1, bx2, by2, p.W, p.H);
+  }
   const int Wp = (p.W + 31) >> 5;
   uint32_t* mask_out = p.masks ? p.masks + row * (size_t)p.H * Wp : nullptr;
   if (tid == 0) { sm.xmin = 1 << 30; sm.ymin = 1 << 30; sm.xmax = -1; sm.ymax = -1; sm.area = 0; }
@@ -246,13 +257,20 @@ int launch_mask_resize(const unsigned char* masks, int B, int oh, int ow, unsign
   return (int)cudaGetLastError();
 }
 
-int launch_score(const ScoreParams& p, cudaStream_t stream) {
+int launch_score(const ScoreParams& p, cudaStream_t stream, const int* image_hw) {
   if (p.n_img <= 0 || p.cap <= 0) return 0;
   dim3 grid(p.cap, p.n_img);
   if (p.tiles) {
     cudaError_t e = cudaFuncSetAttribute(score_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
     if (e != cudaSuccess) return (int)e;
     score_kernel<true><<<grid, kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
+  } else if (image_hw) {
+    ScoreHwParams hp;
+    static_cast<ScoreParams&>(hp) = p;
+    hp.image_hw = image_hw;
+    cudaError_t e = cudaFuncSetAttribute(score_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
+    if (e != cudaSuccess) return (int)e;
+    score_kernel<false, true><<<grid, kScoreThreads, sizeof(ScoreSmem), stream>>>(hp);
   } else {
     cudaError_t e = cudaFuncSetAttribute(score_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
     if (e != cudaSuccess) return (int)e;

@@ -42,7 +42,8 @@ struct TileParams {
   float4* deltas;      // [M] (dx1, dy1, dx2, dy2)
   float* max_sdf;      // [M] or nullptr
 };
-int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream);
+// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
+int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw = nullptr);
 int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
 int launch_tiles(const TileParams& p, cudaStream_t stream);
 int launch_round_update(const RefineParams& p, const float4* deltas, const float* max_sdf, int M, cudaStream_t stream);
@@ -55,6 +56,7 @@ struct ExistParams {
   int boxes_f64;
   WorkList work;
   float* scores;  // [n_img, cap]
+  const int* image_hw;  // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
 };
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream);
 int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
@@ -90,6 +92,7 @@ struct CenterParams {
   unsigned char* cc_counts;  // [n_img, cap] component boxes emitted (0 unless the proposal passes with >= 2 components)
   double* cc_boxes;          // [n_img, cap, kCcCap, 4] enlarged component boxes
   int* cc_overflow;          // incremented once per proposal with more than kCcCap components
+  const int* image_hw;       // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
 };
 int launch_center(const CenterParams& p, int num_sms, cudaStream_t stream);
 int launch_components(const unsigned char* masks, int B, int* counts, int* boxes, cudaStream_t stream);
@@ -153,7 +156,11 @@ struct ScoreParams {
   int* areas;          // [n_img, cap] set pixels
   uint32_t* masks;     // nullable [n_img, cap, H, ceil(W/32)] packed union masks
 };
-int launch_score(const ScoreParams& p, cudaStream_t stream);
+// The sized kernel variant's parameters (a struct of its own: a larger ScoreParams changes the code of score_kernel)
+struct ScoreHwParams : ScoreParams {
+  const int* image_hw; // [n_img, 2] (h, w) of each image inside the (H, W) pitch
+};
+int launch_score(const ScoreParams& p, cudaStream_t stream, const int* image_hw = nullptr);
 int launch_mask_resize(const unsigned char* masks, int B, int oh, int ow, unsigned char* out, cudaStream_t stream);
 
 struct FinalParams {
@@ -170,11 +177,18 @@ struct FinalParams {
 };
 int launch_final_scores(const FinalParams& p, cudaStream_t stream);
 
-// ---- sat.cu --------------------------------------------------------------------------
+// ---- sat.cu, box_sums.cu --------------------------------------------------------------------------
 int launch_sat(const float* in, double* out, int n_planes, int H, int W, int C, const int* channels, int n_ch,
                cudaStream_t stream);
+// tables of a padded field stack: pixels outside each image's (h, w) enter the sums as zeros
+int launch_sat_hw(const float* fields, double* out, int n_img, int H, int W, int C, const int* channels, int n_ch,
+                  const int* image_hw, cudaStream_t stream);
 int launch_box_sums(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
-                    const int* counts, int cap, int n_img, double* sums, double* means, cudaStream_t stream);
+                    const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
+                    cudaStream_t stream);
+int launch_box_sums_hw(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
+                       const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
+                       cudaStream_t stream);
 
 // ---- masks.cu ------------------------------------------------------------------------
 int launch_mask_pack(const unsigned char* in, uint32_t* out, size_t n_masks, int H, int W, int num_sms, cudaStream_t stream);

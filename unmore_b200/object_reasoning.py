@@ -423,17 +423,21 @@ class Object_Discovery:
         return kb[0, : int(kc[0])].cpu().numpy()
 
     def discover_batch(self, fields: torch.Tensor, proposals: torch.Tensor, counts: Optional[torch.Tensor] = None,
-                       stats: Optional[dict] = None):
+                       stats: Optional[dict] = None, image_hw: Optional[torch.Tensor] = None):
         """Existence check -> center reasoning -> re-check of the splits -> boundary reasoning ->
         NMS for a batch of images, entirely on device.
 
         fields [B,4,H,W] fp32, proposals [B,N,4] fp64/fp32, counts [B] int32 or None.
+        ``image_hw`` [B,2] int32 (device): ``fields`` is a padded stack of images of different sizes
+        (``ops.pack_fields``); every image gets what it would get alone.  Not with antialias=True or a tile provider.
         Returns (boxes [B, 5N (9N + 256 with --analyze_cc), 4] fp32, counts [B] int32) in the reference's output order."""
         a = self.args
         ch = self.channels
         B, N = proposals.shape[0], proposals.shape[1]
         dev = fields.device
         f64 = torch.float64
+        if image_hw is not None and (self._tile_path or self.antialias):
+            raise ops.UnmoreError("discover_batch: image_hw (images of different sizes) needs antialias=False and no tile provider")
         if self._tile_path:   # per-crop nets: image by image on the tile path (not the fused kernels)
             dets = [self._discover_image_tiles(fields[b], proposals[b] if counts is None else proposals[b, : int(counts[b])])
                     for b in range(B)]
@@ -447,12 +451,13 @@ class Object_Discovery:
         ws = ops.workspace(B, dev)
         # Step 1: existence checking (:627-630)
         aa = self.antialias
-        ex = ops.existence_scores(fields, proposals, counts, ch=ch, ws=ws, antialias=aa)
+        hw = image_hw
+        ex = ops.existence_scores(fields, proposals, counts, ch=ch, ws=ws, antialias=aa, image_hw=hw)
         p1, c1, _ = ops.compact_boxes(proposals, counts, ops.MODE_SCORE_GE, ex, thr=a.class_score_thres, out_dtype=f64)
         # Step 2: center reasoning (:634-637)
         cc_on = bool(getattr(a, "analyze_cc", False))
         _, am1, sp1, cc = ops.center_reasoning(fields, p1, c1, thr=a.center_score_max_thres, ch=ch, ws=ws,
-                                               analyze_cc=cc_on, antialias=aa)
+                                               analyze_cc=cc_on, antialias=aa, image_hw=hw)
         # 4 split boxes per failing proposal; with --analyze_cc the component boxes of passing proposals follow
         # (a speckled mask can carry dozens: the reference has no limit, here the list holds 4N + 4N + 256 rows)
         split_cap = 8 * N + 256 if cc_on else 4 * N
@@ -473,31 +478,36 @@ class Object_Discovery:
                 # a proposal with more components than the device buffer (unmore_cc_cap()): rebuild the component
                 # part of the split list of the affected images with the unlimited host labelling (rare path)
                 c1h = c1.cpu().tolist()
+                hwh = None if hw is None else hw.cpu().tolist()
                 capc = cc_boxes.shape[2]
                 for b in range(B):
                     n = c1h[b]
                     if n == 0 or int((cc_counts[b, :n] >= capc).sum()) == 0:
                         continue
                     passing = torch.nonzero(am1[b, :n] < 0).flatten().tolist()
-                    extra = self._cc_boxes_with_overflow(fields[b:b + 1], p1[b:b + 1], passing, cc_counts[b], cc_boxes[b],
-                                                         fields.shape[-2], fields.shape[-1])
+                    if hwh is None:
+                        fb, (hb, wb) = fields[b:b + 1], fields.shape[-2:]
+                    else:   # the image alone, at its own size (the kernels clamp the extents the same way)
+                        hb, wb = (min(max(v, 1), p) for v, p in zip(hwh[b], fields.shape[-2:]))
+                        fb = fields[b:b + 1, :, :hb, :wb].contiguous()
+                    extra = self._cc_boxes_with_overflow(fb, p1[b:b + 1], passing, cc_counts[b], cc_boxes[b], hb, wb)
                     n_split = 4 * int((am1[b, :n] >= 0).sum())
                     if n_split + len(extra) > split_cap:
                         raise RuntimeError("analyze_cc: component boxes exceeded the split-list capacity")
                     split[b, n_split:n_split + len(extra)] = torch.as_tensor(extra, device=dev)
                     sc[b] = n_split + len(extra)
         # re-check the split proposals (:639-646)
-        ex2 = ops.existence_scores(fields, split, sc, ch=ch, ws=ws, antialias=aa)
+        ex2 = ops.existence_scores(fields, split, sc, ch=ch, ws=ws, antialias=aa, image_hw=hw)
         p2, c2, _ = ops.compact_boxes(split, sc, ops.MODE_SCORE_GE, ex2, thr=a.class_score_thres, out_dtype=f64)
         _, am2, _, _ = ops.center_reasoning(fields, p2, c2, thr=a.center_score_max_thres, ch=ch, ws=ws, want_splits=False,
-                                            antialias=aa)
+                                            antialias=aa, image_hw=hw)
         ops.compact_boxes(p2, c2, ops.MODE_ARGMAX_LT0, am2, out=refine_in, counts_out=rc, append=True)
         # Step 3: boundary reasoning (:650-658)
         rb, lab, rounds = ops.boundary_refine(fields, refine_in, rc, n_round=a.n_round, apply_small_filter=True,
                                               early_exit=True, proposal_area_thres=a.proposal_area_thres,
                                               max_sdf_thres=a.max_sdf_thres,
                                               max_shrink_threshold=a.max_shrink_threshold, delta_ratio=a.delta_ratio,
-                                              ch=ch, ws=ws, want_rounds=stats is not None, antialias=aa)
+                                              ch=ch, ws=ws, want_rounds=stats is not None, antialias=aa, image_hw=hw)
         # label-1 survivors; the NMS kernel holds its alive set for at most 32768 boxes per image
         lost1 = torch.zeros((1,), dtype=torch.int32, device=dev) if cap_out > 32768 else None
         fin, fc, _ = ops.compact_boxes(rb, rc, ops.MODE_LABEL_EQ, lab, thr=1.0, out_dtype=torch.float32,
@@ -512,15 +522,37 @@ class Object_Discovery:
                          refine_in_boxes=refine_in, pass1_boxes=p1, argmax1=am1, pass2_boxes=p2, pass2=c2)
         return kb, kc
 
-    def main_object_discovery(self, images=None, image_ids=None, proposals=None) -> Dict[int, np.ndarray]:
+    def main_object_discovery(self, images=None, image_ids=None, proposals=None, batch_size: int = 1) -> Dict[int, np.ndarray]:
         """object_reasoning.py:615-665.  Called with no arguments like the reference: loops over
         ``self.test_dataset`` (``get_image_with_index`` -> field stack + ``{'image_id'}``), runs the loop body
         for every image and dumps ``results_dict`` {image_id: [[x1,y1,x2,y2], ...]} to
         ``<result_folder>/discovery_results.json`` (:664-665); images with no detection are absent, as in the
         reference.  ``images`` / ``image_ids`` (not in the reference) run the same loop over in-memory stacks
-        without touching the disk.  Returns ``results_dict`` (the reference returns None)."""
+        without touching the disk.  Returns ``results_dict`` (the reference returns None).
+
+        ``batch_size`` > 1 (not in the reference): consecutive dataset images of any sizes are padded into one stack
+        (``ops.pack_fields``), each with its own anchors, and run through ``discover_batch`` together; the results and the
+        file are identical to ``batch_size=1``.  Ignored with antialias=True or a tile provider."""
         from . import rle
         results = {}
+        if images is None and batch_size > 1 and not self.antialias and not self._tile_path:
+            if self.test_dataset is None:
+                raise RuntimeError("main_object_discovery(): set self.test_dataset (e.g. FieldDataset) first")
+            for start in range(0, len(self.test_dataset), batch_size):
+                batch = [self.test_dataset.get_image_with_index(i)
+                         for i in range(start, min(start + batch_size, len(self.test_dataset)))]
+                ids = [int(lb["image_id"].item()) if torch.is_tensor(lb["image_id"]) else int(lb["image_id"]) for _, lb in batch]
+                fields, hw = ops.pack_fields([im.to(self.device, torch.float32) for im, _ in batch])
+                self.height, self.width = batch[-1][0].shape[-2], batch[-1][0].shape[-1]
+                props = [proposals if proposals is not None else self.generate_random_proposal(im.shape[-2], im.shape[-1])
+                         for im, _ in batch]
+                boxes, counts = ops.stack_proposals([self._boxes(p)[0] for p in props], self.device)
+                kb, kc = self.discover_batch(fields, boxes, counts, image_hw=hw)
+                kb, kc = kb.cpu().numpy(), kc.cpu().tolist()
+                for b, image_id in enumerate(ids):
+                    if kc[b]:
+                        results[image_id] = kb[b, : kc[b]].copy()
+            return self._write_discovery(results)
         if images is not None:
             for img, iid in zip(images, image_ids):
                 det = self.discover_image(img, proposals)
@@ -536,6 +568,10 @@ class Object_Discovery:
             det = self.discover_image(image, proposals)
             if len(det):
                 results[image_id] = det
+        return self._write_discovery(results)
+
+    def _write_discovery(self, results):
+        from . import rle
         if self.result_folder is not None:
             os.makedirs(self.result_folder, exist_ok=True)
             with open(os.path.join(self.result_folder, "discovery_results.json"), "w") as f:

@@ -80,11 +80,15 @@ class Object_Scoring:
                 "pred_existence_scores": ops.existence_scores(f, boxes, ch=ch)[0]}
 
     def score_batch(self, fields: torch.Tensor, boxes: torch.Tensor, counts: Optional[torch.Tensor] = None,
-                    want_masks: bool = True):
+                    want_masks: bool = True, image_hw: Optional[torch.Tensor] = None):
         """Steps 1-8 of main_object_scoring for a batch: returns a dict of device tensors in NMS keep
         order: out [B,cap,5] fp64 (score, existence, center, boundary, area_score), bbox [B,cap,4] xywh,
         selected [B,cap] (post_process predicate), keep [B,cap], keep_counts [B], masks (packed, indexed by
-        the ORIGINAL proposal index: use keep to gather)."""
+        the ORIGINAL proposal index: use keep to gather).  ``image_hw`` [B,2] int32 (device): ``fields`` is a padded
+        stack of images of different sizes (``ops.pack_fields``); image b's masks are ``masks[b, :, :h_b,
+        :ceil(w_b/32)]``.  Not with antialias=True or a tile provider."""
+        if image_hw is not None and (self.tile_provider is not None or self.antialias):
+            raise ops.UnmoreError("score_batch: image_hw (images of different sizes) needs antialias=False and no tile provider")
         if self.tile_provider is not None:   # per-crop nets: (sdf, center) tiles + one classifier scalar per crop
             B, cap = boxes.shape[0], boxes.shape[1]
             tiles = torch.zeros((B, cap, 4, ops.CROP, ops.CROP), dtype=torch.float32, device=fields.device)
@@ -103,7 +107,8 @@ class Object_Scoring:
             scores, tight, areas, masks = ops.score_and_rasterise_from_tiles(tiles, fields.shape[-2], fields.shape[-1], boxes, counts,
                                                                              want_masks=want_masks)
         else:
-            scores, tight, areas, masks = ops.score_and_rasterise(fields, boxes, counts, ch=self.channels, want_masks=want_masks)
+            scores, tight, areas, masks = ops.score_and_rasterise(fields, boxes, counts, ch=self.channels, want_masks=want_masks,
+                                                                  image_hw=image_hw)
         keep, kc, _ = ops.box_nms(tight, scores[:, :, 2].contiguous(), counts, iou_threshold=0.5, want_boxes=False)
         out, bbox, sel = ops.final_scores(scores, tight, areas, keep, kc, self.args.existence_score_thres,
                                           self.args.center_score_thres, self.args.boundary_score_thres)
@@ -142,14 +147,21 @@ class Object_Scoring:
             return []
         boxes = torch.as_tensor(np.asarray(raw_proposals, dtype=np.float64)).reshape(1, -1, 4).to(self.device)
         r = self.score_batch(fields, boxes, None, want_masks=with_masks)
-        n = int(r["keep_counts"][0])
-        keep = r["keep"][0, :n].long()
-        out = r["out"][0, :n].cpu().numpy()
-        bbox = r["bbox"][0, :n].cpu().numpy()
-        dense = unpack_masks(r["masks"][0][keep], W) if (with_masks and not rle) else None
+        return self._annotations(r, 0, H, W, image_id, with_masks, rle)
+
+    @staticmethod
+    def _annotations(r, b, H, W, image_id, with_masks, rle):
+        """Annotations of image ``b`` of a ``score_batch`` result, an (H, W) image; its masks are the [:H, :ceil(W/32)]
+        corner of the (possibly pitched) mask canvas."""
+        n = int(r["keep_counts"][b])
+        keep = r["keep"][b, :n].long()
+        out = r["out"][b, :n].cpu().numpy()
+        bbox = r["bbox"][b, :n].cpu().numpy()
+        masks = r["masks"][b][keep][:, :H, : (W + 31) // 32] if with_masks else None
+        dense = unpack_masks(masks, W) if (with_masks and not rle) else None
         if with_masks and rle:
             from . import rle as rle_codec
-            encoded = rle_codec.encode_packed(r["masks"][0][keep].contiguous(), W)
+            encoded = rle_codec.encode_packed(masks.contiguous(), W)
         anns = []
         for i in range(n):
             ann = {"image_id": image_id, "category_id": 1, "score": out[i, 0], "bbox": [v for v in bbox[i]],
@@ -160,14 +172,38 @@ class Object_Scoring:
             anns.append(ann)
         return anns
 
-    def main_object_scoring(self, images=None, image_ids=None) -> List[dict]:
+    def main_object_scoring(self, images=None, image_ids=None, batch_size: int = 1) -> List[dict]:
         """object_scoring.py:172-272.  Called with no arguments like the reference: loops over
         ``self.test_dataset``, skips images without raw predictions (:177-179), and dumps ``out_annotations``
         (``segmentation`` = COCO RLE dicts, :257-268) to ``<result_folder>/object_discovery_with_scores.json``.
         ``images`` / ``image_ids`` (not in the reference) run the loop over in-memory stacks and keep the masks
-        dense.  Returns ``out_annotations`` (the reference returns None)."""
-        from . import rle
+        dense.  Returns ``out_annotations`` (the reference returns None).
+
+        ``batch_size`` > 1 (not in the reference): consecutive dataset images of any sizes are padded into one stack
+        (``ops.pack_fields``) and scored by one ``score_batch``; the annotations and the file are identical to
+        ``batch_size=1``.  Ignored with antialias=True or a tile provider."""
         out = []
+        if images is None and batch_size > 1 and not self.antialias and self.tile_provider is None:
+            if self.test_dataset is None:
+                raise RuntimeError("main_object_scoring(): set self.test_dataset (e.g. FieldDataset) first")
+            for start in range(0, len(self.test_dataset), batch_size):
+                batch = []
+                for image_idx in range(start, min(start + batch_size, len(self.test_dataset))):
+                    image, label = self.test_dataset.get_image_with_index(image_idx)
+                    image_id = int(label["image_id"].item()) if torch.is_tensor(label["image_id"]) else int(label["image_id"])
+                    if str(image_id) not in self.raw_annotations.keys():
+                        print(image_id, "do not have raw predictions")
+                        continue
+                    batch.append((image, image_id, self.raw_annotations[str(image_id)]))
+                if not batch:
+                    continue
+                fields, hw = ops.pack_fields([self._fields(im)[0] for im, _, _ in batch])
+                boxes, counts = ops.stack_proposals(
+                    [torch.as_tensor(np.asarray(raw, dtype=np.float64)).reshape(-1, 4) for _, _, raw in batch], self.device)
+                r = self.score_batch(fields, boxes, counts, image_hw=hw)
+                for b, (im, image_id, _) in enumerate(batch):
+                    out.extend(self._annotations(r, b, im.shape[-2], im.shape[-1], image_id, True, True))
+            return self._write_scoring(out)
         if images is not None:
             for img, iid in zip(images, image_ids):
                 raw = self.raw_annotations.get(str(int(iid)))
@@ -184,6 +220,10 @@ class Object_Scoring:
                 print(image_id, "do not have raw predictions")
                 continue
             out.extend(self.score_image(image, self.raw_annotations[str(image_id)], image_id=image_id, rle=True))
+        return self._write_scoring(out)
+
+    def _write_scoring(self, out):
+        from . import rle
         if self.result_folder is not None:
             os.makedirs(self.result_folder, exist_ok=True)
             with open(os.path.join(self.result_folder, "object_discovery_with_scores.json"), "w") as f:

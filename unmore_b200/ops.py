@@ -14,6 +14,7 @@ from . import _lib
 from .synth import CH_CCOL, CH_CROW, CH_EXIST, CH_SDF
 
 CROP = 128
+UnmoreError = _lib.UnmoreError
 
 
 @dataclass(frozen=True)
@@ -85,7 +86,9 @@ _KERNELS = {"unmore_crop_resize": 1, "unmore_crop_resize_aa": 2, "unmore_mask_re
             "unmore_score_and_rasterise": 1, "unmore_mask_resize": 1, "unmore_final_scores": 1, "unmore_sat_build": 1, "unmore_sat_build_fields": 1, "unmore_box_sums": 1,
             "unmore_mask_pack": 1, "unmore_mask_stats": 1, "unmore_mask_nms": 3, "unmore_mask_rle_counts": 1,
             "unmore_pack_detections": 1, "unmore_tile_means": 1, "unmore_center_reasoning_from_tiles": 1,
-            "unmore_boundary_round_from_tiles": 2, "unmore_score_and_rasterise_from_tiles": 1}
+            "unmore_boundary_round_from_tiles": 2, "unmore_score_and_rasterise_from_tiles": 1,
+            "unmore_existence_scores_hw": 1, "unmore_center_reasoning_hw": 1, "unmore_boundary_refine_hw": 1,
+            "unmore_score_and_rasterise_hw": 1, "unmore_box_sums_hw": 1, "unmore_sat_build_fields_hw": 1}
 
 
 def set_timer(t: Optional[StageTimer]):
@@ -136,20 +139,88 @@ def _check_counts(counts: Optional[torch.Tensor], n_img: int):
         raise _lib.UnmoreError("counts must be a CUDA int32 tensor of n_img entries")
 
 
+def _check_extents(image_hw, n_img: int, device, what: str = "", antialias: bool = False) -> torch.Tensor:
+    """The (h, w) table of a padded stack: a CUDA int32 [n_img, 2] tensor on the fields' device, 8-byte aligned.  Its
+    values are not read on the host (no sync); the kernels clamp them to [1, pitch]."""
+    if antialias:
+        raise _lib.UnmoreError(f"{what}: image_hw (images of different sizes) is not supported with antialias=True")
+    if not torch.is_tensor(image_hw) or not image_hw.is_cuda or image_hw.dtype != torch.int32 or \
+            tuple(image_hw.shape) != (n_img, 2):
+        raise _lib.UnmoreError(f"{what}: image_hw must be a CUDA int32 [n_img, 2] tensor of (h, w) per image")
+    if image_hw.device != torch.device(device):
+        raise _lib.UnmoreError(f"{what}: image_hw must live on the device of the fields")
+    image_hw = image_hw.contiguous()
+    return image_hw if image_hw.data_ptr() % 8 == 0 else image_hw.clone()
+
+
+def pack_fields(images):
+    """Pads a list of [C, h_i, w_i] fp32 field stacks with zeros into one stack of images of different sizes:
+    -> (fields [B, C, Hp, Wp], image_hw [B, 2] int32 (h_i, w_i)), both on the device of the first image; (Hp, Wp), the
+    pitch, is the largest h and w of the batch.  Image i is ``fields[i, :, :h_i, :w_i]``; no result of the ops that
+    take ``image_hw`` depends on the padding."""
+    images = list(images)
+    if not images:
+        raise _lib.UnmoreError("pack_fields: empty list")
+    for im in images:
+        if not torch.is_tensor(im) or im.dim() != 3:
+            raise _lib.UnmoreError("pack_fields: every image must be a 3-D [C, h, w] tensor")
+        if im.dtype != torch.float32:
+            raise _lib.UnmoreError("pack_fields: every image must be fp32")
+        if im.shape[1] < 1 or im.shape[2] < 1:
+            raise _lib.UnmoreError("pack_fields: empty image")
+    C = images[0].shape[0]
+    if any(im.shape[0] != C for im in images):
+        raise _lib.UnmoreError("pack_fields: all images must have the same number of channels")
+    dev = images[0].device
+    Hp, Wp = max(im.shape[1] for im in images), max(im.shape[2] for im in images)
+    fields = torch.zeros((len(images), C, Hp, Wp), dtype=torch.float32, device=dev)
+    for i, im in enumerate(images):
+        fields[i, :, : im.shape[1], : im.shape[2]] = im.to(dev)
+    hw = torch.tensor([[im.shape[1], im.shape[2]] for im in images], dtype=torch.int32).to(dev)
+    return fields, hw
+
+
+def stack_proposals(proposals, device=None):
+    """Ragged proposal lists [n_i, 4] (tensors or arrays) -> (boxes [B, max n_i, 4], counts [B] int32), on ``device``
+    (default: that of the first tensor).  fp64 unless every list is fp32; rows past a count are zero."""
+    lists = [p if torch.is_tensor(p) else torch.as_tensor(p) for p in proposals]
+    if not lists:
+        raise _lib.UnmoreError("stack_proposals: empty list")
+    if any(p.dim() != 2 or p.shape[1] != 4 for p in lists if p.numel()) or any(p.numel() % 4 for p in lists):
+        raise _lib.UnmoreError("stack_proposals: every list must be [n, 4]")
+    lists = [p.reshape(-1, 4) for p in lists]
+    dev = torch.device(device) if device is not None else lists[0].device
+    dtype = torch.float32 if all(p.dtype == torch.float32 for p in lists) else torch.float64
+    n = max(p.shape[0] for p in lists)
+    boxes = torch.zeros((len(lists), n, 4), dtype=dtype, device=dev)
+    for i, p in enumerate(lists):
+        if p.shape[0]:
+            boxes[i, : p.shape[0]] = p.to(dev, dtype)
+    counts = torch.tensor([p.shape[0] for p in lists], dtype=torch.int32).to(dev)
+    return boxes, counts
+
+
 def workspace(n_img: int, device) -> torch.Tensor:
     n = _lib.load().unmore_workspace_bytes(n_img)
     return torch.empty((n + 3) // 4, dtype=torch.int32, device=device)
 
 
 def existence_scores(fields, boxes, counts=None, ch: Channels = DEFAULT_CHANNELS, ws=None, out=None,
-                     antialias: bool = False):
+                     antialias: bool = False, image_hw=None):
     """Existence score [n_img, cap] fp32 of every proposal: the mean of its resized crop of the existence channel
-    (``antialias=True``: the second resize mode, equal to ``tile_means`` of ``crop_resize(..., antialias=True)``)."""
+    (``antialias=True``: the second resize mode, equal to ``tile_means`` of ``crop_resize(..., antialias=True)``).
+    ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes (``pack_fields``)."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     ws = workspace(n_img, fields.device) if ws is None else ws
     out = torch.zeros((n_img, cap), dtype=torch.float32, device=fields.device) if out is None else out
+    if image_hw is not None:
+        hw = _check_extents(image_hw, n_img, fields.device, "existence_scores", antialias)
+        _on(fields)
+        _call("unmore_existence_scores_hw", fields.data_ptr(), n_img, C, H, W, hw.data_ptr(), ch.exist, boxes.data_ptr(), f64,
+              _ptr(counts), cap, out.data_ptr(), ws.data_ptr(), _stream(), counts=counts)
+        return out
     _call("unmore_existence_scores_aa" if antialias else "unmore_existence_scores", fields.data_ptr(), n_img, C, H, W, ch.exist, boxes.data_ptr(), f64,
               _ptr(counts), cap, out.data_ptr(), ws.data_ptr(), _stream(), counts=counts)
     return out
@@ -189,19 +260,22 @@ CENTER_AA_SLICE_BYTES = 1 << 30   # tiles + resampling scratch of one slice of c
 
 
 def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channels = DEFAULT_CHANNELS, ws=None,
-                     want_splits: bool = True, analyze_cc: bool = False, antialias: bool = False):
+                     want_splits: bool = True, analyze_cc: bool = False, antialias: bool = False, image_hw=None):
     """-> (max_values [n_img,cap] fp64, argmax [n_img,cap] int32 (-1 = passes), splits [n_img,cap,4,4] fp64 or None,
     cc) where cc is None or (cc_counts [n_img,cap] u8, cc_boxes [n_img,cap,CC_CAP,4] fp64, overflow [1] int32).
     ``antialias=True`` (the second resize mode) has no fused kernel: it resamples antialiased tiles and runs
     ``center_reasoning_from_tiles`` on them, in slices of the proposal capacity so that the tiles and their
     scratch stay within CENTER_AA_SLICE_BYTES; the counts are clamped per slice on the device (no host sync).  A slice
     is at least one proposal of every image, so the bound holds up to ~1150 images per call at 480 px field height.
-    Slices walk the whole capacity whatever the counts, so most of them are empty on split lists."""
+    Slices walk the whole capacity whatever the counts, so most of them are empty on split lists.
+    ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes (``pack_fields``); the
+    --analyze_cc boxes are clipped against each image's own size."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = fields.device
     ws = workspace(n_img, dev) if ws is None else ws
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "center_reasoning", antialias)
     if antialias:
         return _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc)
     maxv = torch.zeros((n_img, cap), dtype=torch.float64, device=dev)
@@ -213,7 +287,9 @@ def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channel
         cc = (torch.zeros((n_img, cap), dtype=torch.uint8, device=dev),
               torch.zeros((n_img, cap, cc_cap, 4), dtype=torch.float64, device=dev),
               torch.zeros((1,), dtype=torch.int32, device=dev))
-    _call("unmore_center_reasoning", fields.data_ptr(), n_img, C, H, W, ch.sdf, ch.center_row, ch.center_col,
+    _on(fields)
+    name, size = ("unmore_center_reasoning", (H, W)) if hw is None else ("unmore_center_reasoning_hw", (H, W, hw.data_ptr()))
+    _call(name, fields.data_ptr(), n_img, C, *size, ch.sdf, ch.center_row, ch.center_col,
           boxes.data_ptr(), f64, _ptr(counts), cap, float(thr), maxv.data_ptr(), argmax.data_ptr(),
           _ptr(splits), _ptr(cc[0]) if cc else None, _ptr(cc[1]) if cc else None, _ptr(cc[2]) if cc else None,
           ws.data_ptr(), _stream(), counts=counts)
@@ -265,19 +341,23 @@ def _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyz
 def boundary_refine(fields, boxes, counts=None, n_round: int = 50, apply_small_filter: bool = True,
                     early_exit: bool = True, proposal_area_thres: float = 50.0, max_sdf_thres: float = 0.5,
                     max_shrink_threshold: float = 16.0, delta_ratio: float = 0.5, ch: Channels = DEFAULT_CHANNELS,
-                    ws=None, want_rounds: bool = True, antialias: bool = False):
+                    ws=None, want_rounds: bool = True, antialias: bool = False, image_hw=None):
     """Up to ``n_round`` rounds of boundary reasoning per proposal -> (boxes [n_img,cap,4] fp32, labels [n_img,cap]
     fp32 (-2 = removed by the area filter), rounds [n_img,cap] int32 or None); ``antialias=True``: the second
-    resize mode."""
+    resize mode.  ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes
+    (``pack_fields``); boxes are clipped against, and glued to, each image's own edges."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = fields.device
     ws = workspace(n_img, dev) if ws is None else ws
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "boundary_refine", antialias)
     out = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     labels = torch.full((n_img, cap), -2.0, dtype=torch.float32, device=dev)
     rounds = torch.zeros((n_img, cap), dtype=torch.int32, device=dev) if want_rounds else None
-    _call("unmore_boundary_refine_aa" if antialias else "unmore_boundary_refine", fields.data_ptr(), n_img, C, H, W, ch.sdf,
+    _on(fields)
+    name = "unmore_boundary_refine_aa" if antialias else "unmore_boundary_refine" if hw is None else "unmore_boundary_refine_hw"
+    _call(name, fields.data_ptr(), n_img, C, H, W, *(() if hw is None else (hw.data_ptr(),)), ch.sdf,
               boxes.data_ptr(), f64,
               _ptr(counts), cap, int(n_round), int(apply_small_filter), int(early_exit), float(proposal_area_thres),
               float(max_sdf_thres), float(max_shrink_threshold), float(delta_ratio), out.data_ptr(),
@@ -381,19 +461,25 @@ def anti_center_map(vote_maps: torch.Tensor, kernel_size: int = 5) -> torch.Tens
     return out
 
 
-def score_and_rasterise(fields, boxes, counts=None, ch: Channels = DEFAULT_CHANNELS, want_masks: bool = True):
+def score_and_rasterise(fields, boxes, counts=None, ch: Channels = DEFAULT_CHANNELS, want_masks: bool = True,
+                        image_hw=None):
     """-> scores [n_img,cap,4] (existence, center, boundary, 0), tight xyxy [n_img,cap,4], areas [n_img,cap],
-    packed masks [n_img,cap,H,ceil(W/32)] int32 (or None)."""
+    packed masks [n_img,cap,H,ceil(W/32)] int32 (or None).  ``image_hw`` [n_img, 2] int32: ``fields`` is a padded
+    stack of images of different sizes (``pack_fields``); the masks stay on the pitched canvas, image i's mask is
+    ``masks[i, :, :h_i, :ceil(w_i/32)]`` and every bit outside the image is 0."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = fields.device
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "score_and_rasterise")
     scores = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     tight = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     areas = torch.zeros((n_img, cap), dtype=torch.int32, device=dev)
     masks = torch.zeros((n_img, cap, H, (W + 31) // 32), dtype=torch.int32, device=dev) if want_masks else None
     if cap > 0:
-        _call("unmore_score_and_rasterise", fields.data_ptr(), n_img, C, H, W, ch.sdf, ch.center_row, ch.center_col,
+        _on(fields)
+        name, size = ("unmore_score_and_rasterise", (H, W)) if hw is None else ("unmore_score_and_rasterise_hw", (H, W, hw.data_ptr()))
+        _call(name, fields.data_ptr(), n_img, C, *size, ch.sdf, ch.center_row, ch.center_col,
                   ch.exist, boxes.data_ptr(), f64, _ptr(counts), cap, scores.data_ptr(), tight.data_ptr(),
                   areas.data_ptr(), _ptr(masks), _stream())
     return scores, tight, areas, masks
@@ -443,25 +529,42 @@ def sat_build(planes: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def sat_build_fields(fields: torch.Tensor, channels, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+def sat_build_fields(fields: torch.Tensor, channels, out: Optional[torch.Tensor] = None, image_hw=None) -> torch.Tensor:
     """Tables of selected channels straight from the field stack: [n_img, C, H, W] fp32 ->
-    [n_img, len(channels), H+1, W+1] fp64 (no gather copy)."""
+    [n_img, len(channels), H+1, W+1] fp64 (no gather copy).  ``image_hw`` [n_img, 2] int32: ``fields`` is a padded
+    stack (``pack_fields``) and the padding enters the sums as zeros, so entries [:h_i+1, :w_i+1] of image i's tables
+    are those of the image alone."""
     import ctypes
     n_img, C, H, W = _check_fields(fields)
     ch = (ctypes.c_int * len(channels))(*[int(c) for c in channels])
     if out is None:
         out = torch.empty((n_img, len(channels), H + 1, W + 1), dtype=torch.float64, device=fields.device)
+    if image_hw is not None:
+        hw = _check_extents(image_hw, n_img, fields.device, "sat_build_fields")
+        _on(fields)
+        _call("unmore_sat_build_fields_hw", fields.data_ptr(), n_img, C, H, W, hw.data_ptr(), ctypes.cast(ch, ctypes.c_void_p),
+              len(channels), out.data_ptr(), _stream())
+        return out
     _call("unmore_sat_build_fields", fields.data_ptr(), n_img, C, H, W, ctypes.cast(ch, ctypes.c_void_p), len(channels),
           out.data_ptr(), _stream())
     return out
 
 
-def box_sums(sat: torch.Tensor, plane: int, boxes: torch.Tensor, counts=None):
-    """sat [n_img, P, H+1, W+1] fp64, boxes [n_img, cap, 4] -> (sums, means) [n_img, cap] fp64."""
+def box_sums(sat: torch.Tensor, plane: int, boxes: torch.Tensor, counts=None, image_hw=None):
+    """sat [n_img, P, H+1, W+1] fp64, boxes [n_img, cap, 4] -> (sums, means) [n_img, cap] fp64.  ``image_hw``
+    [n_img, 2] int32: the tables are those of a padded stack (``sat_build_fields(..., image_hw=)``); windows snap to
+    each image's own size."""
     n_img, P, H1, W1 = _on(sat).shape
     cap, f64 = _check_boxes(boxes, n_img)
     sums = torch.zeros((n_img, cap), dtype=torch.float64, device=sat.device)
     means = torch.zeros((n_img, cap), dtype=torch.float64, device=sat.device)
+    if image_hw is not None:
+        hw = _check_extents(image_hw, n_img, sat.device, "box_sums")
+        if cap > 0:
+            _on(sat)
+            _call("unmore_box_sums_hw", sat.data_ptr(), n_img, P, int(plane), H1 - 1, W1 - 1, hw.data_ptr(), boxes.data_ptr(), f64,
+                  _ptr(counts), cap, sums.data_ptr(), means.data_ptr(), _stream())
+        return sums, means
     if cap > 0:
         _call("unmore_box_sums", sat.data_ptr(), n_img, P, int(plane), H1 - 1, W1 - 1, boxes.data_ptr(), f64,
                   _ptr(counts), cap, sums.data_ptr(), means.data_ptr(), _stream())
