@@ -297,7 +297,14 @@ int unmore_mask_nms(const uint32_t* masks, int K, int H, int W, const float* sco
  * Masks of unmore_score_and_rasterise_hw stay on the pitched canvas [n_img, cap, H, ceil(W/32)]: image i's are the
  * [:h_i, :ceil(w_i/32)] corner, every bit outside the image is 0.  unmore_sat_build_fields_hw reads the padding as
  * zeros, so entries [:h_i+1, :w_i+1] of image i's tables are those of the image alone; unmore_box_sums_hw takes such
- * tables.  A null, misaligned, host or other-device image_hw is rejected (UNMORE_E_INVALID) before anything runs. */
+ * tables.  A null, misaligned, host or other-device image_hw is rejected (UNMORE_E_INVALID) before anything runs.
+ *
+ * The second resize mode (antialias=True) has the same five forms: unmore_existence_scores_aa_hw,
+ * unmore_boundary_refine_aa_hw, unmore_crop_resize_aa_hw, unmore_center_reasoning_from_tiles_hw and
+ * unmore_score_and_rasterise_from_tiles_hw, each with image_hw after W.  unmore_crop_resize_aa_hw snaps every window
+ * to its image and sizes its scratch by the pitch (n_img*cap*n_channels*H*128 floats).  The two *_from_tiles_hw calls
+ * take tiles cropped from the stack by unmore_crop_resize_aa_hw and the pitch as (H, W): the extents give the window
+ * snap behind the split boxes, the --analyze_cc clip and the mask raster, whose canvas is the pitched one above. */
 int unmore_existence_scores_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_exist,
                                const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out,
                                void* ws, unmore_stream_t stream);
@@ -322,6 +329,29 @@ int unmore_box_sums_hw(const double* sat, int n_img, int planes_per_img, int pla
                        double* sums_out, double* means_out, unmore_stream_t stream);
 int unmore_sat_build_fields_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
                                const int* channels_host, int n_channels, double* out, unmore_stream_t stream);
+int unmore_existence_scores_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                                  int ch_exist, const void* boxes, int boxes_f64, const int* counts, int cap,
+                                  float* scores_out, void* ws, unmore_stream_t stream);
+int unmore_boundary_refine_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                                 const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
+                                 int apply_small_filter, int early_exit, float proposal_area_thres,
+                                 float max_sdf_thres, float max_shrink_threshold, float delta_ratio,
+                                 float* boxes_out, float* labels_out, int* rounds_out, void* ws,
+                                 unmore_stream_t stream);
+int unmore_crop_resize_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                             const int* channels_host, int n_channels, const void* boxes, int boxes_f64,
+                             const int* counts, int cap, float* out, void* scratch, size_t scratch_bytes,
+                             unmore_stream_t stream);
+int unmore_center_reasoning_from_tiles_hw(const float* tiles, int n_img, int H, int W, const int* image_hw,
+                                          const void* boxes, int boxes_f64, const int* counts, int cap,
+                                          double center_score_max_thres, double* max_values_out, int* argmax_out,
+                                          double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out,
+                                          int* cc_overflow, void* ws, unmore_stream_t stream);
+int unmore_score_and_rasterise_from_tiles_hw(const float* tiles, const float* existence_scores, int antialias,
+                                             int n_img, int H, int W, const int* image_hw, const void* boxes,
+                                             int boxes_f64, const int* counts, int cap, float* scores_out,
+                                             float* tight_out, int* areas_out, uint32_t* masks_out,
+                                             unmore_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -3,11 +3,11 @@
   (b) same_size  - batches of identical size only, through the uniform path;
   (c) padded     - padded mixed batches (ops.pack_fields + image_hw) of --batch images.
 Plus a uniform 480x640 batch through the sized (*_hw) kernels against the uniform ones.  Asserts that all ways give
-identical outputs and prints one JSON line.
+identical outputs and prints one JSON line.  --antialias runs all of it in the second resize mode (antialias=True).
 
 The shape table below is a plausible mix of photo shapes with a 640-px longer side (4:3, 3:2, 16:9, portrait, square)
 plus a few small images.  It is NOT COCO's measured size distribution.
-usage: python scripts/mixed_size_throughput.py [--images 250] [--batch 250] [--proposals 4096] [--seed 0]"""
+usage: python scripts/mixed_size_throughput.py [--images 250] [--batch 250] [--proposals 4096] [--seed 0] [--antialias]"""
 import argparse
 import json
 import os
@@ -71,6 +71,7 @@ def main():
     ap.add_argument("--batch", type=int, default=250)
     ap.add_argument("--proposals", type=int, default=4096)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--antialias", action="store_true", help="the second resize mode (antialias=True)")
     a = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("needs a CUDA device")
@@ -78,7 +79,8 @@ def main():
     shapes = draw_shapes(a.images, a.seed)
     images = [synth.make_fields(i, h, w).to(dev) for i, (h, w) in enumerate(shapes)]
     props = [torch.from_numpy(synth.make_proposals(i, a.proposals, h, w)).to(dev) for i, (h, w) in enumerate(shapes)]
-    od, osc = Object_Discovery(default_args(), device=dev), Object_Scoring(device=dev)
+    od = Object_Discovery(default_args(antialias=a.antialias), device=dev)
+    osc = Object_Scoring(argparse.Namespace(antialias=a.antialias), device=dev)
 
     def per_image():
         return [outputs(*run_batch(od, osc, im[None].contiguous(), p[None].contiguous(), None), 0, *im.shape[1:])
@@ -116,7 +118,7 @@ def main():
     bx, ct = ops.stack_proposals(props[:n_warm], dev)
     run_batch(od, osc, f, bx, ct, hw)
 
-    result = {"images": a.images, "batch": a.batch, "proposals_per_image": a.proposals, "ways": {}}
+    result = {"images": a.images, "batch": a.batch, "proposals_per_image": a.proposals, "antialias": a.antialias, "ways": {}}
     outs = {}
     torch.cuda.reset_peak_memory_stats()
     for name, fn in (("per_image", per_image), ("same_size", same_size), ("padded", padded)):
@@ -153,7 +155,7 @@ def main():
                                  "runs_s": {k: [round(t, 4) for t in v] for k, v in times.items()}}
     try:
         import subprocess
-        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
                            capture_output=True, text=True).stdout.strip()
     except OSError:
         q = ""

@@ -117,8 +117,8 @@ int check_extents(const char* name, const int* image_hw) {
   return 0;
 }
 
-// unmore_existence_scores / unmore_existence_scores_aa / unmore_existence_scores_hw: the same call in either resize
-// mode, and on a padded stack (image_hw non-null)
+// unmore_existence_scores / unmore_existence_scores_aa and their _hw forms: the same call in either resize mode, and
+// on a padded stack (image_hw non-null)
 int existence_scores(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_exist,
                      const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
                      cudaStream_t s, const int* image_hw = nullptr) {
@@ -134,7 +134,7 @@ int existence_scores(const char* name, bool aa, const float* fields, int n_img, 
   return cuda_fail(launch_existence(p, num_sms(), s), "existence_kernel");
 }
 
-// unmore_boundary_refine / unmore_boundary_refine_aa / unmore_boundary_refine_hw
+// unmore_boundary_refine / unmore_boundary_refine_aa and their _hw forms
 int boundary_refine(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_sdf,
                     const void* boxes, int boxes_f64, const int* counts, int cap, int n_round, int apply_small_filter,
                     int early_exit, float proposal_area_thres, float max_sdf_thres, float max_shrink_threshold,
@@ -157,7 +157,7 @@ int boundary_refine(const char* name, bool aa, const float* fields, int n_img, i
     const int e = (int)cudaMemsetAsync(p.windows, 0, sizeof(WindowSlot) * kWindowSlots * (size_t)n_img, s);
     if (e) return cuda_fail(e, "memset window tables");
   }
-  if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s), "refine_aa_kernel");
+  if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s, image_hw), "refine_aa_kernel");
   return cuda_fail(launch_refine(p, num_sms(), s, image_hw), "refine_kernel");
 }
 
@@ -217,6 +217,59 @@ int box_sums(const char* name, const double* sat, int n_img, int planes_per_img,
                    "box_sums_kernel");
 }
 
+// unmore_crop_resize_aa / unmore_crop_resize_aa_hw
+int crop_resize_aa(const char* name, const float* fields, int n_img, int C, int H, int W, const int* channels_host,
+                   int n_channels, const void* boxes, int boxes_f64, const int* counts, int cap, float* out, void* scratch,
+                   size_t scratch_bytes, cudaStream_t s, const int* image_hw = nullptr) {
+  if (int e = check_fields(fields, n_img, C, H, W)) return e;
+  if (!boxes || !out || !channels_host || cap < 0 || n_channels < 1 || n_channels > 4)
+    return fail(UNMORE_E_INVALID, "%s: bad argument (1..4 channels)", name);
+  for (int i = 0; i < n_channels; ++i)
+    if (channels_host[i] < 0 || channels_host[i] >= C) return fail(UNMORE_E_INVALID, "%s: channel out of range", name);
+  const size_t need = (size_t)n_img * cap * n_channels * H * 128 * sizeof(float);
+  if (need && (!scratch || scratch_bytes < need))
+    return fail(UNMORE_E_CAPACITY, "%s: scratch must hold n_img*cap*n_channels*H*128 floats (%zu bytes)", name, need);
+  return cuda_fail(launch_crop_resize_aa(fields, n_img, C, H, W, channels_host, n_channels, boxes, boxes_f64, counts, cap, out,
+                                         reinterpret_cast<float*>(scratch), s, image_hw),
+                   "crop_resize_aa kernels");
+}
+
+// unmore_center_reasoning_from_tiles / unmore_center_reasoning_from_tiles_hw
+int center_from_tiles(const char* name, const float* tiles, int n_img, int H, int W, const void* boxes, int boxes_f64,
+                      const int* counts, int cap, double center_score_max_thres, double* max_values_out, int* argmax_out,
+                      double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow, void* ws,
+                      cudaStream_t s, const int* image_hw = nullptr) {
+  if (!tiles || !boxes || !max_values_out || !argmax_out || !ws || cap < 0 || n_img <= 0 || H <= 0 || W <= 0)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (cap == 0) return 0;
+  CenterParams p{};
+  p.tiles = tiles; p.C = 3; p.H = H; p.W = W; p.ch_sdf = 0; p.ch_crow = 1; p.ch_ccol = 2;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.thr = center_score_max_thres;
+  p.max_values = max_values_out; p.argmax = argmax_out; p.splits = splits_out;
+  if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
+    return fail(UNMORE_E_INVALID, "%s: the three analyze_cc outputs go together", name);
+  p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
+  p.image_hw = image_hw;
+  center_filters(p);
+  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  return cuda_fail(launch_center(p, num_sms(), s), "center_kernel (tiles)");
+}
+
+// unmore_score_and_rasterise_from_tiles / unmore_score_and_rasterise_from_tiles_hw
+int score_from_tiles(const char* name, const float* tiles, const float* existence_scores, int antialias, int n_img, int H,
+                     int W, const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, float* tight_out,
+                     int* areas_out, uint32_t* masks_out, cudaStream_t s, const int* image_hw = nullptr) {
+  if (!tiles || !boxes || !scores_out || !tight_out || !areas_out || cap < 0 || n_img <= 0 || H <= 0 || W <= 0)
+    return fail(UNMORE_E_INVALID, "%s: bad argument", name);
+  if (n_img > 65535) return fail(UNMORE_E_CAPACITY, "%s: n_img > 65535 per call", name);
+  ScoreParams p{};
+  p.tiles = tiles; p.exist_scores = existence_scores; p.aa_raster = antialias; p.n_img = n_img; p.C = 4; p.H = H; p.W = W;
+  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
+  p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
+  p.areas = areas_out; p.masks = masks_out;
+  return cuda_fail(launch_score(p, s, image_hw), "score_kernel (tiles)");
+}
+
 }  // namespace
 
 extern "C" {
@@ -257,17 +310,8 @@ int unmore_crop_resize(const float* fields, int n_img, int C, int H, int W, cons
 int unmore_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, const int* channels_host, int n_channels,
                           const void* boxes, int boxes_f64, const int* counts, int cap, float* out, void* scratch,
                           size_t scratch_bytes, unmore_stream_t stream) {
-  if (int e = check_fields(fields, n_img, C, H, W)) return e;
-  if (!boxes || !out || !channels_host || cap < 0 || n_channels < 1 || n_channels > 4)
-    return fail(UNMORE_E_INVALID, "unmore_crop_resize_aa: bad argument (1..4 channels)");
-  for (int i = 0; i < n_channels; ++i)
-    if (channels_host[i] < 0 || channels_host[i] >= C) return fail(UNMORE_E_INVALID, "unmore_crop_resize_aa: channel out of range");
-  const size_t need = (size_t)n_img * cap * n_channels * H * 128 * sizeof(float);
-  if (need && (!scratch || scratch_bytes < need))
-    return fail(UNMORE_E_CAPACITY, "unmore_crop_resize_aa: scratch must hold n_img*cap*n_channels*H*128 floats (%zu bytes)", need);
-  return cuda_fail(launch_crop_resize_aa(fields, n_img, C, H, W, channels_host, n_channels, boxes, boxes_f64, counts, cap, out,
-                                         reinterpret_cast<float*>(scratch), (cudaStream_t)stream),
-                   "crop_resize_aa kernels");
+  return crop_resize_aa("unmore_crop_resize_aa", fields, n_img, C, H, W, channels_host, n_channels, boxes, boxes_f64, counts,
+                        cap, out, scratch, scratch_bytes, (cudaStream_t)stream);
 }
 
 int unmore_mask_resize_aa(const unsigned char* masks, int B, int H, int W, int out_h, int out_w, unsigned char* out,
@@ -328,20 +372,9 @@ int unmore_center_reasoning_from_tiles(const float* tiles, int n_img, int H, int
                                        const int* counts, int cap, double center_score_max_thres, double* max_values_out,
                                        int* argmax_out, double* splits_out, unsigned char* cc_counts_out,
                                        double* cc_boxes_out, int* cc_overflow, void* ws, unmore_stream_t stream) {
-  if (!tiles || !boxes || !max_values_out || !argmax_out || !ws || cap < 0 || n_img <= 0 || H <= 0 || W <= 0)
-    return fail(UNMORE_E_INVALID, "unmore_center_reasoning_from_tiles: bad argument");
-  if (cap == 0) return 0;
-  cudaStream_t s = (cudaStream_t)stream;
-  CenterParams p{};
-  p.tiles = tiles; p.C = 3; p.H = H; p.W = W; p.ch_sdf = 0; p.ch_crow = 1; p.ch_ccol = 2;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.thr = center_score_max_thres;
-  p.max_values = max_values_out; p.argmax = argmax_out; p.splits = splits_out;
-  if ((cc_counts_out != nullptr) != (cc_boxes_out != nullptr) || (cc_counts_out != nullptr) != (cc_overflow != nullptr))
-    return fail(UNMORE_E_INVALID, "unmore_center_reasoning_from_tiles: the three analyze_cc outputs go together");
-  p.cc_counts = cc_counts_out; p.cc_boxes = cc_boxes_out; p.cc_overflow = cc_overflow;
-  center_filters(p);
-  if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
-  return cuda_fail(launch_center(p, num_sms(), s), "center_kernel (tiles)");
+  return center_from_tiles("unmore_center_reasoning_from_tiles", tiles, n_img, H, W, boxes, boxes_f64, counts, cap,
+                           center_score_max_thres, max_values_out, argmax_out, splits_out, cc_counts_out, cc_boxes_out,
+                           cc_overflow, ws, (cudaStream_t)stream);
 }
 
 int unmore_boundary_round_from_tiles(const float* tiles, int M, const void* boxes, int boxes_f64, int H, int W,
@@ -364,15 +397,8 @@ int unmore_score_and_rasterise_from_tiles(const float* tiles, const float* exist
                                           int W, const void* boxes, int boxes_f64, const int* counts, int cap,
                                           float* scores_out, float* tight_out, int* areas_out, uint32_t* masks_out,
                                           unmore_stream_t stream) {
-  if (!tiles || !boxes || !scores_out || !tight_out || !areas_out || cap < 0 || n_img <= 0 || H <= 0 || W <= 0)
-    return fail(UNMORE_E_INVALID, "unmore_score_and_rasterise_from_tiles: bad argument");
-  if (n_img > 65535) return fail(UNMORE_E_CAPACITY, "unmore_score_and_rasterise_from_tiles: n_img > 65535 per call");
-  ScoreParams p{};
-  p.tiles = tiles; p.exist_scores = existence_scores; p.aa_raster = antialias; p.n_img = n_img; p.C = 4; p.H = H; p.W = W;
-  p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
-  p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
-  p.areas = areas_out; p.masks = masks_out;
-  return cuda_fail(launch_score(p, (cudaStream_t)stream), "score_kernel (tiles)");
+  return score_from_tiles("unmore_score_and_rasterise_from_tiles", tiles, existence_scores, antialias, n_img, H, W, boxes,
+                          boxes_f64, counts, cap, scores_out, tight_out, areas_out, masks_out, (cudaStream_t)stream);
 }
 
 int unmore_cc_cap(void) { return kCcCap; }
@@ -605,6 +631,59 @@ int unmore_sat_build_fields_hw(const float* fields, int n_img, int C, int H, int
   if (W > 2048) return fail(UNMORE_E_CAPACITY, "%s: W %d > 2048", name, W);
   return cuda_fail(launch_sat_hw(fields, out, n_img, H, W, C, channels_host, n_channels, image_hw, (cudaStream_t)stream),
                    "sat_hw_kernel");
+}
+
+// the second resize mode (antialias=True) on a padded stack
+int unmore_existence_scores_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_exist,
+                                  const void* boxes, int boxes_f64, const int* counts, int cap, float* scores_out, void* ws,
+                                  unmore_stream_t stream) {
+  const char* name = "unmore_existence_scores_aa_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return existence_scores(name, true, fields, n_img, C, H, W, ch_exist, boxes, boxes_f64, counts, cap, scores_out, ws,
+                          (cudaStream_t)stream, image_hw);
+}
+
+int unmore_boundary_refine_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                                 const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
+                                 int apply_small_filter, int early_exit, float proposal_area_thres, float max_sdf_thres,
+                                 float max_shrink_threshold, float delta_ratio, float* boxes_out, float* labels_out,
+                                 int* rounds_out, void* ws, unmore_stream_t stream) {
+  const char* name = "unmore_boundary_refine_aa_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return boundary_refine(name, true, fields, n_img, C, H, W, ch_sdf, boxes, boxes_f64, counts, cap, n_round,
+                         apply_small_filter, early_exit, proposal_area_thres, max_sdf_thres, max_shrink_threshold,
+                         delta_ratio, boxes_out, labels_out, rounds_out, ws, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_crop_resize_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                             const int* channels_host, int n_channels, const void* boxes, int boxes_f64, const int* counts,
+                             int cap, float* out, void* scratch, size_t scratch_bytes, unmore_stream_t stream) {
+  const char* name = "unmore_crop_resize_aa_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return crop_resize_aa(name, fields, n_img, C, H, W, channels_host, n_channels, boxes, boxes_f64, counts, cap, out, scratch,
+                        scratch_bytes, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_center_reasoning_from_tiles_hw(const float* tiles, int n_img, int H, int W, const int* image_hw,
+                                          const void* boxes, int boxes_f64, const int* counts, int cap,
+                                          double center_score_max_thres, double* max_values_out, int* argmax_out,
+                                          double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out,
+                                          int* cc_overflow, void* ws, unmore_stream_t stream) {
+  const char* name = "unmore_center_reasoning_from_tiles_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return center_from_tiles(name, tiles, n_img, H, W, boxes, boxes_f64, counts, cap, center_score_max_thres, max_values_out,
+                           argmax_out, splits_out, cc_counts_out, cc_boxes_out, cc_overflow, ws, (cudaStream_t)stream,
+                           image_hw);
+}
+
+int unmore_score_and_rasterise_from_tiles_hw(const float* tiles, const float* existence_scores, int antialias, int n_img,
+                                             int H, int W, const int* image_hw, const void* boxes, int boxes_f64,
+                                             const int* counts, int cap, float* scores_out, float* tight_out,
+                                             int* areas_out, uint32_t* masks_out, unmore_stream_t stream) {
+  const char* name = "unmore_score_and_rasterise_from_tiles_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return score_from_tiles(name, tiles, existence_scores, antialias, n_img, H, W, boxes, boxes_f64, counts, cap, scores_out,
+                          tight_out, areas_out, masks_out, (cudaStream_t)stream, image_hw);
 }
 
 }  // extern "C"

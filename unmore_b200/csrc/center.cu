@@ -225,8 +225,9 @@ struct CenterTileRows {
 
 // PLANE_ELEMS: 0 = any field size / channel order; H*W = the three channels are consecutive planes of a field
 // of exactly that size (the COCO-val shape the batch path runs on), see MultiPlaneRows.
-// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window snap and the
-// --analyze_cc clip use the image's extent; plane addressing and PLANE_ELEMS go by the pitch.
+// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window snap (and with it
+// the split boxes) and the --analyze_cc clip use the image's extent; plane addressing and PLANE_ELEMS go by the pitch.
+// On tiles (PLANE_ELEMS = -1) only the snap and the clip change.
 constexpr int kSpecPlaneElems = 480 * 640;
 template <bool ANALYZE_CC, int PLANE_ELEMS, bool ROW_SKIP, bool SIZED = false>
 __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterParams p) {
@@ -784,13 +785,11 @@ int launch_components(const unsigned char* masks, int B, int* counts, int* boxes
 template <bool CC, int PE, bool RS = false>
 static int launch_center_t(const CenterParams& p, int num_sms, cudaStream_t stream) {
   // function attributes are per device: set on every launch (microseconds), no cached state
-  if constexpr (PE >= 0) {
-    if (p.image_hw) {   // a padded stack: the sized variant
-      cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CenterSmem));
-      if (e != cudaSuccess) return (int)e;
-      center_kernel<CC, PE, RS, true><<<num_sms * 2, kCenterThreads, sizeof(CenterSmem), stream>>>(p);
-      return (int)cudaGetLastError();
-    }
+  if (p.image_hw) {   // a padded stack (fields or tiles): the sized variant
+    cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CenterSmem));
+    if (e != cudaSuccess) return (int)e;
+    center_kernel<CC, PE, RS, true><<<num_sms * 2, kCenterThreads, sizeof(CenterSmem), stream>>>(p);
+    return (int)cudaGetLastError();
   }
   cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CenterSmem));
   if (e != cudaSuccess) return (int)e;

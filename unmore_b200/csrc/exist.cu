@@ -83,9 +83,11 @@ __global__ void __launch_bounds__(kExistWarps * 32) existence_hw_kernel(const Ex
 
 // The second resize mode (antialias=True): the mean of the antialiased crop (aa_rows.cuh), summed in exactly the order
 // above, so the score equals tile_means_kernel on the tile of unmore_crop_resize_aa bit for bit.
+// SIZED: as existence_items; the rows keep the pitch as their stride.
 constexpr int kAaExistWarps = 2;   // 15 KB of shared memory per warp
 constexpr int kAaExistMinBlocks = 7;
-__global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_kernel(const ExistParams p) {
+template <bool SIZED>
+__device__ __forceinline__ void existence_aa_items(const ExistParams& p) {
   __shared__ AaRowsSmem rows_all[kAaExistWarps];
   const int lane = threadIdx.x & 31;
   AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
@@ -99,7 +101,13 @@ __global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existen
     const size_t row = (size_t)img * p.work.cap + k;
     double x1, y1, x2, y2;
     load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
-    const Window win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    Window win;
+    if constexpr (SIZED) {
+      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
+    } else {
+      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
+    }
     float score = 0.f;
     if (!win.empty()) {
       AaCropRows src;
@@ -123,6 +131,13 @@ __global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existen
     }
     if (lane == 0) p.scores[row] = score;
   }
+}
+
+__global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_kernel(const ExistParams p) {
+  existence_aa_items<false>(p);
+}
+__global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_hw_kernel(const ExistParams p) {
+  existence_aa_items<true>(p);
 }
 
 // ---- a2 / a4 as a stand-alone op: the resized crops themselves --------------------------------
@@ -222,7 +237,8 @@ int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream) {
 }
 
 int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream) {
-  existence_aa_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
+  if (p.image_hw) existence_aa_hw_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
+  else existence_aa_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

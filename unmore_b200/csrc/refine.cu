@@ -495,17 +495,27 @@ __global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_hw
 // memory for the weight table and the row ring, so fewer warps fit an SM.
 constexpr int kAaRefineWarps = 2;
 constexpr int kAaRefineMinBlocks = 5;
-__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_kernel(const RefineParams p) {
+template <bool SIZED>
+__device__ __forceinline__ void refine_aa(const RefineParams& p, const int* image_hw) {
   __shared__ BorderCols cols_all[kAaRefineWarps];
   __shared__ AaRowsSmem rows_all[kAaRefineWarps];
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
   AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
-  refine_proposals<false>(p, cols, lane, [&](const float* plane, const Window& win) {
+  refine_proposals<SIZED>(p, cols, lane, [&](const float* plane, const Window& win) {
     AaCropRows src;
     src.init(lane, rows, plane, p.W, win);
     return boundary_terms(src, cols, lane);
-  });
+  }, image_hw);
+}
+
+__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_kernel(const RefineParams p) {
+  refine_aa<false>(p, nullptr);
+}
+// the same on a padded stack, as refine_hw_kernel
+__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_hw_kernel(const RefineParams p,
+                                                                                              const int* __restrict__ image_hw) {
+  refine_aa<true>(p, image_hw);
 }
 
 __global__ void __launch_bounds__(kRefineWarps * 32) tiles_kernel(const TileParams p) {
@@ -564,8 +574,10 @@ int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const
   return (int)cudaGetLastError();
 }
 
-int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream) {
-  refine_aa_kernel<<<num_sms * kAaRefineMinBlocks, kAaRefineWarps * 32, 0, stream>>>(p);
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw) {
+  const int ctas = num_sms * kAaRefineMinBlocks;
+  if (image_hw) refine_aa_hw_kernel<<<ctas, kAaRefineWarps * 32, 0, stream>>>(p, image_hw);
+  else refine_aa_kernel<<<ctas, kAaRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

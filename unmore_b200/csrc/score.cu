@@ -65,8 +65,9 @@ __device__ __forceinline__ bool resized_mask_bit_aa(const uint32_t m[kCrop][4], 
 // of the reference's original mode); the masks are rasterised back to the box with the antialiased kernel when
 // p.aa_raster is set and with the plain one otherwise; p.exist_scores, when given, replaces the mean of the fourth
 // tile (the reference's classifier puts out one scalar per crop, object_scoring.py:140-150).
-// SIZED (fused path only): a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window
-// snaps to the image's extent; the mask canvas stays H x ceil(W/32) words (bits outside the image stay 0).
+// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch (on the tile path, the tiles
+// were cropped from such a stack).  The window snaps to the image's extent; the mask canvas stays H x ceil(W/32) words
+// (bits outside the image stay 0).
 template <bool SIZED> struct ScoreArgs { using type = ScoreParams; };
 template <> struct ScoreArgs<true> { using type = ScoreHwParams; };
 
@@ -257,26 +258,23 @@ int launch_mask_resize(const unsigned char* masks, int B, int oh, int ow, unsign
   return (int)cudaGetLastError();
 }
 
+template <bool TILES_AA, bool SIZED>
+static int launch_score_t(const typename ScoreArgs<SIZED>::type& p, cudaStream_t stream) {
+  cudaError_t e = cudaFuncSetAttribute(score_kernel<TILES_AA, SIZED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
+  if (e != cudaSuccess) return (int)e;
+  score_kernel<TILES_AA, SIZED><<<dim3(p.cap, p.n_img), kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
 int launch_score(const ScoreParams& p, cudaStream_t stream, const int* image_hw) {
   if (p.n_img <= 0 || p.cap <= 0) return 0;
-  dim3 grid(p.cap, p.n_img);
-  if (p.tiles) {
-    cudaError_t e = cudaFuncSetAttribute(score_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
-    if (e != cudaSuccess) return (int)e;
-    score_kernel<true><<<grid, kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
-  } else if (image_hw) {
+  if (image_hw) {
     ScoreHwParams hp;
     static_cast<ScoreParams&>(hp) = p;
     hp.image_hw = image_hw;
-    cudaError_t e = cudaFuncSetAttribute(score_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
-    if (e != cudaSuccess) return (int)e;
-    score_kernel<false, true><<<grid, kScoreThreads, sizeof(ScoreSmem), stream>>>(hp);
-  } else {
-    cudaError_t e = cudaFuncSetAttribute(score_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
-    if (e != cudaSuccess) return (int)e;
-    score_kernel<false><<<grid, kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
+    return p.tiles ? launch_score_t<true, true>(hp, stream) : launch_score_t<false, true>(hp, stream);
   }
-  return (int)cudaGetLastError();
+  return p.tiles ? launch_score_t<true, false>(p, stream) : launch_score_t<false, false>(p, stream);
 }
 
 // area_score, final score, COCO xywh box and the post_process predicate (object_scoring.py:244-266,

@@ -44,7 +44,7 @@ struct TileParams {
 };
 // image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
 int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw = nullptr);
-int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw = nullptr);   // antialiased crops
 int launch_tiles(const TileParams& p, cudaStream_t stream);
 int launch_round_update(const RefineParams& p, const float4* deltas, const float* max_sdf, int M, cudaStream_t stream);
 
@@ -64,9 +64,10 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 int launch_crop_resize(const float* fields, int n_img, int C, int H, int W, const int* channels, int n_ch,
                        const void* boxes, int boxes_f64, const int* counts, int cap, float* out, cudaStream_t stream);
 
+// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variants
 int launch_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, const int* channels, int n_ch,
                           const void* boxes, int boxes_f64, const int* counts, int cap, float* out, float* scratch,
-                          cudaStream_t stream);
+                          cudaStream_t stream, const int* image_hw = nullptr);
 int launch_mask_resize_aa(const unsigned char* masks, int B, int oh, int ow, unsigned char* out, float* scratch, cudaStream_t stream);
 
 // ---- center.cu -----------------------------------------------------------------------

@@ -429,15 +429,15 @@ class Object_Discovery:
 
         fields [B,4,H,W] fp32, proposals [B,N,4] fp64/fp32, counts [B] int32 or None.
         ``image_hw`` [B,2] int32 (device): ``fields`` is a padded stack of images of different sizes
-        (``ops.pack_fields``); every image gets what it would get alone.  Not with antialias=True or a tile provider.
+        (``ops.pack_fields``); every image gets what it would get alone, in either resize mode.  Not with a tile provider.
         Returns (boxes [B, 5N (9N + 256 with --analyze_cc), 4] fp32, counts [B] int32) in the reference's output order."""
         a = self.args
         ch = self.channels
         B, N = proposals.shape[0], proposals.shape[1]
         dev = fields.device
         f64 = torch.float64
-        if image_hw is not None and (self._tile_path or self.antialias):
-            raise ops.UnmoreError("discover_batch: image_hw (images of different sizes) needs antialias=False and no tile provider")
+        if image_hw is not None and self._tile_path:
+            raise ops.UnmoreError("discover_batch: image_hw (images of different sizes) is not supported with a tile provider")
         if self._tile_path:   # per-crop nets: image by image on the tile path (not the fused kernels)
             dets = [self._discover_image_tiles(fields[b], proposals[b] if counts is None else proposals[b, : int(counts[b])])
                     for b in range(B)]
@@ -532,10 +532,10 @@ class Object_Discovery:
 
         ``batch_size`` > 1 (not in the reference): consecutive dataset images of any sizes are padded into one stack
         (``ops.pack_fields``), each with its own anchors, and run through ``discover_batch`` together; the results and the
-        file are identical to ``batch_size=1``.  Ignored with antialias=True or a tile provider."""
+        file are identical to ``batch_size=1``, in either resize mode.  Ignored with a tile provider."""
         from . import rle
         results = {}
-        if images is None and batch_size > 1 and not self.antialias and not self._tile_path:
+        if images is None and batch_size > 1 and not self._tile_path:
             if self.test_dataset is None:
                 raise RuntimeError("main_object_discovery(): set self.test_dataset (e.g. FieldDataset) first")
             for start in range(0, len(self.test_dataset), batch_size):

@@ -86,9 +86,9 @@ class Object_Scoring:
         selected [B,cap] (post_process predicate), keep [B,cap], keep_counts [B], masks (packed, indexed by
         the ORIGINAL proposal index: use keep to gather).  ``image_hw`` [B,2] int32 (device): ``fields`` is a padded
         stack of images of different sizes (``ops.pack_fields``); image b's masks are ``masks[b, :, :h_b,
-        :ceil(w_b/32)]``.  Not with antialias=True or a tile provider."""
-        if image_hw is not None and (self.tile_provider is not None or self.antialias):
-            raise ops.UnmoreError("score_batch: image_hw (images of different sizes) needs antialias=False and no tile provider")
+        :ceil(w_b/32)]``.  In either resize mode; not with a tile provider."""
+        if image_hw is not None and self.tile_provider is not None:
+            raise ops.UnmoreError("score_batch: image_hw (images of different sizes) is not supported with a tile provider")
         if self.tile_provider is not None:   # per-crop nets: (sdf, center) tiles + one classifier scalar per crop
             B, cap = boxes.shape[0], boxes.shape[1]
             tiles = torch.zeros((B, cap, 4, ops.CROP, ops.CROP), dtype=torch.float32, device=fields.device)
@@ -103,9 +103,10 @@ class Object_Scoring:
                 antialias=self.tile_provider.antialias, existence_scores=ex)
         elif self.antialias:
             ch = self.channels
-            tiles = ops.crop_resize(fields, boxes, [ch.sdf, ch.center_row, ch.center_col, ch.exist], counts, antialias=True)
+            tiles = ops.crop_resize(fields, boxes, [ch.sdf, ch.center_row, ch.center_col, ch.exist], counts, antialias=True,
+                                    image_hw=image_hw)
             scores, tight, areas, masks = ops.score_and_rasterise_from_tiles(tiles, fields.shape[-2], fields.shape[-1], boxes, counts,
-                                                                             want_masks=want_masks)
+                                                                             want_masks=want_masks, image_hw=image_hw)
         else:
             scores, tight, areas, masks = ops.score_and_rasterise(fields, boxes, counts, ch=self.channels, want_masks=want_masks,
                                                                   image_hw=image_hw)
@@ -181,9 +182,9 @@ class Object_Scoring:
 
         ``batch_size`` > 1 (not in the reference): consecutive dataset images of any sizes are padded into one stack
         (``ops.pack_fields``) and scored by one ``score_batch``; the annotations and the file are identical to
-        ``batch_size=1``.  Ignored with antialias=True or a tile provider."""
+        ``batch_size=1``, in either resize mode.  Ignored with a tile provider."""
         out = []
-        if images is None and batch_size > 1 and not self.antialias and self.tile_provider is None:
+        if images is None and batch_size > 1 and self.tile_provider is None:
             if self.test_dataset is None:
                 raise RuntimeError("main_object_scoring(): set self.test_dataset (e.g. FieldDataset) first")
             for start in range(0, len(self.test_dataset), batch_size):

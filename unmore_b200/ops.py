@@ -88,7 +88,9 @@ _KERNELS = {"unmore_crop_resize": 1, "unmore_crop_resize_aa": 2, "unmore_mask_re
             "unmore_pack_detections": 1, "unmore_tile_means": 1, "unmore_center_reasoning_from_tiles": 1,
             "unmore_boundary_round_from_tiles": 2, "unmore_score_and_rasterise_from_tiles": 1,
             "unmore_existence_scores_hw": 1, "unmore_center_reasoning_hw": 1, "unmore_boundary_refine_hw": 1,
-            "unmore_score_and_rasterise_hw": 1, "unmore_box_sums_hw": 1, "unmore_sat_build_fields_hw": 1}
+            "unmore_score_and_rasterise_hw": 1, "unmore_box_sums_hw": 1, "unmore_sat_build_fields_hw": 1,
+            "unmore_existence_scores_aa_hw": 1, "unmore_boundary_refine_aa_hw": 1, "unmore_crop_resize_aa_hw": 2,
+            "unmore_center_reasoning_from_tiles_hw": 1, "unmore_score_and_rasterise_from_tiles_hw": 1}
 
 
 def set_timer(t: Optional[StageTimer]):
@@ -139,11 +141,9 @@ def _check_counts(counts: Optional[torch.Tensor], n_img: int):
         raise _lib.UnmoreError("counts must be a CUDA int32 tensor of n_img entries")
 
 
-def _check_extents(image_hw, n_img: int, device, what: str = "", antialias: bool = False) -> torch.Tensor:
+def _check_extents(image_hw, n_img: int, device, what: str = "") -> torch.Tensor:
     """The (h, w) table of a padded stack: a CUDA int32 [n_img, 2] tensor on the fields' device, 8-byte aligned.  Its
     values are not read on the host (no sync); the kernels clamp them to [1, pitch]."""
-    if antialias:
-        raise _lib.UnmoreError(f"{what}: image_hw (images of different sizes) is not supported with antialias=True")
     if not torch.is_tensor(image_hw) or not image_hw.is_cuda or image_hw.dtype != torch.int32 or \
             tuple(image_hw.shape) != (n_img, 2):
         raise _lib.UnmoreError(f"{what}: image_hw must be a CUDA int32 [n_img, 2] tensor of (h, w) per image")
@@ -216,9 +216,9 @@ def existence_scores(fields, boxes, counts=None, ch: Channels = DEFAULT_CHANNELS
     ws = workspace(n_img, fields.device) if ws is None else ws
     out = torch.zeros((n_img, cap), dtype=torch.float32, device=fields.device) if out is None else out
     if image_hw is not None:
-        hw = _check_extents(image_hw, n_img, fields.device, "existence_scores", antialias)
+        hw = _check_extents(image_hw, n_img, fields.device, "existence_scores")
         _on(fields)
-        _call("unmore_existence_scores_hw", fields.data_ptr(), n_img, C, H, W, hw.data_ptr(), ch.exist, boxes.data_ptr(), f64,
+        _call("unmore_existence_scores_aa_hw" if antialias else "unmore_existence_scores_hw", fields.data_ptr(), n_img, C, H, W, hw.data_ptr(), ch.exist, boxes.data_ptr(), f64,
               _ptr(counts), cap, out.data_ptr(), ws.data_ptr(), _stream(), counts=counts)
         return out
     _call("unmore_existence_scores_aa" if antialias else "unmore_existence_scores", fields.data_ptr(), n_img, C, H, W, ch.exist, boxes.data_ptr(), f64,
@@ -226,13 +226,20 @@ def existence_scores(fields, boxes, counts=None, ch: Channels = DEFAULT_CHANNELS
     return out
 
 
-def crop_resize(fields, boxes, channels, counts=None, antialias: bool = False):
+def crop_resize(fields, boxes, channels, counts=None, antialias: bool = False, image_hw=None):
     """Resized crops [n_img, cap, len(channels), 128, 128] fp32 (a2 / a4 as a stand-alone op).
-    ``antialias=True`` is the second resize mode (torchvision >= 0.17's default for transforms.Resize)."""
+    ``antialias=True`` is the second resize mode (torchvision >= 0.17's default for transforms.Resize).
+    ``image_hw`` [n_img, 2] int32, with ``antialias=True`` only: ``fields`` is a padded stack of images of different
+    sizes (``pack_fields``) and every window snaps to its own image."""
     import ctypes
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
+    hw = None
+    if image_hw is not None:
+        if not antialias:
+            raise _lib.UnmoreError("crop_resize: image_hw (images of different sizes) needs antialias=True")
+        hw = _check_extents(image_hw, n_img, fields.device, "crop_resize")
     ch = (ctypes.c_int * len(channels))(*[int(c) for c in channels])
     out = torch.zeros((n_img, cap, len(channels), CROP, CROP), dtype=torch.float32, device=fields.device)
     if cap and antialias:
@@ -246,7 +253,8 @@ def crop_resize(fields, boxes, channels, counts=None, antialias: bool = False):
             cnt = None if counts is None else (counts - c0).clamp(0, c1 - c0).to(torch.int32)
             scratch = torch.empty((n_img * (c1 - c0) * per_box // 4,), dtype=torch.float32, device=fields.device)
             _on(fields)
-            _call("unmore_crop_resize_aa", fields.data_ptr(), n_img, C, H, W, ctypes.cast(ch, ctypes.c_void_p), len(channels),
+            name, size = ("unmore_crop_resize_aa", (H, W)) if hw is None else ("unmore_crop_resize_aa_hw", (H, W, hw.data_ptr()))
+            _call(name, fields.data_ptr(), n_img, C, *size, ctypes.cast(ch, ctypes.c_void_p), len(channels),
                   bsl.data_ptr(), f64, _ptr(cnt), c1 - c0, osl.data_ptr(), scratch.data_ptr(), scratch.numel() * 4, _stream())
             out[:, c0:c1] = osl
         return out
@@ -269,15 +277,16 @@ def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channel
     is at least one proposal of every image, so the bound holds up to ~1150 images per call at 480 px field height.
     Slices walk the whole capacity whatever the counts, so most of them are empty on split lists.
     ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes (``pack_fields``); the
-    --analyze_cc boxes are clipped against each image's own size."""
+    --analyze_cc boxes are clipped against each image's own size (with ``antialias=True`` the table goes to the crop and
+    to ``center_reasoning_from_tiles``)."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = fields.device
     ws = workspace(n_img, dev) if ws is None else ws
-    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "center_reasoning", antialias)
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "center_reasoning")
     if antialias:
-        return _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc)
+        return _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc, hw)
     maxv = torch.zeros((n_img, cap), dtype=torch.float64, device=dev)
     argmax = torch.full((n_img, cap), -1, dtype=torch.int32, device=dev)
     splits = torch.zeros((n_img, cap, 4, 4), dtype=torch.float64, device=dev) if want_splits else None
@@ -296,7 +305,7 @@ def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channel
     return maxv, argmax, splits, cc
 
 
-def _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc):
+def _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc, hw=None):
     import ctypes
     n_img, C, H, W = fields.shape
     cap = boxes.shape[1]
@@ -321,12 +330,13 @@ def _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyz
         tiles = torch.empty((n_img, m, 3, CROP, CROP), dtype=torch.float32, device=dev)   # rows past the counts are never read
         scratch = torch.empty((n_img * m * 3 * H * CROP,), dtype=torch.float32, device=dev)
         _on(fields)
-        _call("unmore_crop_resize_aa", fields.data_ptr(), n_img, C, H, W, ctypes.cast(chp, ctypes.c_void_p), 3,
+        name, size = ("unmore_crop_resize_aa", (H, W)) if hw is None else ("unmore_crop_resize_aa_hw", (H, W, hw.data_ptr()))
+        _call(name, fields.data_ptr(), n_img, C, *size, ctypes.cast(chp, ctypes.c_void_p), 3,
               bsl.data_ptr(), int(boxes.dtype == torch.float64), _ptr(cnt), m, tiles.data_ptr(), scratch.data_ptr(),
               scratch.numel() * 4, _stream())
         del scratch
         mv, am, sp, cs = center_reasoning_from_tiles(tiles, H, W, bsl, cnt, thr=thr, ws=ws, want_splits=want_splits,
-                                                     analyze_cc=analyze_cc)
+                                                     analyze_cc=analyze_cc, image_hw=hw)
         maxv[:, c0:c1] = mv
         argmax[:, c0:c1] = am
         if want_splits:
@@ -351,12 +361,12 @@ def boundary_refine(fields, boxes, counts=None, n_round: int = 50, apply_small_f
     _check_counts(counts, n_img)
     dev = fields.device
     ws = workspace(n_img, dev) if ws is None else ws
-    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "boundary_refine", antialias)
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "boundary_refine")
     out = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     labels = torch.full((n_img, cap), -2.0, dtype=torch.float32, device=dev)
     rounds = torch.zeros((n_img, cap), dtype=torch.int32, device=dev) if want_rounds else None
     _on(fields)
-    name = "unmore_boundary_refine_aa" if antialias else "unmore_boundary_refine" if hw is None else "unmore_boundary_refine_hw"
+    name = ("unmore_boundary_refine_aa" if antialias else "unmore_boundary_refine") + ("" if hw is None else "_hw")
     _call(name, fields.data_ptr(), n_img, C, H, W, *(() if hw is None else (hw.data_ptr(),)), ch.sdf,
               boxes.data_ptr(), f64,
               _ptr(counts), cap, int(n_round), int(apply_small_filter), int(early_exit), float(proposal_area_thres),
@@ -661,14 +671,17 @@ def tile_means(tiles: torch.Tensor) -> torch.Tensor:
 
 
 def center_reasoning_from_tiles(tiles, H, W, boxes, counts=None, thr: float = 0.009, ws=None, want_splits: bool = True,
-                                analyze_cc: bool = False):
+                                analyze_cc: bool = False, image_hw=None):
     """center_reasoning on tiles [n_img, cap, 3, 128, 128] = (sdf, center_row, center_col); same returns as
-    ``center_reasoning``.  H, W: image size (the --analyze_cc enlargement clips against it)."""
+    ``center_reasoning``.  H, W: image size (the --analyze_cc enlargement clips against it).  ``image_hw`` [n_img, 2]
+    int32: the tiles come from a padded stack (``crop_resize(..., antialias=True, image_hw=)``), H, W are its pitch and
+    each image's windows and clip use its own size."""
     tiles = _on(tiles.contiguous())
     n_img, cap = tiles.shape[0], tiles.shape[1]
     _, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = tiles.device
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "center_reasoning_from_tiles")
     ws = workspace(n_img, dev) if ws is None else ws
     maxv = torch.zeros((n_img, cap), dtype=torch.float64, device=dev)
     argmax = torch.full((n_img, cap), -1, dtype=torch.int32, device=dev)
@@ -681,7 +694,9 @@ def center_reasoning_from_tiles(tiles, H, W, boxes, counts=None, thr: float = 0.
               torch.zeros((1,), dtype=torch.int32, device=dev))
     _on(tiles)
     if cap:
-        _call("unmore_center_reasoning_from_tiles", tiles.data_ptr(), n_img, int(H), int(W), boxes.data_ptr(), f64, _ptr(counts), cap,
+        name, size = ("unmore_center_reasoning_from_tiles", (int(H), int(W))) if hw is None else \
+            ("unmore_center_reasoning_from_tiles_hw", (int(H), int(W), hw.data_ptr()))
+        _call(name, tiles.data_ptr(), n_img, *size, boxes.data_ptr(), f64, _ptr(counts), cap,
               float(thr), maxv.data_ptr(), argmax.data_ptr(), _ptr(splits), _ptr(cc[0]) if cc else None,
               _ptr(cc[1]) if cc else None, _ptr(cc[2]) if cc else None, ws.data_ptr(), _stream(), counts=counts)
     return maxv, argmax, splits, cc
@@ -710,15 +725,18 @@ def boundary_round_from_tiles(tiles, boxes, H, W, max_sdf_thres: float = 0.5, ma
 
 
 def score_and_rasterise_from_tiles(tiles, H, W, boxes, counts=None, want_masks: bool = True, antialias: bool = True,
-                                   existence_scores: Optional[torch.Tensor] = None):
+                                   existence_scores: Optional[torch.Tensor] = None, image_hw=None):
     """score_and_rasterise on tiles [n_img, cap, 4, 128, 128] = (sdf, center_row, center_col, existence); the masks are
     resized back to the box with the antialiased kernel (``antialias``) or the plain one; ``existence_scores``
-    [n_img, cap] fp32, when given, replaces the mean of the fourth tile.  Same returns as ``score_and_rasterise``."""
+    [n_img, cap] fp32, when given, replaces the mean of the fourth tile.  Same returns as ``score_and_rasterise``.
+    ``image_hw`` [n_img, 2] int32: the tiles come from a padded stack (``crop_resize(..., antialias=True, image_hw=)``)
+    and H, W are its pitch; the masks stay on the pitched canvas as in ``score_and_rasterise``."""
     tiles = _on(tiles.contiguous())
     n_img, cap = tiles.shape[0], tiles.shape[1]
     _, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = tiles.device
+    hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "score_and_rasterise_from_tiles")
     scores = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     tight = torch.zeros((n_img, cap, 4), dtype=torch.float32, device=dev)
     areas = torch.zeros((n_img, cap), dtype=torch.int32, device=dev)
@@ -727,7 +745,9 @@ def score_and_rasterise_from_tiles(tiles, H, W, boxes, counts=None, want_masks: 
     if cap > 0:
         if existence_scores is not None:
             existence_scores = existence_scores.to(dev, torch.float32).reshape(n_img, cap).contiguous()
-        _call("unmore_score_and_rasterise_from_tiles", tiles.data_ptr(), _ptr(existence_scores), int(antialias), n_img, int(H), int(W),
+        name, size = ("unmore_score_and_rasterise_from_tiles", (int(H), int(W))) if hw is None else \
+            ("unmore_score_and_rasterise_from_tiles_hw", (int(H), int(W), hw.data_ptr()))
+        _call(name, tiles.data_ptr(), _ptr(existence_scores), int(antialias), n_img, *size,
               boxes.data_ptr(), f64, _ptr(counts), cap,
               scores.data_ptr(), tight.data_ptr(), areas.data_ptr(), _ptr(masks), _stream())
     return scores, tight, areas, masks
