@@ -66,8 +66,9 @@ int unmore_crop_resize(const float* fields, int n_img, int C, int H, int W,
  * what torchvision >= 0.17 makes of the reference's transforms.Resize calls (object_reasoning.py:319,407,505;
  * object_scoring.py:131,206,222) when the pinned 0.14.1 is not what is installed.  Bit-exact against torch 2.11
  * CPU (weights with ATen's float/double mix, horizontal pass first, its accumulation order).  The fused
- * existence and refine kernels have antialiased forms (unmore_existence_scores_aa, unmore_boundary_refine_aa);
- * these produce the tiles for the center and scoring stages, for unmore_update_bbox_from_tiles and for inspection.  `scratch`: n_img*cap*n_channels*H*128 floats (crop) / B*128*out_w floats (mask). */
+ * existence, center and refine kernels have antialiased forms (unmore_existence_scores_aa,
+ * unmore_center_reasoning_aa, unmore_boundary_refine_aa); these produce the tiles for the scoring stage, for the
+ * other *_from_tiles stages, for unmore_update_bbox_from_tiles and for inspection.  `scratch`: n_img*cap*n_channels*H*128 floats (crop) / B*128*out_w floats (mask). */
 int unmore_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, const int* channels_host,
                           int n_channels, const void* boxes, int boxes_f64, const int* counts, int cap,
                           float* out, void* scratch, size_t scratch_bytes, unmore_stream_t stream);
@@ -137,14 +138,23 @@ int unmore_boundary_refine(const float* fields, int n_img, int C, int H, int W, 
                            float* boxes_out, float* labels_out, int* rounds_out, void* ws,
                            unmore_stream_t stream);
 
-/* unmore_existence_scores and unmore_boundary_refine in the SECOND resize mode (antialias=True, see
- * unmore_crop_resize_aa): same arguments, validation, workspace and outputs, with every crop resampled by ATen's
- * antialiased kernel inside the fused kernels instead of materialised as a tile.  Bit-identical to the tile path:
- * the existence score equals unmore_tile_means of the unmore_crop_resize_aa tile, and every refine round equals
- * unmore_boundary_round_from_tiles on it (window cache, early exit and rounds_out as in the primary mode). */
+/* unmore_existence_scores, unmore_center_reasoning and unmore_boundary_refine in the SECOND resize mode
+ * (antialias=True, see unmore_crop_resize_aa): same arguments, validation, workspace and outputs, with every crop
+ * resampled by ATen's antialiased kernel inside the fused kernels instead of materialised as a tile; no scratch, one
+ * kernel per call (plus the counts prefix).  Bit-identical to the tile path: the existence score equals
+ * unmore_tile_means of the unmore_crop_resize_aa tile, center reasoning equals unmore_center_reasoning_from_tiles on
+ * the (sdf, center_row, center_col) tiles (--analyze_cc included), and every refine round equals
+ * unmore_boundary_round_from_tiles on the sdf tile (window cache, early exit and rounds_out as in the primary mode).
+ * Callers detect these entry points by their symbols (unmore_version() is unchanged). */
 int unmore_existence_scores_aa(const float* fields, int n_img, int C, int H, int W, int ch_exist,
                                const void* boxes, int boxes_f64, const int* counts, int cap,
                                float* scores_out, void* ws, unmore_stream_t stream);
+int unmore_center_reasoning_aa(const float* fields, int n_img, int C, int H, int W, int ch_sdf,
+                               int ch_center_row, int ch_center_col, const void* boxes, int boxes_f64,
+                               const int* counts, int cap, double center_score_max_thres,
+                               double* max_values_out, int* argmax_out, double* splits_out,
+                               unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow,
+                               void* ws, unmore_stream_t stream);
 int unmore_boundary_refine_aa(const float* fields, int n_img, int C, int H, int W, int ch_sdf,
                               const void* boxes, int boxes_f64, const int* counts, int cap, int n_round,
                               int apply_small_filter, int early_exit, float proposal_area_thres,
@@ -299,9 +309,9 @@ int unmore_mask_nms(const uint32_t* masks, int K, int H, int W, const float* sco
  * zeros, so entries [:h_i+1, :w_i+1] of image i's tables are those of the image alone; unmore_box_sums_hw takes such
  * tables.  A null, misaligned, host or other-device image_hw is rejected (UNMORE_E_INVALID) before anything runs.
  *
- * The second resize mode (antialias=True) has the same five forms: unmore_existence_scores_aa_hw,
- * unmore_boundary_refine_aa_hw, unmore_crop_resize_aa_hw, unmore_center_reasoning_from_tiles_hw and
- * unmore_score_and_rasterise_from_tiles_hw, each with image_hw after W.  unmore_crop_resize_aa_hw snaps every window
+ * The second resize mode (antialias=True) has the same six forms: unmore_existence_scores_aa_hw,
+ * unmore_center_reasoning_aa_hw, unmore_boundary_refine_aa_hw, unmore_crop_resize_aa_hw,
+ * unmore_center_reasoning_from_tiles_hw and unmore_score_and_rasterise_from_tiles_hw, each with image_hw after W.  unmore_crop_resize_aa_hw snaps every window
  * to its image and sizes its scratch by the pitch (n_img*cap*n_channels*H*128 floats).  The two *_from_tiles_hw calls
  * take tiles cropped from the stack by unmore_crop_resize_aa_hw and the pitch as (H, W): the extents give the window
  * snap behind the split boxes, the --analyze_cc clip and the mask raster, whose canvas is the pitched one above. */
@@ -338,6 +348,12 @@ int unmore_boundary_refine_aa_hw(const float* fields, int n_img, int C, int H, i
                                  float max_sdf_thres, float max_shrink_threshold, float delta_ratio,
                                  float* boxes_out, float* labels_out, int* rounds_out, void* ws,
                                  unmore_stream_t stream);
+int unmore_center_reasoning_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
+                                  int ch_sdf, int ch_center_row, int ch_center_col, const void* boxes,
+                                  int boxes_f64, const int* counts, int cap, double center_score_max_thres,
+                                  double* max_values_out, int* argmax_out, double* splits_out,
+                                  unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow, void* ws,
+                                  unmore_stream_t stream);
 int unmore_crop_resize_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,
                              const int* channels_host, int n_channels, const void* boxes, int boxes_f64,
                              const int* counts, int cap, float* out, void* scratch, size_t scratch_bytes,

@@ -4,12 +4,12 @@ plus scoring, on the inputs of ``bench.py --config antialias`` (synth.make_field
 * tile path: what this mode ran before the fused kernels, one image at a time: antialiased crops of the existence
   channel + tile_means, of the three center-stage channels + center_reasoning_from_tiles, of the boundary-distance
   channel alone in every round of the host loop _boundary_reasoning_tiles; then Object_Scoring.score_batch;
-* batched path: ReasoningPipeline.run_chunk on all images (fused antialiased existence and refine, center stage on
-  sliced tiles, batched scoring).
+* batched path: ReasoningPipeline.run_chunk on all images (fused antialiased existence, center reasoning and refine,
+  batched scoring).
 
 Warm-up, then the two paths alternately, timed with CUDA events around synchronised runs; then one more run of each
 with ops.StageTimer for the stage split, and the batched path's center stage once more with every count zero: its
-time is the cost of walking the proposal capacity in slices with no work in them.  Launches are the kernels of the
+time is what the stage costs with no work in it.  Peak device memory is that of one batched run.  Launches are the kernels of the
 C-ABI calls (ops.LAUNCHES); the fills and copies torch launches around them are not counted.  Prints one JSON line and
 asserts that both paths produced identical boxes, scores and masks.  usage: python scripts/aa_throughput.py [--images 16] [--repeats 3]"""
 import argparse
@@ -90,10 +90,10 @@ def main():
     pipe = ReasoningPipeline(dev, rargs, with_sat=False)
     # stage labels for the split (the wrappers only name the timer's entries)
     ops.existence_scores = _staged(ops.existence_scores, "existence")
-    ops.center_reasoning = _staged(ops.center_reasoning, "center tiles")
+    ops.center_reasoning = _staged(ops.center_reasoning, "center")
     ops.boundary_refine = _staged(ops.boundary_refine, "refine")
     tile_od.existence_checking = _staged(tile_od.existence_checking, "existence")
-    tile_od.center_reasoning = _staged(tile_od.center_reasoning, "center tiles")
+    tile_od.center_reasoning = _staged(tile_od.center_reasoning, "center")
     tile_od.boundary_reasoning = _staged(tile_od.boundary_reasoning, "refine")
     scoring.score_batch = _staged(scoring.score_batch, "scoring")
     pipe.scoring.score_batch = _staged(pipe.scoring.score_batch, "scoring")
@@ -147,6 +147,9 @@ def main():
         assert torch.equal(r["masks"][b][keep], sc["masks"][0][keep]), f"masks differ, image {b}"
         n_ann += kk
 
+    torch.cuda.reset_peak_memory_stats()
+    batched_path()
+    peak = torch.cuda.max_memory_allocated()
     split = {}
     for name, fn in (("tile", tile_path), ("batched", batched_path)):
         t = LabelledTimer()
@@ -166,8 +169,6 @@ def main():
 
     timed(empty_center)
     t_empty, _, _ = timed(empty_center)
-    slices = sum(-(-cap // max(1, min(cap, ops.CENTER_AA_SLICE_BYTES // (3 * (128 * 128 + H * 128) * 4 * n))))
-                 for cap in (N, 4 * N))
 
     try:
         power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
@@ -181,7 +182,7 @@ def main():
         "speedup": round(med(t_tile) / med(t_batch), 2), "tile_s": [round(v, 3) for v in t_tile],
         "batched_s": [round(v, 3) for v in t_batch], "tile_launches_per_image": round(l_tile / n, 1),
         "batched_launches_per_image": round(l_batch / n, 1), "stage_ms": split,
-        "center_slices": slices, "center_empty_ms": round(t_empty * 1e3, 2),
+        "center_empty_ms": round(t_empty * 1e3, 2), "batched_peak_device_memory_gb": round(peak / 1e9, 2),
         "launches_counted": "C-ABI kernels (ops.LAUNCHES); torch fills and copies not counted", "discovered": n_det, "annotations": n_ann,
         "outputs_identical": True}))
 

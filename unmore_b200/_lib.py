@@ -28,6 +28,7 @@ SIGNATURES = {
     "unmore_boundary_round_from_tiles": [_p, _i, _p, _i, _i, _i, _f, _f, _f, _p, _p, _p, _p, _p],
     "unmore_score_and_rasterise_from_tiles": [_p, _p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _p, _p, _p, _p],
     "unmore_center_reasoning": [_p, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
+    "unmore_center_reasoning_aa": [_p, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
     "unmore_boundary_refine": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
     "unmore_boundary_refine_aa": [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
     "unmore_update_bbox_from_tiles": [_p, _i, _p, _p, _p],
@@ -57,6 +58,7 @@ SIGNATURES = {
     "unmore_sat_build_fields_hw": [_p, _i, _i, _i, _i, _p, _p, _i, _p, _p],
     "unmore_existence_scores_aa_hw": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _p, _p, _p],
     "unmore_boundary_refine_aa_hw": [_p, _i, _i, _i, _i, _p, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _f, _p, _p, _p, _p, _p],
+    "unmore_center_reasoning_aa_hw": [_p, _i, _i, _i, _i, _p, _i, _i, _i, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
     "unmore_crop_resize_aa_hw": [_p, _i, _i, _i, _i, _p, _p, _i, _p, _i, _p, _i, _p, _p, C.c_size_t, _p],
     "unmore_center_reasoning_from_tiles_hw": [_p, _i, _i, _i, _p, _p, _i, _p, _i, _d, _p, _p, _p, _p, _p, _p, _p, _p],
     "unmore_score_and_rasterise_from_tiles_hw": [_p, _p, _i, _i, _i, _i, _p, _p, _i, _p, _i, _p, _p, _p, _p, _p],

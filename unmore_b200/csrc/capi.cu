@@ -161,8 +161,8 @@ int boundary_refine(const char* name, bool aa, const float* fields, int n_img, i
   return cuda_fail(launch_refine(p, num_sms(), s, image_hw), "refine_kernel");
 }
 
-// unmore_center_reasoning / unmore_center_reasoning_hw
-int center_reasoning(const char* name, const float* fields, int n_img, int C, int H, int W, int ch_sdf, int ch_center_row,
+// unmore_center_reasoning / unmore_center_reasoning_aa and their _hw forms
+int center_reasoning(const char* name, bool aa, const float* fields, int n_img, int C, int H, int W, int ch_sdf, int ch_center_row,
                      int ch_center_col, const void* boxes, int boxes_f64, const int* counts, int cap,
                      double center_score_max_thres, double* max_values_out, int* argmax_out, double* splits_out,
                      unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow, void* ws, cudaStream_t s,
@@ -183,6 +183,7 @@ int center_reasoning(const char* name, const float* fields, int n_img, int C, in
   p.image_hw = image_hw;
   center_filters(p);
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
+  if (aa) return cuda_fail(launch_center_aa(p, num_sms(), s), "center_aa_kernel");
   return cuda_fail(launch_center(p, num_sms(), s), "center_kernel");
 }
 
@@ -330,8 +331,18 @@ int unmore_center_reasoning(const float* fields, int n_img, int C, int H, int W,
                             double center_score_max_thres, double* max_values_out, int* argmax_out,
                             double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow,
                             void* ws, unmore_stream_t stream) {
-  return center_reasoning("unmore_center_reasoning", fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes,
+  return center_reasoning("unmore_center_reasoning", false, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes,
                           boxes_f64, counts, cap, center_score_max_thres, max_values_out, argmax_out, splits_out,
+                          cc_counts_out, cc_boxes_out, cc_overflow, ws, (cudaStream_t)stream);
+}
+
+int unmore_center_reasoning_aa(const float* fields, int n_img, int C, int H, int W, int ch_sdf, int ch_center_row,
+                               int ch_center_col, const void* boxes, int boxes_f64, const int* counts, int cap,
+                               double center_score_max_thres, double* max_values_out, int* argmax_out,
+                               double* splits_out, unsigned char* cc_counts_out, double* cc_boxes_out, int* cc_overflow,
+                               void* ws, unmore_stream_t stream) {
+  return center_reasoning("unmore_center_reasoning_aa", true, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col,
+                          boxes, boxes_f64, counts, cap, center_score_max_thres, max_values_out, argmax_out, splits_out,
                           cc_counts_out, cc_boxes_out, cc_overflow, ws, (cudaStream_t)stream);
 }
 
@@ -583,7 +594,7 @@ int unmore_center_reasoning_hw(const float* fields, int n_img, int C, int H, int
                                void* ws, unmore_stream_t stream) {
   const char* name = "unmore_center_reasoning_hw";
   if (int e = check_extents(name, image_hw)) return e;
-  return center_reasoning(name, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes, boxes_f64, counts, cap,
+  return center_reasoning(name, false, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes, boxes_f64, counts, cap,
                           center_score_max_thres, max_values_out, argmax_out, splits_out, cc_counts_out, cc_boxes_out,
                           cc_overflow, ws, (cudaStream_t)stream, image_hw);
 }
@@ -653,6 +664,18 @@ int unmore_boundary_refine_aa_hw(const float* fields, int n_img, int C, int H, i
   return boundary_refine(name, true, fields, n_img, C, H, W, ch_sdf, boxes, boxes_f64, counts, cap, n_round,
                          apply_small_filter, early_exit, proposal_area_thres, max_sdf_thres, max_shrink_threshold,
                          delta_ratio, boxes_out, labels_out, rounds_out, ws, (cudaStream_t)stream, image_hw);
+}
+
+int unmore_center_reasoning_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw, int ch_sdf,
+                                  int ch_center_row, int ch_center_col, const void* boxes, int boxes_f64,
+                                  const int* counts, int cap, double center_score_max_thres, double* max_values_out,
+                                  int* argmax_out, double* splits_out, unsigned char* cc_counts_out,
+                                  double* cc_boxes_out, int* cc_overflow, void* ws, unmore_stream_t stream) {
+  const char* name = "unmore_center_reasoning_aa_hw";
+  if (int e = check_extents(name, image_hw)) return e;
+  return center_reasoning(name, true, fields, n_img, C, H, W, ch_sdf, ch_center_row, ch_center_col, boxes, boxes_f64, counts,
+                          cap, center_score_max_thres, max_values_out, argmax_out, splits_out, cc_counts_out, cc_boxes_out,
+                          cc_overflow, ws, (cudaStream_t)stream, image_hw);
 }
 
 int unmore_crop_resize_aa_hw(const float* fields, int n_img, int C, int H, int W, const int* image_hw,

@@ -15,7 +15,7 @@
 //     remaining (n-1) mod 4 taps with a fused multiply-add.
 //
 // Two kernels (aa_crop.cuh) with the intermediate in a caller-provided scratch buffer: tiles for the *_from_tiles stages.  The fused
-// existence and refine kernels compute the same values row by row (aa_rows.cuh).
+// existence and refine kernels compute the same values row by row (aa_rows.cuh), so does the center kernel (center.cuh).
 #include "aa_crop.cuh"
 #include "unmore_internal.h"
 

@@ -1,6 +1,6 @@
 // Weights and accumulation order of ATen's antialiased bilinear kernel (_upsample_bilinear2d_aa), shared by the
 // stand-alone antialias ops (resample_aa.cu), the antialiased mask rasteriser of the scoring kernel (score.cu) and the
-// antialiased row source of the fused existence and refine kernels (aa_rows.cuh).
+// antialiased row sources of the fused existence and refine kernels (aa_rows.cuh) and of the center kernel (center.cuh).
 // See resample_aa.cu for the arithmetic contract; pinned by oracle/oracle.py::aa_index_weights / _aa_pass.
 #pragma once
 #include "common.cuh"

@@ -96,6 +96,7 @@ struct CenterParams {
   const int* image_hw;       // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
 };
 int launch_center(const CenterParams& p, int num_sms, cudaStream_t stream);
+int launch_center_aa(const CenterParams& p, int num_sms, cudaStream_t stream);   // antialiased crops, from the fields
 int launch_components(const unsigned char* masks, int B, int* counts, int* boxes, cudaStream_t stream);
 int launch_erode(const unsigned char* in, unsigned char* out, int B, int kernel_size, int num_round, cudaStream_t stream);
 int launch_anti_center(const float* vote, double* out, int B, int H, int W, const double* filt25, cudaStream_t stream);

@@ -80,7 +80,7 @@ LAUNCHES = 0  # kernels launched through the C ABI since import (gpu_launches in
 
 # kernels per C-ABI call (memsets not counted); +1 when a counts prefix is built
 _KERNELS = {"unmore_crop_resize": 1, "unmore_crop_resize_aa": 2, "unmore_mask_resize_aa": 2, "unmore_existence_scores": 1, "unmore_center_reasoning": 1, "unmore_boundary_refine": 1,
-            "unmore_existence_scores_aa": 1, "unmore_boundary_refine_aa": 1,
+            "unmore_existence_scores_aa": 1, "unmore_boundary_refine_aa": 1, "unmore_center_reasoning_aa": 1,
             "unmore_update_bbox_from_tiles": 1, "unmore_compact_boxes": 1, "unmore_box_nms": 1,
             "unmore_batch_erode": 1, "unmore_anti_center_map": 1, "unmore_connected_components": 1, "unmore_box_nms_matrix": 3,
             "unmore_score_and_rasterise": 1, "unmore_mask_resize": 1, "unmore_final_scores": 1, "unmore_sat_build": 1, "unmore_sat_build_fields": 1, "unmore_box_sums": 1,
@@ -89,7 +89,8 @@ _KERNELS = {"unmore_crop_resize": 1, "unmore_crop_resize_aa": 2, "unmore_mask_re
             "unmore_boundary_round_from_tiles": 2, "unmore_score_and_rasterise_from_tiles": 1,
             "unmore_existence_scores_hw": 1, "unmore_center_reasoning_hw": 1, "unmore_boundary_refine_hw": 1,
             "unmore_score_and_rasterise_hw": 1, "unmore_box_sums_hw": 1, "unmore_sat_build_fields_hw": 1,
-            "unmore_existence_scores_aa_hw": 1, "unmore_boundary_refine_aa_hw": 1, "unmore_crop_resize_aa_hw": 2,
+            "unmore_existence_scores_aa_hw": 1, "unmore_boundary_refine_aa_hw": 1, "unmore_center_reasoning_aa_hw": 1,
+            "unmore_crop_resize_aa_hw": 2,
             "unmore_center_reasoning_from_tiles_hw": 1, "unmore_score_and_rasterise_from_tiles_hw": 1}
 
 
@@ -264,29 +265,23 @@ def crop_resize(fields, boxes, channels, counts=None, antialias: bool = False, i
     return out
 
 
-CENTER_AA_SLICE_BYTES = 1 << 30   # tiles + resampling scratch of one slice of center_reasoning(antialias=True)
+CENTER_AA_SLICE_BYTES = 1 << 30   # unused: center_reasoning(antialias=True) is one fused call, nothing is sliced
 
 
 def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channels = DEFAULT_CHANNELS, ws=None,
                      want_splits: bool = True, analyze_cc: bool = False, antialias: bool = False, image_hw=None):
     """-> (max_values [n_img,cap] fp64, argmax [n_img,cap] int32 (-1 = passes), splits [n_img,cap,4,4] fp64 or None,
     cc) where cc is None or (cc_counts [n_img,cap] u8, cc_boxes [n_img,cap,CC_CAP,4] fp64, overflow [1] int32).
-    ``antialias=True`` (the second resize mode) has no fused kernel: it resamples antialiased tiles and runs
-    ``center_reasoning_from_tiles`` on them, in slices of the proposal capacity so that the tiles and their
-    scratch stay within CENTER_AA_SLICE_BYTES; the counts are clamped per slice on the device (no host sync).  A slice
-    is at least one proposal of every image, so the bound holds up to ~1150 images per call at 480 px field height.
-    Slices walk the whole capacity whatever the counts, so most of them are empty on split lists.
-    ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes (``pack_fields``); the
-    --analyze_cc boxes are clipped against each image's own size (with ``antialias=True`` the table goes to the crop and
-    to ``center_reasoning_from_tiles``)."""
+    ``antialias=True`` is the second resize mode: the fused kernel resamples every antialiased crop from the fields
+    itself, bit-identical to ``center_reasoning_from_tiles`` on the tiles of ``crop_resize(..., antialias=True)``.
+    ``image_hw`` [n_img, 2] int32: ``fields`` is a padded stack of images of different sizes (``pack_fields``); every
+    window snaps to, and the --analyze_cc boxes are clipped against, each image's own size."""
     n_img, C, H, W = _check_fields(fields)
     cap, f64 = _check_boxes(boxes, n_img)
     _check_counts(counts, n_img)
     dev = fields.device
     ws = workspace(n_img, dev) if ws is None else ws
     hw = None if image_hw is None else _check_extents(image_hw, n_img, dev, "center_reasoning")
-    if antialias:
-        return _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc, hw)
     maxv = torch.zeros((n_img, cap), dtype=torch.float64, device=dev)
     argmax = torch.full((n_img, cap), -1, dtype=torch.int32, device=dev)
     splits = torch.zeros((n_img, cap, 4, 4), dtype=torch.float64, device=dev) if want_splits else None
@@ -297,54 +292,12 @@ def center_reasoning(fields, boxes, counts=None, thr: float = 0.009, ch: Channel
               torch.zeros((n_img, cap, cc_cap, 4), dtype=torch.float64, device=dev),
               torch.zeros((1,), dtype=torch.int32, device=dev))
     _on(fields)
-    name, size = ("unmore_center_reasoning", (H, W)) if hw is None else ("unmore_center_reasoning_hw", (H, W, hw.data_ptr()))
+    name = ("unmore_center_reasoning_aa" if antialias else "unmore_center_reasoning") + ("" if hw is None else "_hw")
+    size = (H, W) if hw is None else (H, W, hw.data_ptr())
     _call(name, fields.data_ptr(), n_img, C, *size, ch.sdf, ch.center_row, ch.center_col,
           boxes.data_ptr(), f64, _ptr(counts), cap, float(thr), maxv.data_ptr(), argmax.data_ptr(),
           _ptr(splits), _ptr(cc[0]) if cc else None, _ptr(cc[1]) if cc else None, _ptr(cc[2]) if cc else None,
           ws.data_ptr(), _stream(), counts=counts)
-    return maxv, argmax, splits, cc
-
-
-def _center_reasoning_aa(fields, boxes, counts, thr, ch, ws, want_splits, analyze_cc, hw=None):
-    import ctypes
-    n_img, C, H, W = fields.shape
-    cap = boxes.shape[1]
-    dev = fields.device
-    maxv = torch.zeros((n_img, cap), dtype=torch.float64, device=dev)
-    argmax = torch.full((n_img, cap), -1, dtype=torch.int32, device=dev)
-    splits = torch.zeros((n_img, cap, 4, 4), dtype=torch.float64, device=dev) if want_splits else None
-    cc = None
-    if analyze_cc:
-        cc = (torch.zeros((n_img, cap), dtype=torch.uint8, device=dev),
-              torch.zeros((n_img, cap, _lib.load().unmore_cc_cap(), 4), dtype=torch.float64, device=dev),
-              torch.zeros((1,), dtype=torch.int32, device=dev))
-    chans = [ch.sdf, ch.center_row, ch.center_col]
-    chp = (ctypes.c_int * 3)(*chans)
-    per_box = 3 * (CROP * CROP + H * CROP) * 4 * n_img     # one proposal column of tiles + scratch, all images
-    step = max(1, min(cap, CENTER_AA_SLICE_BYTES // per_box))
-    for c0 in range(0, cap, step):
-        c1 = min(cap, c0 + step)
-        m = c1 - c0
-        bsl = boxes[:, c0:c1].contiguous()
-        cnt = None if counts is None else (counts - c0).clamp(0, m).to(torch.int32)
-        tiles = torch.empty((n_img, m, 3, CROP, CROP), dtype=torch.float32, device=dev)   # rows past the counts are never read
-        scratch = torch.empty((n_img * m * 3 * H * CROP,), dtype=torch.float32, device=dev)
-        _on(fields)
-        name, size = ("unmore_crop_resize_aa", (H, W)) if hw is None else ("unmore_crop_resize_aa_hw", (H, W, hw.data_ptr()))
-        _call(name, fields.data_ptr(), n_img, C, *size, ctypes.cast(chp, ctypes.c_void_p), 3,
-              bsl.data_ptr(), int(boxes.dtype == torch.float64), _ptr(cnt), m, tiles.data_ptr(), scratch.data_ptr(),
-              scratch.numel() * 4, _stream())
-        del scratch
-        mv, am, sp, cs = center_reasoning_from_tiles(tiles, H, W, bsl, cnt, thr=thr, ws=ws, want_splits=want_splits,
-                                                     analyze_cc=analyze_cc, image_hw=hw)
-        maxv[:, c0:c1] = mv
-        argmax[:, c0:c1] = am
-        if want_splits:
-            splits[:, c0:c1] = sp
-        if analyze_cc:
-            cc[0][:, c0:c1] = cs[0]
-            cc[1][:, c0:c1] = cs[1]
-            cc[2].add_(cs[2])
     return maxv, argmax, splits, cc
 
 
