@@ -2,8 +2,8 @@
   (a) per_image  - one image per call, the loop the zero-argument mains run with batch_size=1;
   (b) same_size  - batches of identical size only, through the uniform path;
   (c) padded     - padded mixed batches (ops.pack_fields + image_hw) of --batch images.
-Plus a uniform 480x640 batch through the sized (*_hw) kernels against the uniform ones.  Asserts that all ways give
-identical outputs and prints one JSON line.  --antialias runs all of it in the second resize mode (antialias=True).
+Plus a uniform 480x640 batch with an image_hw table (the *_hw entry points) against the same batch without one.
+Asserts that all ways give identical outputs and prints one JSON line.  --antialias runs all of it in the second resize mode (antialias=True).
 
 The shape table below is a plausible mix of photo shapes with a 640-px longer side (4:3, 3:2, 16:9, portrait, square)
 plus a few small images.  It is NOT COCO's measured size distribution.
@@ -136,7 +136,7 @@ def main():
     result["padded_pixel_fraction"] = round(pad_stats["padded"] / max(pad_stats["pixels"], 1), 4)
     result["speedup_padded_vs_per_image"] = round(result["ways"]["padded"]["images_per_s"] / result["ways"]["per_image"]["images_per_s"], 2)
 
-    # the sized kernels on a uniform 480x640 batch (no padding) against the uniform kernels, alternating
+    # a uniform 480x640 batch (no padding) with an image_hw table against the same batch without one, alternating
     nu = min(a.batch, 64)
     uf = torch.stack([synth.make_fields(1000 + i) for i in range(nu)]).to(dev)
     up = torch.stack([torch.from_numpy(synth.make_proposals(1000 + i, a.proposals)) for i in range(nu)]).to(dev)

@@ -1,8 +1,6 @@
 """Compares the sm_100a SASS of two builds of the library, kernel by kernel: every kernel of the first build must have
-byte-identical instructions in the second.  A kernel that gained a trailing template parameter with the value false (the
-SIZED flag of the kernels that take per-image extents, e.g. center_kernel<false, 0, true> ->
-center_kernel<false, 0, true, false>) is matched to its old name.  Kernels only the second build has are listed.
-Needs cuobjdump and cu++filt, no GPU.
+byte-identical instructions in the second.  Kernels only the second build has are listed.
+Needs cuobjdump, no GPU.
 usage: python scripts/sass_compare.py old.so new.so"""
 import re
 import subprocess
@@ -26,28 +24,8 @@ def kernels(lib):
     return out
 
 
-def demangle(names):
-    """mangled name -> name with its template arguments, without return type and parameter list"""
-    out = subprocess.run(["cu++filt"], input="\n".join(names), capture_output=True, text=True, check=True).stdout
-    plain = [v.replace("void ", "", 1) for v in out.splitlines()]
-    return {k: v[: v.index(">(") + 1] if ">(" in v else v[: v.index("(")] for k, v in zip(names, plain)}
-
-
 def main(old, new):
     a, b = kernels(old), kernels(new)
-    plain_a, plain_b = demangle(list(a)), demangle(list(b))
-    by_plain = {v: k for k, v in plain_a.items()}
-    for k in list(b):
-        if k in a:
-            continue
-        plain = plain_b[k]
-        for tail, repl in ((", (bool)0>", ">"), ("<(bool)0>", "")):   # cu++filt spells false as (bool)0
-            if plain.endswith(tail):
-                plain = plain[: -len(tail)] + repl
-                break
-        old_name = by_plain.get(plain)
-        if old_name is not None and old_name not in b:
-            b[old_name] = b.pop(k)
     changed = [k for k in a if k not in b or a[k] != b[k]]
     for k in sorted(a):
         print(("unchanged " if k not in changed else "CHANGED   ") + k)

@@ -151,14 +151,15 @@ int boundary_refine(const char* name, bool aa, const float* fields, int n_img, i
   p.area_thres = proposal_area_thres; p.max_sdf_thres = max_sdf_thres;
   p.max_shrink_thres = max_shrink_threshold; p.delta_ratio = delta_ratio;
   p.boxes_out = reinterpret_cast<float4*>(boxes_out); p.labels_out = labels_out; p.rounds_out = rounds_out;
+  p.image_hw = image_hw;
   if (int e = make_worklist(p.work, counts, n_img, cap, ws, s)) return e;
   if (W <= kWindowMaxSide && H <= kWindowMaxSide) {
     p.windows = window_tables(ws, n_img);
     const int e = (int)cudaMemsetAsync(p.windows, 0, sizeof(WindowSlot) * kWindowSlots * (size_t)n_img, s);
     if (e) return cuda_fail(e, "memset window tables");
   }
-  if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s, image_hw), "refine_aa_kernel");
-  return cuda_fail(launch_refine(p, num_sms(), s, image_hw), "refine_kernel");
+  if (aa) return cuda_fail(launch_refine_aa(p, num_sms(), s), "refine_aa_kernel");
+  return cuda_fail(launch_refine(p, num_sms(), s), "refine_kernel");
 }
 
 // unmore_center_reasoning / unmore_center_reasoning_aa and their _hw forms
@@ -202,8 +203,8 @@ int score_and_rasterise(const char* name, const float* fields, int n_img, int C,
   p.ch_sdf = ch_sdf; p.ch_crow = ch_center_row; p.ch_ccol = ch_center_col; p.ch_exist = ch_exist;
   p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
   p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
-  p.areas = areas_out; p.masks = masks_out;
-  return cuda_fail(launch_score(p, s, image_hw), "score_kernel");
+  p.areas = areas_out; p.masks = masks_out; p.image_hw = image_hw;
+  return cuda_fail(launch_score(p, s), "score_kernel");
 }
 
 // unmore_box_sums / unmore_box_sums_hw
@@ -267,8 +268,8 @@ int score_from_tiles(const char* name, const float* tiles, const float* existenc
   p.tiles = tiles; p.exist_scores = existence_scores; p.aa_raster = antialias; p.n_img = n_img; p.C = 4; p.H = H; p.W = W;
   p.boxes = boxes; p.boxes_f64 = boxes_f64; p.counts = counts; p.cap = cap;
   p.scores = reinterpret_cast<float4*>(scores_out); p.tight = reinterpret_cast<float4*>(tight_out);
-  p.areas = areas_out; p.masks = masks_out;
-  return cuda_fail(launch_score(p, s, image_hw), "score_kernel (tiles)");
+  p.areas = areas_out; p.masks = masks_out; p.image_hw = image_hw;
+  return cuda_fail(launch_score(p, s), "score_kernel (tiles)");
 }
 
 }  // namespace
@@ -522,7 +523,7 @@ int unmore_sat_build(const float* in, int n_planes, int H, int W, double* out, u
   if (n_planes < 0 || H <= 0 || W <= 0 || (n_planes > 0 && (!in || !out)))
     return fail(UNMORE_E_INVALID, "unmore_sat_build: bad argument");
   if (W > 2048) return fail(UNMORE_E_CAPACITY, "unmore_sat_build: W %d > 2048", W);
-  return cuda_fail(launch_sat(in, out, n_planes, H, W, 0, nullptr, 0, (cudaStream_t)stream), "sat_kernel");
+  return cuda_fail(launch_sat(in, out, n_planes, H, W, 0, nullptr, 0, nullptr, (cudaStream_t)stream), "sat_kernel");
 }
 
 int unmore_sat_build_fields(const float* fields, int n_img, int C, int H, int W, const int* channels_host, int n_channels,
@@ -533,7 +534,7 @@ int unmore_sat_build_fields(const float* fields, int n_img, int C, int H, int W,
   for (int i = 0; i < n_channels; ++i)
     if (channels_host[i] < 0 || channels_host[i] >= C) return fail(UNMORE_E_INVALID, "unmore_sat_build_fields: channel out of range");
   if (W > 2048) return fail(UNMORE_E_CAPACITY, "unmore_sat_build_fields: W %d > 2048", W);
-  return cuda_fail(launch_sat(fields, out, n_img * n_channels, H, W, C, channels_host, n_channels, (cudaStream_t)stream),
+  return cuda_fail(launch_sat(fields, out, n_img * n_channels, H, W, C, channels_host, n_channels, nullptr, (cudaStream_t)stream),
                    "sat_kernel");
 }
 
@@ -640,8 +641,8 @@ int unmore_sat_build_fields_hw(const float* fields, int n_img, int C, int H, int
   for (int i = 0; i < n_channels; ++i)
     if (channels_host[i] < 0 || channels_host[i] >= C) return fail(UNMORE_E_INVALID, "%s: channel out of range", name);
   if (W > 2048) return fail(UNMORE_E_CAPACITY, "%s: W %d > 2048", name, W);
-  return cuda_fail(launch_sat_hw(fields, out, n_img, H, W, C, channels_host, n_channels, image_hw, (cudaStream_t)stream),
-                   "sat_hw_kernel");
+  return cuda_fail(launch_sat(fields, out, n_img * n_channels, H, W, C, channels_host, n_channels, image_hw, (cudaStream_t)stream),
+                   "sat_kernel");
 }
 
 // the second resize mode (antialias=True) on a padded stack

@@ -12,7 +12,7 @@
 // that window is what is staged in shared memory (93,312 B, channels interleaved -> two CTAs per SM).
 //
 // The kernel template and its row sources live in this header; center.cu instantiates it for the primary mode and
-// the tiles, center_aa.cu for the second resize mode on fields (compiled beside them, the others' code changes).
+// the tiles, center_aa.cu for the second resize mode on fields.
 #pragma once
 #include <type_traits>
 
@@ -348,11 +348,10 @@ struct CenterAaRows {
 // PLANE_ELEMS: 0 = any field size / channel order; H*W = the three channels are consecutive planes of a field
 // of exactly that size (the COCO-val shape the batch path runs on), see MultiPlaneRows.  kAaFields = any field, the
 // second resize mode (CenterAaRows; the table after CenterSmem).
-// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The window snap (and with it
-// the split boxes) and the --analyze_cc clip use the image's extent; plane addressing and PLANE_ELEMS go by the pitch.
-// On tiles (PLANE_ELEMS = -1) only the snap and the clip change.
+// The window snap (and with it the split boxes) and the --analyze_cc clip use the image's extent (image_extent); plane
+// addressing and PLANE_ELEMS go by the (H, W) pitch.
 constexpr int kSpecPlaneElems = 480 * 640;
-template <bool ANALYZE_CC, int PLANE_ELEMS, bool ROW_SKIP, bool SIZED = false>
+template <bool ANALYZE_CC, int PLANE_ELEMS, bool ROW_SKIP>
 __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   CenterSmem& sm = *reinterpret_cast<CenterSmem*>(smem_raw);
@@ -412,13 +411,8 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
         next_located = true;
       }
     };
-    Window win;
-    if constexpr (SIZED) {
-      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
-      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
-    } else {
-      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
-    }
+    const int2 ext = image_extent(p.image_hw, img, p.H, p.W);
+    const Window win = snap_window<double>(x1, y1, x2, y2, ext.y, ext.x);
     double best = 0.0;
     int best_idx = -1;
     if (!win.empty()) {
@@ -767,14 +761,9 @@ __global__ void __launch_bounds__(kCenterThreads, 2) center_kernel(const CenterP
             double* o = p.cc_boxes + (row * kCcCap + tid) * 4;
             o[0] = (double)(int)fmax(cx - nw / 2, 0.0);
             o[1] = (double)(int)fmax(cy - nh / 2, 0.0);
-            if constexpr (SIZED) {
-              const int2 e = image_extent(p.image_hw, img, p.H, p.W);
-              o[2] = (double)(int)fmin(cx + nw / 2, (double)e.y);
-              o[3] = (double)(int)fmin(cy + nh / 2, (double)e.x);
-            } else {
-              o[2] = (double)(int)fmin(cx + nw / 2, (double)p.W);
-              o[3] = (double)(int)fmin(cy + nh / 2, (double)p.H);
-            }
+            const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+            o[2] = (double)(int)fmin(cx + nw / 2, (double)e.y);
+            o[3] = (double)(int)fmin(cy + nh / 2, (double)e.x);
           }
           if (tid == 0 && n_comp > kCcCap) atomicAdd(p.cc_overflow, 1);
         }
@@ -794,12 +783,6 @@ template <bool CC, int PE, bool RS = false>
 static int launch_center_t(const CenterParams& p, int num_sms, cudaStream_t stream) {
   constexpr int smem = (int)(sizeof(CenterSmem) + (PE == kAaFields ? sizeof(AaColTable) : 0));
   // function attributes are per device: set on every launch (microseconds), no cached state
-  if (p.image_hw) {   // a padded stack (fields or tiles): the sized variant
-    cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return (int)e;
-    center_kernel<CC, PE, RS, true><<<num_sms * 2, kCenterThreads, smem, stream>>>(p);
-    return (int)cudaGetLastError();
-  }
   cudaError_t e = cudaFuncSetAttribute(center_kernel<CC, PE, RS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return (int)e;
   center_kernel<CC, PE, RS><<<num_sms * 2, kCenterThreads, smem, stream>>>(p);

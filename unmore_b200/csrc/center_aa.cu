@@ -1,5 +1,5 @@
 // center_reasoning in the second resize mode (antialias=True) straight from the fields: the kernel of center.cuh on the
-// antialiased row source (CenterAaRows), in a file of its own so that the kernels of center.cu keep their code.
+// antialiased row source (CenterAaRows).
 #include "center.cuh"
 
 namespace unmore {

@@ -12,9 +12,10 @@ namespace unmore {
 
 constexpr int kExistWarps = 8;
 
-// SIZED: the fields are a padded stack and p.image_hw holds each image's (h, w) inside the (H, W) pitch; addresses
-// come from the pitch, the window snap from the image's own extent.
-template <bool SIZED>
+// Addresses come from the (H, W) pitch, the window snap from the image's own extent (image_extent).
+// PADDED = false compiles the stage without the table (p.image_hw is null): on uniform stacks the kernel that reads it
+// took 2% longer (227.1 -> 231.8 ms per bench.py step, one B200 at 1000 W).
+template <bool PADDED>
 __device__ __forceinline__ void existence_items(const ExistParams& p) {
   __shared__ int2 tapy_all[kExistWarps][kCrop];   // vertical taps of the warp's current window: (i0, bits of l1)
   const int lane = threadIdx.x & 31;
@@ -30,13 +31,8 @@ __device__ __forceinline__ void existence_items(const ExistParams& p) {
     const size_t row = (size_t)img * p.work.cap + k;
     double x1, y1, x2, y2;
     load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
-    Window win;
-    if constexpr (SIZED) {
-      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
-      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
-    } else {
-      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
-    }
+    const int2 e = image_extent(PADDED ? p.image_hw : nullptr, img, p.H, p.W);
+    const Window win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
     float score = 0.f;  // zero-size crop: the reference raises; defined as "nothing there"
     if (!win.empty()) {
       ColTaps taps;
@@ -78,15 +74,14 @@ __device__ __forceinline__ void existence_items(const ExistParams& p) {
   }
 }
 
-__global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const ExistParams p) { existence_items<false>(p); }
-__global__ void __launch_bounds__(kExistWarps * 32) existence_hw_kernel(const ExistParams p) { existence_items<true>(p); }
+template <bool PADDED>
+__global__ void __launch_bounds__(kExistWarps * 32) existence_kernel(const ExistParams p) { existence_items<PADDED>(p); }
 
 // The second resize mode (antialias=True): the mean of the antialiased crop (aa_rows.cuh), summed in exactly the order
 // above, so the score equals tile_means_kernel on the tile of unmore_crop_resize_aa bit for bit.
-// SIZED: as existence_items; the rows keep the pitch as their stride.
+// The window snaps as in existence_items; the rows keep the pitch as their stride.
 constexpr int kAaExistWarps = 2;   // 15 KB of shared memory per warp
 constexpr int kAaExistMinBlocks = 7;
-template <bool SIZED>
 __device__ __forceinline__ void existence_aa_items(const ExistParams& p) {
   __shared__ AaRowsSmem rows_all[kAaExistWarps];
   const int lane = threadIdx.x & 31;
@@ -101,13 +96,8 @@ __device__ __forceinline__ void existence_aa_items(const ExistParams& p) {
     const size_t row = (size_t)img * p.work.cap + k;
     double x1, y1, x2, y2;
     load_box<double>(p.boxes, p.boxes_f64 != 0, row, x1, y1, x2, y2);
-    Window win;
-    if constexpr (SIZED) {
-      const int2 e = image_extent(p.image_hw, img, p.H, p.W);
-      win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
-    } else {
-      win = snap_window<double>(x1, y1, x2, y2, p.W, p.H);
-    }
+    const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+    const Window win = snap_window<double>(x1, y1, x2, y2, e.y, e.x);
     float score = 0.f;
     if (!win.empty()) {
       AaCropRows src;
@@ -134,10 +124,7 @@ __device__ __forceinline__ void existence_aa_items(const ExistParams& p) {
 }
 
 __global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_kernel(const ExistParams p) {
-  existence_aa_items<false>(p);
-}
-__global__ void __launch_bounds__(kAaExistWarps * 32, kAaExistMinBlocks) existence_aa_hw_kernel(const ExistParams p) {
-  existence_aa_items<true>(p);
+  existence_aa_items(p);
 }
 
 // ---- a2 / a4 as a stand-alone op: the resized crops themselves --------------------------------
@@ -231,14 +218,13 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 }
 
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream) {
-  if (p.image_hw) existence_hw_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
-  else existence_kernel<<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
+  if (p.image_hw) existence_kernel<true><<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
+  else existence_kernel<false><<<num_sms * 4, kExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 
 int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream) {
-  if (p.image_hw) existence_aa_hw_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
-  else existence_aa_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
+  existence_aa_kernel<<<num_sms * kAaExistMinBlocks, kAaExistWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

@@ -359,11 +359,10 @@ constexpr int kRefineMinBlocks = 3;   // resident CTAs per SM, in __launch_bound
 constexpr int kSpecRowElems = 640;   // row pitch of the COCO-val-shaped fields the batch path runs on
 // The persistent round loop: warps pull proposals from the worklist until it is empty.  `terms(plane, win)` computes
 // the boundary terms of a window from its resampled rows; the resize mode only changes where those rows come from.
-// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch.  The extent is read where the
-// window is snapped and again where the box is updated, so it is not live across the terms (registers are tight).
-template <bool SIZED, class Terms>
-__device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCols& cols, int lane, Terms terms,
-                                                 const int* image_hw = nullptr) {
+// The image's extent (image_extent) is read where the window is snapped and again where the box is updated, so it is
+// not live across the terms (registers are tight).
+template <class Terms>
+__device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCols& cols, int lane, Terms terms) {
   const int total = worklist_total(p.work);
   int img = 0;   // image of the previous work item: the locate hint
   for (;;) {
@@ -388,19 +387,15 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
       const bool dbl = (r == 0) && p.boxes_f64;
       Window win;
       bool keep;
-      int ih = p.H, iw = p.W;
-      if constexpr (SIZED) {
-        const int2 e = image_extent(image_hw, img, p.H, p.W);
-        ih = e.x; iw = e.y;
-      }
+      int2 e = image_extent(p.image_hw, img, p.H, p.W);
       if (dbl) {
         BoxT<double> bd;
         load_box<double>(p.boxes, true, row, bd.x1, bd.y1, bd.x2, bd.y2);
         keep = __dmul_rn(__dsub_rn(bd.x2, bd.x1), __dsub_rn(bd.y2, bd.y1)) > (double)p.area_thres;
-        win = snap_window<double>(bd.x1, bd.y1, bd.x2, bd.y2, iw, ih);
+        win = snap_window<double>(bd.x1, bd.y1, bd.x2, bd.y2, e.y, e.x);
       } else {
         keep = __fmul_rn(__fsub_rn(bf.x2, bf.x1), __fsub_rn(bf.y2, bf.y1)) > p.area_thres;
-        win = snap_window<float>(bf.x1, bf.y1, bf.x2, bf.y2, iw, ih);
+        win = snap_window<float>(bf.x1, bf.y1, bf.x2, bf.y2, e.y, e.x);
       }
       if (p.apply_small_filter && !keep) { label = -2.f; break; }  // filter_small_proposal (:293-299), strict '>'
       float4 nb = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -425,21 +420,16 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
       }
       if (!win.empty()) {
         if (d.max_sdf > p.max_sdf_thres) {
-          if constexpr (SIZED) {
-            const int2 e = image_extent(image_hw, img, p.H, p.W);
-            ih = e.x; iw = e.y;
-          } else {
-            ih = p.H; iw = p.W;
-          }
+          e = image_extent(p.image_hw, img, p.H, p.W);
           if (dbl) {
             BoxT<double> bd;
             load_box<double>(p.boxes, true, row, bd.x1, bd.y1, bd.x2, bd.y2);
-            lab = apply_update<double>(p, iw, ih, win, d, bd, nb);
+            lab = apply_update<double>(p, e.y, e.x, win, d, bd, nb);
             // fp64 round 0: the fp32 cast must be exact and the fp32 area test of round 1 must agree
             fixed = (double)nb.x == bd.x1 && (double)nb.y == bd.y1 && (double)nb.z == bd.x2 && (double)nb.w == bd.y2 &&
                     (!p.apply_small_filter || __fmul_rn(__fsub_rn(nb.z, nb.x), __fsub_rn(nb.w, nb.y)) > p.area_thres);
           } else {
-            lab = apply_update<float>(p, iw, ih, win, d, bf, nb);
+            lab = apply_update<float>(p, e.y, e.x, win, d, bf, nb);
             fixed = true;
           }
         }
@@ -466,56 +456,35 @@ __device__ __forceinline__ void refine_proposals(const RefineParams& p, BorderCo
   }
 }
 
-template <int ROW_ELEMS, bool SIZED>
-__device__ __forceinline__ void refine_crops(const RefineParams& p, const int* image_hw) {
+template <int ROW_ELEMS>
+__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
   __shared__ BorderCols cols_all[kRefineWarps];
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
-  refine_proposals<SIZED>(p, cols, lane, [&](const float* plane, const Window& win) {
+  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
     CropRows<ROW_ELEMS> src;
     src.taps.template init<kStrided>(lane, win.w());
     src.plane.init(plane, p.W, win);
     src.init_rows(lane, cols.tapy, win.h());
     return boundary_terms(src, cols, lane);
-  }, image_hw);
-}
-
-template <int ROW_ELEMS>
-__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_kernel(const RefineParams p) {
-  refine_crops<ROW_ELEMS, false>(p, nullptr);
-}
-// the same on a padded stack: image_hw [n_img, 2] holds each image's (h, w) inside the (H, W) pitch
-template <int ROW_ELEMS>
-__global__ void __launch_bounds__(kRefineWarps * 32, kRefineMinBlocks) refine_hw_kernel(const RefineParams p,
-                                                                                        const int* __restrict__ image_hw) {
-  refine_crops<ROW_ELEMS, true>(p, image_hw);
+  });
 }
 
 // The second resize mode: the same round loop on antialiased rows (aa_rows.cuh).  A warp needs 15 KB more shared
 // memory for the weight table and the row ring, so fewer warps fit an SM.
 constexpr int kAaRefineWarps = 2;
 constexpr int kAaRefineMinBlocks = 5;
-template <bool SIZED>
-__device__ __forceinline__ void refine_aa(const RefineParams& p, const int* image_hw) {
+__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_kernel(const RefineParams p) {
   __shared__ BorderCols cols_all[kAaRefineWarps];
   __shared__ AaRowsSmem rows_all[kAaRefineWarps];
   const int lane = threadIdx.x & 31;
   BorderCols& cols = cols_all[threadIdx.x >> 5];
   AaRowsSmem& rows = rows_all[threadIdx.x >> 5];
-  refine_proposals<SIZED>(p, cols, lane, [&](const float* plane, const Window& win) {
+  refine_proposals(p, cols, lane, [&](const float* plane, const Window& win) {
     AaCropRows src;
     src.init(lane, rows, plane, p.W, win);
     return boundary_terms(src, cols, lane);
-  }, image_hw);
-}
-
-__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_kernel(const RefineParams p) {
-  refine_aa<false>(p, nullptr);
-}
-// the same on a padded stack, as refine_hw_kernel
-__global__ void __launch_bounds__(kAaRefineWarps * 32, kAaRefineMinBlocks) refine_aa_hw_kernel(const RefineParams p,
-                                                                                              const int* __restrict__ image_hw) {
-  refine_aa<true>(p, image_hw);
+  });
 }
 
 __global__ void __launch_bounds__(kRefineWarps * 32) tiles_kernel(const TileParams p) {
@@ -564,20 +533,16 @@ int launch_round_update(const RefineParams& p, const float4* deltas, const float
   return (int)cudaGetLastError();
 }
 
-int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw) {
+int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream) {
   const int ctas = num_sms * kRefineMinBlocks;  // warps pull proposals dynamically
-  if (image_hw) {   // the row-pitch specialisation goes by the pitch
-    if (p.W == kSpecRowElems) refine_hw_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p, image_hw);
-    else refine_hw_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p, image_hw);
-  } else if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
+  if (p.W == kSpecRowElems) refine_kernel<kSpecRowElems><<<ctas, kRefineWarps * 32, 0, stream>>>(p);   // by the pitch
   else refine_kernel<0><<<ctas, kRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 
-int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw) {
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream) {
   const int ctas = num_sms * kAaRefineMinBlocks;
-  if (image_hw) refine_aa_hw_kernel<<<ctas, kAaRefineWarps * 32, 0, stream>>>(p, image_hw);
-  else refine_aa_kernel<<<ctas, kAaRefineWarps * 32, 0, stream>>>(p);
+  refine_aa_kernel<<<ctas, kAaRefineWarps * 32, 0, stream>>>(p);
   return (int)cudaGetLastError();
 }
 

@@ -24,10 +24,12 @@ __device__ __forceinline__ double shfl_up_d(double v, int o) { return __shfl_up_
 // the field stack without a gather copy.
 struct PlaneSel { int n, C, ch[4]; };
 
-// SIZED: `in` is a padded field stack (sel.n > 0) and image_hw holds each image's (h, w) inside the (H, W) pitch; the
-// pixels outside it are read as zeros, so every entry S[y][x] with y <= h, x <= w is, bit for bit, that of the image
-// built alone (a padded value would otherwise reach the lane's scan total, and through it the columns left of it).
-template <int STEPS, bool SIZED = false>
+// On a padded field stack (sel.n > 0, image_hw non-null) the pixels outside each image's (h, w) are read as zeros, so
+// every entry S[y][x] with y <= h, x <= w is, bit for bit, that of the image built alone (a padded value would
+// otherwise reach the lane's scan total, and through it the columns left of it).  PADDED = false compiles the kernel
+// without the table and the mask (image_hw is null): with them, a uniform 642-px-wide stack took 2% longer (168
+// instead of 128 registers at STEPS = 8; one B200 at 1000 W).
+template <int STEPS, bool PADDED>
 __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel(const float* __restrict__ in, double* __restrict__ out,
                                                               int n_planes, int H, int W, const PlaneSel sel,
                                                               const int* __restrict__ image_hw) {
@@ -35,9 +37,9 @@ __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel(const float* __rest
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int plane = blockIdx.x * kSatWarps + warp;
   if (plane >= n_planes) return;
-  int2 ext = make_int2(H, W);
-  if constexpr (SIZED) ext = image_extent(image_hw, plane / sel.n, H, W);
-  const size_t src_plane = sel.n ? (size_t)(plane / sel.n) * sel.C + sel.ch[plane % sel.n] : (size_t)plane;
+  const int img = sel.n ? plane / sel.n : 0;   // sel.n == 0 (a dense stack of planes) comes without a table
+  const int2 ext = image_extent(PADDED ? image_hw : nullptr, img, H, W);
+  const size_t src_plane = sel.n ? (size_t)img * sel.C + sel.ch[plane % sel.n] : (size_t)plane;
   const float* src = in + src_plane * H * W;
   double* dst = out + (size_t)plane * (H + 1) * (W + 1);
   const int OW = W + 1;
@@ -61,7 +63,7 @@ __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel(const float* __rest
         v[s].z = x + 2 < W ? rowp[x + 2] : 0.f;
         v[s].w = x + 3 < W ? rowp[x + 3] : 0.f;
       }
-      if constexpr (SIZED) {   // padding was read (inside the pitch); it enters the sums as zeros
+      if constexpr (PADDED) {   // padding was read (inside the pitch); it enters the sums as zeros
         const int rw = y < ext.x ? ext.y : 0;
         v[s].x = x < rw ? v[s].x : 0.f;
         v[s].y = x + 1 < rw ? v[s].y : 0.f;
@@ -104,7 +106,7 @@ __global__ void __launch_bounds__(kSatWarps * 32) sat_kernel(const float* __rest
 // ring, completion tracked by one mbarrier per slot.  The rows wait in shared memory instead of in
 // registers, so a warp has 6 rows (15 KB at W=640) outstanding instead of one
 // (ring depth 3 / 4 / 6 / 8 measured: 4720 / 4699 / 5433 / 4387 GB/s at 3000 planes; 5-7 tie at 5950 GB/s at 8000).
-// Needs W % 4 == 0 (16-byte rows); launch_sat falls back to the register-fed kernel otherwise.
+// Needs W % 4 == 0 (16-byte rows) and a stack without padding; launch_sat takes the register-fed kernel otherwise.
 constexpr int kSatStages = 6;
 
 template <int STEPS>
@@ -189,8 +191,17 @@ static int launch_sat_tma(const float* in, double* out, int n_planes, int H, int
   return (int)cudaGetLastError();
 }
 
+template <bool PADDED>
+static int launch_sat_regs(const float* in, double* out, int n_planes, int H, int W, const PlaneSel& sel,
+                           const int* image_hw, int grid, int steps, cudaStream_t stream) {
+  if (steps <= 5) sat_kernel<5, PADDED><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, image_hw);
+  else if (steps <= 8) sat_kernel<8, PADDED><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, image_hw);
+  else sat_kernel<16, PADDED><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, image_hw);
+  return (int)cudaGetLastError();
+}
+
 int launch_sat(const float* in, double* out, int n_planes, int H, int W, int C, const int* channels, int n_ch,
-               cudaStream_t stream) {
+               const int* image_hw, cudaStream_t stream) {
   if (n_planes <= 0) return 0;
   PlaneSel sel{};
   sel.n = n_ch; sel.C = C;
@@ -198,39 +209,20 @@ int launch_sat(const float* in, double* out, int n_planes, int H, int W, int C, 
   const int grid = (n_planes + kSatWarps - 1) / kSatWarps;
   const int steps = (W + 127) / 128;
   // bulk-copy path: 16-byte aligned rows (W % 4 == 0; planes of a 16-byte aligned tensor then are too)
-  if ((W & 3) == 0 && ((size_t)H * W & 3) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && steps <= 8) {
+  if (!image_hw && (W & 3) == 0 && ((size_t)H * W & 3) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && steps <= 8) {
     if (steps <= 5) return launch_sat_tma<5>(in, out, n_planes, H, W, sel, grid, stream);
     return launch_sat_tma<8>(in, out, n_planes, H, W, sel, grid, stream);
   }
-  if (steps <= 5) sat_kernel<5><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, nullptr);
-  else if (steps <= 8) sat_kernel<8><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, nullptr);
-  else if (steps <= 16) sat_kernel<16><<<grid, kSatWarps * 32, 0, stream>>>(in, out, n_planes, H, W, sel, nullptr);
-  else return -2;
-  return (int)cudaGetLastError();
+  if (steps > 16) return -2;
+  if (image_hw) return launch_sat_regs<true>(in, out, n_planes, H, W, sel, image_hw, grid, steps, stream);
+  return launch_sat_regs<false>(in, out, n_planes, H, W, sel, nullptr, grid, steps, stream);
 }
 
-int launch_sat_hw(const float* fields, double* out, int n_img, int H, int W, int C, const int* channels, int n_ch,
-                  const int* image_hw, cudaStream_t stream) {
-  const int n_planes = n_img * n_ch;
-  if (n_planes <= 0) return 0;
-  PlaneSel sel{};
-  sel.n = n_ch; sel.C = C;
-  for (int i = 0; i < n_ch && i < 4; ++i) sel.ch[i] = channels[i];
-  const int grid = (n_planes + kSatWarps - 1) / kSatWarps;
-  const int steps = (W + 127) / 128;
-  if (steps <= 5) sat_kernel<5, true><<<grid, kSatWarps * 32, 0, stream>>>(fields, out, n_planes, H, W, sel, image_hw);
-  else if (steps <= 8) sat_kernel<8, true><<<grid, kSatWarps * 32, 0, stream>>>(fields, out, n_planes, H, W, sel, image_hw);
-  else if (steps <= 16) sat_kernel<16, true><<<grid, kSatWarps * 32, 0, stream>>>(fields, out, n_planes, H, W, sel, image_hw);
-  else return -2;
-  return (int)cudaGetLastError();
-}
-
-// box_sums_kernel (box_sums.cu) on the tables of a padded stack (launch_sat_hw), indexed on the pitch; the window snaps
-// to the image's own extent.
-__global__ void box_sums_hw_kernel(const double* __restrict__ sat, int planes_per_img, int plane, int H, int W,
-                                   const void* __restrict__ boxes, int boxes_f64, const int* __restrict__ counts, int cap,
-                                   int n_img, double* __restrict__ sums, double* __restrict__ means,
-                                   const int* __restrict__ image_hw) {
+// boxsum (top of the file): the tables are indexed on the pitch, the window snaps to the image's own extent.
+__global__ void box_sums_kernel(const double* __restrict__ sat, int planes_per_img, int plane, int H, int W,
+                                const void* __restrict__ boxes, int boxes_f64, const int* __restrict__ counts, int cap,
+                                int n_img, double* __restrict__ sums, double* __restrict__ means,
+                                const int* __restrict__ image_hw) {
   const int id = blockIdx.x * blockDim.x + threadIdx.x;
   if (id >= n_img * cap) return;
   const int img = id / cap, k = id - img * cap;
@@ -248,13 +240,13 @@ __global__ void box_sums_hw_kernel(const double* __restrict__ sat, int planes_pe
   if (means) means[id] = w.empty() ? 0.0 : s / ((double)w.w() * (double)w.h());
 }
 
-int launch_box_sums_hw(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
-                       const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
-                       cudaStream_t stream) {
+int launch_box_sums(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
+                    const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
+                    cudaStream_t stream) {
   const int total = n_img * cap;
   if (total <= 0) return 0;
-  box_sums_hw_kernel<<<(total + 255) / 256, 256, 0, stream>>>(sat, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap,
-                                                              n_img, sums, means, image_hw);
+  box_sums_kernel<<<(total + 255) / 256, 256, 0, stream>>>(sat, planes_per_img, plane, H, W, boxes, boxes_f64, counts, cap,
+                                                            n_img, sums, means, image_hw);
   return (int)cudaGetLastError();
 }
 

@@ -65,14 +65,10 @@ __device__ __forceinline__ bool resized_mask_bit_aa(const uint32_t m[kCrop][4], 
 // of the reference's original mode); the masks are rasterised back to the box with the antialiased kernel when
 // p.aa_raster is set and with the plain one otherwise; p.exist_scores, when given, replaces the mean of the fourth
 // tile (the reference's classifier puts out one scalar per crop, object_scoring.py:140-150).
-// SIZED: a padded stack, p.image_hw holds each image's (h, w) inside the (H, W) pitch (on the tile path, the tiles
-// were cropped from such a stack).  The window snaps to the image's extent; the mask canvas stays H x ceil(W/32) words
-// (bits outside the image stay 0).
-template <bool SIZED> struct ScoreArgs { using type = ScoreParams; };
-template <> struct ScoreArgs<true> { using type = ScoreHwParams; };
-
-template <bool TILES_AA, bool SIZED = false>
-__global__ void __launch_bounds__(kScoreThreads) score_kernel(const typename ScoreArgs<SIZED>::type p) {
+// The window snaps to the image's extent (image_extent; on the tile path, that of the image the tiles were cropped
+// from); the mask canvas stays H x ceil(W/32) words of the pitch (bits outside the image stay 0).
+template <bool TILES_AA>
+__global__ void __launch_bounds__(kScoreThreads) score_kernel(const ScoreParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ScoreSmem& sm = *reinterpret_cast<ScoreSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -82,13 +78,8 @@ __global__ void __launch_bounds__(kScoreThreads) score_kernel(const typename Sco
   const size_t row = (size_t)img * p.cap + k;
   double bx1, by1, bx2, by2;
   load_box<double>(p.boxes, p.boxes_f64 != 0, row, bx1, by1, bx2, by2);
-  Window win;
-  if constexpr (SIZED) {
-    const int2 e = image_extent(p.image_hw, img, p.H, p.W);
-    win = snap_window<double>(bx1, by1, bx2, by2, e.y, e.x);
-  } else {
-    win = snap_window<double>(bx1, by1, bx2, by2, p.W, p.H);
-  }
+  const int2 e = image_extent(p.image_hw, img, p.H, p.W);
+  const Window win = snap_window<double>(bx1, by1, bx2, by2, e.y, e.x);
   const int Wp = (p.W + 31) >> 5;
   uint32_t* mask_out = p.masks ? p.masks + row * (size_t)p.H * Wp : nullptr;
   if (tid == 0) { sm.xmin = 1 << 30; sm.ymin = 1 << 30; sm.xmax = -1; sm.ymax = -1; sm.area = 0; }
@@ -258,23 +249,17 @@ int launch_mask_resize(const unsigned char* masks, int B, int oh, int ow, unsign
   return (int)cudaGetLastError();
 }
 
-template <bool TILES_AA, bool SIZED>
-static int launch_score_t(const typename ScoreArgs<SIZED>::type& p, cudaStream_t stream) {
-  cudaError_t e = cudaFuncSetAttribute(score_kernel<TILES_AA, SIZED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
+template <bool TILES_AA>
+static int launch_score_t(const ScoreParams& p, cudaStream_t stream) {
+  cudaError_t e = cudaFuncSetAttribute(score_kernel<TILES_AA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScoreSmem));
   if (e != cudaSuccess) return (int)e;
-  score_kernel<TILES_AA, SIZED><<<dim3(p.cap, p.n_img), kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
+  score_kernel<TILES_AA><<<dim3(p.cap, p.n_img), kScoreThreads, sizeof(ScoreSmem), stream>>>(p);
   return (int)cudaGetLastError();
 }
 
-int launch_score(const ScoreParams& p, cudaStream_t stream, const int* image_hw) {
+int launch_score(const ScoreParams& p, cudaStream_t stream) {
   if (p.n_img <= 0 || p.cap <= 0) return 0;
-  if (image_hw) {
-    ScoreHwParams hp;
-    static_cast<ScoreParams&>(hp) = p;
-    hp.image_hw = image_hw;
-    return p.tiles ? launch_score_t<true, true>(hp, stream) : launch_score_t<false, true>(hp, stream);
-  }
-  return p.tiles ? launch_score_t<true, false>(p, stream) : launch_score_t<false, false>(p, stream);
+  return p.tiles ? launch_score_t<true>(p, stream) : launch_score_t<false>(p, stream);
 }
 
 // area_score, final score, COCO xywh box and the post_process predicate (object_scoring.py:244-266,

@@ -35,6 +35,7 @@ struct RefineParams {
   float* labels_out;   // 1 / 0 / -1 as the reference; -2 = removed by filter_small_proposal
   int* rounds_out;     // rounds actually evaluated (nullable)
   WindowSlot* windows; // [n_img][kWindowSlots], zeroed before launch; nullptr: every round computes its terms
+  const int* image_hw; // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch
 };
 struct TileParams {
   const float* tiles;  // [M, 128, 128]
@@ -42,9 +43,8 @@ struct TileParams {
   float4* deltas;      // [M] (dx1, dy1, dx2, dy2)
   float* max_sdf;      // [M] or nullptr
 };
-// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
-int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw = nullptr);
-int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream, const int* image_hw = nullptr);   // antialiased crops
+int launch_refine(const RefineParams& p, int num_sms, cudaStream_t stream);
+int launch_refine_aa(const RefineParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
 int launch_tiles(const TileParams& p, cudaStream_t stream);
 int launch_round_update(const RefineParams& p, const float4* deltas, const float* max_sdf, int M, cudaStream_t stream);
 
@@ -56,7 +56,7 @@ struct ExistParams {
   int boxes_f64;
   WorkList work;
   float* scores;  // [n_img, cap]
-  const int* image_hw;  // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
+  const int* image_hw;  // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch
 };
 int launch_existence(const ExistParams& p, int num_sms, cudaStream_t stream);
 int launch_existence_aa(const ExistParams& p, int num_sms, cudaStream_t stream);   // antialiased crops
@@ -64,7 +64,7 @@ int launch_tile_means(const float* tiles, long long tile_stride, int M, float* o
 int launch_crop_resize(const float* fields, int n_img, int C, int H, int W, const int* channels, int n_ch,
                        const void* boxes, int boxes_f64, const int* counts, int cap, float* out, cudaStream_t stream);
 
-// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variants
+// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch
 int launch_crop_resize_aa(const float* fields, int n_img, int C, int H, int W, const int* channels, int n_ch,
                           const void* boxes, int boxes_f64, const int* counts, int cap, float* out, float* scratch,
                           cudaStream_t stream, const int* image_hw = nullptr);
@@ -93,7 +93,7 @@ struct CenterParams {
   unsigned char* cc_counts;  // [n_img, cap] component boxes emitted (0 unless the proposal passes with >= 2 components)
   double* cc_boxes;          // [n_img, cap, kCcCap, 4] enlarged component boxes
   int* cc_overflow;          // incremented once per proposal with more than kCcCap components
-  const int* image_hw;       // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch: the sized kernel variant
+  const int* image_hw;       // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch
 };
 int launch_center(const CenterParams& p, int num_sms, cudaStream_t stream);
 int launch_center_aa(const CenterParams& p, int num_sms, cudaStream_t stream);   // antialiased crops, from the fields
@@ -157,12 +157,9 @@ struct ScoreParams {
   float4* tight;       // [n_img, cap] tight box xyxy of the union mask (zeros if empty)
   int* areas;          // [n_img, cap] set pixels
   uint32_t* masks;     // nullable [n_img, cap, H, ceil(W/32)] packed union masks
+  const int* image_hw; // nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch
 };
-// The sized kernel variant's parameters (a struct of its own: a larger ScoreParams changes the code of score_kernel)
-struct ScoreHwParams : ScoreParams {
-  const int* image_hw; // [n_img, 2] (h, w) of each image inside the (H, W) pitch
-};
-int launch_score(const ScoreParams& p, cudaStream_t stream, const int* image_hw = nullptr);
+int launch_score(const ScoreParams& p, cudaStream_t stream);
 int launch_mask_resize(const unsigned char* masks, int B, int oh, int ow, unsigned char* out, cudaStream_t stream);
 
 struct FinalParams {
@@ -179,18 +176,14 @@ struct FinalParams {
 };
 int launch_final_scores(const FinalParams& p, cudaStream_t stream);
 
-// ---- sat.cu, box_sums.cu --------------------------------------------------------------------------
+// ---- sat.cu --------------------------------------------------------------------------
+// image_hw: nullable [n_img, 2] (h, w) of each image inside the (H, W) pitch; null: every image fills the pitch;
+// pixels outside each image's (h, w) enter the sums as zeros
 int launch_sat(const float* in, double* out, int n_planes, int H, int W, int C, const int* channels, int n_ch,
-               cudaStream_t stream);
-// tables of a padded field stack: pixels outside each image's (h, w) enter the sums as zeros
-int launch_sat_hw(const float* fields, double* out, int n_img, int H, int W, int C, const int* channels, int n_ch,
-                  const int* image_hw, cudaStream_t stream);
+               const int* image_hw, cudaStream_t stream);
 int launch_box_sums(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
                     const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
                     cudaStream_t stream);
-int launch_box_sums_hw(const double* sat, int planes_per_img, int plane, int H, int W, const void* boxes, int boxes_f64,
-                       const int* counts, int cap, int n_img, double* sums, double* means, const int* image_hw,
-                       cudaStream_t stream);
 
 // ---- masks.cu ------------------------------------------------------------------------
 int launch_mask_pack(const unsigned char* in, uint32_t* out, size_t n_masks, int H, int W, int num_sms, cudaStream_t stream);
